@@ -9,6 +9,9 @@ in-silico assembly, level 4, single chain); ``--workload G`` is configs[3] (~1 G
   python bench.py --gpus N --steps K --warmup W            our arm (CUDA through the C ABI)
   python bench.py --impl reference ...                     CPU arm: the oracle port of the reference
                                                            algorithm on all host cores
+  python bench.py ... --dump-outputs DIR                   also write the timed path's last outputs to DIR/*.npy
+
+Our arm runs the library that build() compiled (``__graft_entry__.build()``) and writes nothing into the tree.
 
 value   = proposals scored / device time (sum of per-step CUDA-event intervals on the launching
           stream; chain state and contacts resident in HBM; L2 flushed between steps, untimed)
@@ -32,6 +35,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # nothing is written into the tree, which may be read-only
 DEFAULT_MODE = "exact"
 
 def params_for(level):
@@ -152,6 +156,34 @@ def frag_orders(level, n_chains, n_steps, seed):
             v.extend(rng.permutation(level.n_frags).tolist())
         out[c] = v[:n_steps]
     return out
+
+
+def dump_outputs(folder, records, rs, best, lik, nc):
+    """Writes what the replica pass (the timed path of the headline value) handed its caller after its last step, as
+    float64 .npy files, so that two builds run with the same arguments can be compared output for output:
+      last_step_<field>[chain]           the last step's record of every chain (ReplicaSet.run_cycle)
+      allgather_{best,likelihood,n_contigs}  the exchange that follows it (ReplicaSet.allgather)
+      scaffold_<field>[chain, i]         each chain's live scaffold (13 x NF int32) at fragments scaffold_fragment_index[i]:
+                                         all of them, or a fixed seeded sample when all chains' full arrays would exceed 48 MB
+    With several GPUs the chains are those of rank 0."""
+    from instagraal_b200._lib import FIELDS13
+    os.makedirs(folder, exist_ok=True)
+
+    def save(name, a):
+        np.save(os.path.join(folder, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+    for field in records.dtype.names:
+        save("last_step_" + field, records[field][:, -1])
+    save("allgather_best", [best])
+    save("allgather_likelihood", lik)
+    save("allgather_n_contigs", nc)
+    nf = rs.nf
+    cap = (48 << 20) // (8 * 13 * rs.n)
+    idx = np.arange(nf) if nf <= cap else np.sort(np.random.RandomState(0).choice(nf, cap, replace=False))
+    states = np.stack([c._get_state()[:, idx] for c in rs.chains])
+    save("scaffold_fragment_index", idx)
+    for i, field in enumerate(FIELDS13):
+        save("scaffold_" + field, states[:, i])
 
 
 def nuis_stats(s, reset=True):
@@ -326,10 +358,10 @@ def run_ours(args):
     with ClockSampler(local) as clk:
         t_wall0 = time.perf_counter()
         for a in range(0, args.steps, seg):
-            out = rs.run_cycle(orders[:, a:a + seg], 5, cycle=200 + a)
+            records = rs.run_cycle(orders[:, a:a + seg], 5, cycle=200 + a)
             sts = [c.get_stats(reset=True) for c in rs.chains]
             dev_ms_multi += max(x["ms_step"] for x in sts)      # the chains of one GPU start together: the slowest one
-            prop_multi += float(out["n_proposals"].sum())
+            prop_multi += float(records["n_proposals"].sum())
             launches += int(sum(x["launches"] for x in sts))
             best, lik, nc = rs.allgather()
         torch.cuda.synchronize()
@@ -355,6 +387,8 @@ def run_ours(args):
         if dist is not None:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, records, rs, best, lik, nc)
 
     peak, peak_src = measured_peak()
     nnz, ns = s.n_non_zero, int(s.init_n_sub_frags)
@@ -646,14 +680,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-ref-gpu", action="store_true")
     ap.add_argument("--ref-gpu-budget-s", type=float, default=10.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed replica pass returned after its last step to DIR/<name>.npy (rank 0's chains)")
     args = ap.parse_args()
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     if args.impl == "reference":
         run_reference(args)
     else:
-        import __graft_entry__ as g
-        if int(os.environ.get("LOCAL_RANK", "0")) == 0:
-            g.build()
         run_ours(args)
 
 

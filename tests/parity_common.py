@@ -108,6 +108,43 @@ def replay(golden, impl, max_steps=None, check_state=True, check_nuis=True):
     return res
 
 
+class OracleTeacher:
+    """The NumPy port of the reference (oracle/sampler_oracle.py, held to the reference's recorded trajectories by
+    tests/test_oracle_golden.py) behind the interface of oracle.ref_replay.RefReplaySampler.  Lockstep tests whose teacher is
+    the reference's own compiled kernels (oracle/_ref/, built from a checkout of the reference) use it where those are not
+    built.  Its scores follow the host's powf / log10, so they are compared within score_tol and ties at 2e-8 relative,
+    not at the 1e-9 that holds between the reference's kernels and the product (same libdevice code on the GPU)."""
+
+    def __init__(self, level, p8):
+        from oracle.sampler_oracle import OracleSampler
+        self.o = OracleSampler(level, p8)
+        self.valid_insert = self   # RefReplaySampler.valid_insert.get()
+
+    def get(self):
+        return np.asarray(self.o.valid, dtype=np.int32)
+
+    def set_state(self, st):
+        self.o.live = {k: np.array(st[i], dtype=np.int32) for i, k in enumerate(FIELDS13)}
+
+    def get_state(self):
+        return np.stack([self.o.live[k] for k in FIELDS13]).astype(np.int32)
+
+    def set_valid(self, v):
+        self.o.valid = [int(x) for x in v]
+
+    def set_params(self, p8):
+        from oracle import score as sc
+        self.o.params8 = np.asarray(p8, dtype=np.float32).copy()
+        self.o.params = sc.Params(self.o.params8)
+
+    def step_sampler(self, a, cands):
+        return self.o.step_sampler(int(a), candidates=[int(c) for c in cands])
+
+    @property
+    def all_scores(self):
+        return self.o.all_scores
+
+
 def state_mismatch_modulo_length_ties(got, want):
     """Fields that differ between two [13, NF] scaffolds, with contig labels compared the way BASELINE.md prescribes:
     modulo relabelling among contigs of EQUAL length.  The reference numbers contigs by descending length through a

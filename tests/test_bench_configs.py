@@ -21,7 +21,7 @@ import numpy as np
 import pytest
 
 from instagraal_b200.synth import make_workload, workload_params
-from parity_common import FIELDS13, state_mismatch_modulo_length_ties
+from parity_common import FIELDS13, OracleTeacher, score_tol, state_mismatch_modulo_length_ties
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -78,11 +78,17 @@ def lockstep_vs_reference_kernels(level, p8, state13, n_steps, seed, probes=(), 
     (RefReplaySampler(canonical_slice_order=True)): on a GPU that order is decided by the execution order of slice_sp_mat's
     atomicAdd and changes from run to run, and through eval_sub_likelihood's last-block quirk (KA:4362) it changes the scores
     of the uniq positions >= n_sub % 64.  raw_slice_order=True keeps the reference's own (arbitrary) order and checks that
-    every disagreement is confined to exactly those positions (then nothing else of the step is compared)."""
+    every disagreement is confined to exactly those positions (then nothing else of the step is compared).
+
+    Where the reference's kernels are not built, the teacher is its NumPy port (parity_common.OracleTeacher) and scores,
+    ties and the chosen move's likelihood are compared at the port's tolerance."""
     from oracle.ref_replay import RefReplaySampler
     from oracle.sampler_oracle import return_neighbours, setup_distri_frags
     from test_gpu_parity import GpuImpl
-    ref = RefReplaySampler(level, p8, backend="gpu", canonical_slice_order=not raw_slice_order)
+    kernels = _cubin()
+    assert kernels or not raw_slice_order
+    ref = RefReplaySampler(level, p8, backend="gpu", canonical_slice_order=not raw_slice_order) if kernels else OracleTeacher(level, p8)
+    tie = 1e-9 if kernels else 2e-8
     order_dependent_steps = 0
     mine = GpuImpl(level)
     extra = {name: GpuImpl(level, **kw) for name, kw in probes}
@@ -136,7 +142,10 @@ def lockstep_vs_reference_kernels(level, p8, state13, n_steps, seed, probes=(), 
             continue
         rel = float(relv.max())
         worst = max(worst, rel)
-        assert rel < 1e-9, (t, f, cands, rel)
+        if kernels:
+            assert rel < 1e-9, (t, f, cands, rel)
+        else:
+            assert np.all(np.abs(sa[nz] - sb[nz]) <= score_tol(sa[nz])), (t, f, cands, rel)
         gid_ref = cands.index(int(b)) * 24 + int(op)
         gid = cands.index(int(r["B"])) * 24 + int(r["op"])
         new_state = ref.get_state()
@@ -148,10 +157,10 @@ def lockstep_vs_reference_kernels(level, p8, state13, n_steps, seed, probes=(), 
             assert float(r["dist"]) == float(dist), (t, r["dist"], dist)
             assert int(r["n_contigs"]) == int(nc), (t, r["n_contigs"], nc)
             assert np.float32(r["mean_len"]) == np.float32(mean_len), (t, r["mean_len"], mean_len)
-            assert abs(float(r["o"]) - float(o)) <= 1e-9 * abs(float(o)), (t, r["o"], o)
+            assert abs(float(r["o"]) - float(o)) <= tie * abs(float(o)), (t, r["o"], o)
         else:
             gap = abs(sa[gid] - sa[gid_ref])
-            assert gap <= 1e-9 * abs(sa[gid_ref]), ("different move without a tie", t, gid, gid_ref, float(gap))
+            assert gap <= tie * abs(sa[gid_ref]), ("different move without a tie", t, gid, gid_ref, float(gap))
             ties += 1
         for name, impl in extra.items():
             rr = impl.step(f, cands)
@@ -188,7 +197,6 @@ def _probe_summary(stats):
     return out
 
 
-@pytest.mark.skipif(not _cubin(), reason="reference cubin not built")
 def test_T_full_cycle_from_the_bench_state(built):
     """config T: one full MCMC cycle (NF steps) from the bench's burnt-in state (bomb + 2 cycles)"""
     level = level_of("T")
@@ -215,7 +223,6 @@ def test_T_reference_own_slice_order_only_moves_the_last_block_positions(built):
     assert res["steps"] == 400
 
 
-@pytest.mark.skipif(not _cubin(), reason="reference cubin not built")
 def test_Y3_200_steps(built):
     level = level_of("Y3")
     p8 = workload_params(level)
@@ -224,16 +231,16 @@ def test_Y3_200_steps(built):
     assert res["steps"] == 200 and res["same"] >= 0.9 * res["steps"], res
 
 
-@pytest.mark.skipif(not _cubin(), reason="reference cubin not built")
 @pytest.mark.parametrize("start", ["bomb", "true"])
 def test_G_steps_and_rigid_pruning_error(built, start):
     """config G (the ~1 Gb level the north-star target is stated on): 10 steps from the mid-assembly start (bomb + 3
-    cycles) and from the fully assembled start; also measures the score error of rigid pruning (D2)."""
+    cycles) and from the fully assembled start; also measures the score error of rigid pruning (D2).  With the reference's
+    NumPy port as teacher (~30 s a step at this level on one host core) the default is 3 steps."""
     level = level_of("G")
     p8 = workload_params(level)
     n_burn = int(os.environ.get("IG_TEST_G_BURN", "3"))
     st = burnt_state(level, p8, n_burn, 1000, start)
-    n_steps = int(os.environ.get("IG_TEST_G_STEPS", "10"))
+    n_steps = int(os.environ.get("IG_TEST_G_STEPS", "10" if _cubin() else "3"))
     res = lockstep_vs_reference_kernels(level, p8, st, n_steps, seed=5, probes=(("rigid", dict(rigid_pruning=True)),))
     _dump("rigid_error_G_%s.json" % start, dict(workload="G", start=start, burn_cycles=n_burn, steps=res["steps"], ties=res["ties"],
                                                worst_rel=res["worst_rel"], n_contigs=int((st[0] == 0).sum()),

@@ -8,13 +8,16 @@ import pytest
 from conftest import load_golden
 from instagraal_b200.synth import WORKLOADS, make_level
 from oracle import ref_kernels as rk
-from parity_common import replay
+from parity_common import OracleTeacher, replay, score_tol
 
 
 class ReplayImpl:
     def __init__(self, level, p8, backend):
         from oracle.ref_replay import RefReplaySampler
-        self.r = RefReplaySampler(level, p8, backend=backend, canonical_slice_order=(backend == "gpu"))  # GPU: atomic order varies run to run
+        if backend == "oracle":   # the reference's NumPy port, where its kernels are not built
+            self.r = OracleTeacher(level, p8)
+        else:
+            self.r = RefReplaySampler(level, p8, backend=backend, canonical_slice_order=(backend == "gpu"))  # GPU: atomic order varies run to run
 
     def set_state(self, st):
         self.r.set_state(st)
@@ -48,15 +51,15 @@ def test_replay_cpu_backend_matches_golden_exactly():
 @pytest.mark.parametrize("d_exp", [None, 2.37])
 def test_reference_kernels_on_gpu_vs_product(built, d_exp):
     """GPU-vs-GPU: the reference's own kernels (cubin) and the product agree on every score to 1e-9
-    relative (same libdevice powf/log10) over a replayed trajectory."""
+    relative (same libdevice powf/log10) over a replayed trajectory.  Where the cubin is not built, the teacher is the
+    reference's NumPy port and every score is held to parity_common.score_tol."""
     import os
     from oracle.ref_replay import _HERE
-    if not os.path.exists(os.path.join(_HERE, "_ref", "ref_kernels.cubin")):
-        pytest.skip("reference cubin not built")
+    kernels = os.path.exists(os.path.join(_HERE, "_ref", "ref_kernels.cubin"))
     from test_gpu_parity import GpuImpl
     g = load_golden("toy_bomb_seed2")
     level = make_level(WORKLOADS["toy"])
-    ref = ReplayImpl(level, g["params8"], "gpu")
+    ref = ReplayImpl(level, g["params8"], "gpu" if kernels else "oracle")
     mine = GpuImpl(level)
     worst = 0.0
     n = 60
@@ -77,5 +80,7 @@ def test_reference_kernels_on_gpu_vs_product(built, d_exp):
         assert np.array_equal(sa != 0, sb != 0), t
         nz = sa != 0
         worst = max(worst, float(np.max(np.abs(sa[nz] - sb[nz]) / np.abs(sa[nz]))))
-    assert worst < 1e-9, worst
+        if not kernels:
+            assert np.all(np.abs(sa[nz] - sb[nz]) <= score_tol(sa[nz])), t
+    assert worst < 1e-9 or not kernels, worst
     mine.s.free_gpu()
