@@ -81,6 +81,18 @@ typedef struct ig_cycle_step {   /* compact per-step record of ig_run_cycle (wha
     int32_t q4_hits;
 } ig_cycle_step;
 
+typedef struct ig_nuisance_step {   /* one nuisance step of a production-mode cycle (ig_set_device_nuisance), 80 B */
+    double likelihood_nuis;    /* eval_likelihood_4_nuisance under p_test (CL:1296-1344) */
+    double likelihood_t_after; /* likelihood_t after the step: likelihood_nuis if accepted, else the step's o */
+    double u;                  /* acceptance draw */
+    double draw;               /* the normal draw added to the moved parameter (NaN: none, d_nuc <= 0) */
+    float p_test[8];           /* the proposed parameter set: kuhn, lm, c1, slope, d, d_max, fact, v_inter */
+    int32_t id_modif;          /* 0 fact, 1 slope, 2 d_max, 3 d_nuc (= v_inter) */
+    int32_t accepted;          /* exp(likelihood_nuis - o) >= u, and valid */
+    int32_t valid;             /* 0: non-finite value, fact <= 0, slope >= 0, no d_max root, d_max <= 0 or v_inter <= 0 */
+    int32_t pad;
+} ig_nuisance_step;
+
 /* sampler.__init__ device part (CL:92-319: sparse_data_2_gpu, setup_all_gpu_struct, loadProgram) */
 int ig_create(const ig_config* cfg, const ig_level_data* data, ig_handle** out);
 /* sampler.free_gpu (CL:3167-3177) */
@@ -117,6 +129,22 @@ int ig_set_neighbour_weights(ig_handle* h, const int64_t* ptr, const int32_t* id
 int ig_run_cycle_device(ig_handle* h, int32_t n_steps, const int32_t* frags, int32_t n_neighbours, uint64_t seed,
                         uint32_t cycle, ig_cycle_step* out);
 int ig_get_cycle_plan(ig_handle* h, int32_t n_steps, int32_t* out /* [n_steps][2 + IG_MAX_CANDS] */);
+/* The nuisance-parameter step of the production RNG mode (step_nuisance_parameters, CL:2961-3051; full_em runs it after
+ * every step_sampler from cycle 5 on, IG:242-252).  While on, ig_run_cycle_device, ig_run_cycles_device_multi and
+ * ig_run_cycle_device_async / ig_cycle_wait run one nuisance step on the device after every step, without host work:
+ *   draws     Philox4x32-10 with the chain's seed as key, A = (t, cycle, 0x80000000, 0), B = (t, cycle, 0x80000001, 0):
+ *             id_modif = A.x >> 30, acceptance u = 53-bit uniform of (A.y, A.z), draw = sigma * Box-Muller normal of (B)
+ *   proposal  the float32 arithmetic of the reference's proposal; d_max = the root of rippe(x) = d_nuc in double,
+ *             rounded to float32 (DESIGN.md D3) instead of scipy's fsolve
+ *   invalid   (non-finite, fact <= 0, slope >= 0, no root, d_max <= 0, v_inter <= 0): rejected, nothing changes
+ *   decision  exp(L_nuis - o) >= u with L_nuis = eval_likelihood_4_nuisance under the proposal on the coordinates of
+ *             the step's start (quirk Q5); on acceptance the live parameters become the proposal and the next step
+ *             recomputes its likelihood sums (decided on the device).
+ * Needs the per-contact likelihood records (not with IG_LNZ_CACHE=0), parameters set with v_inter > 0, and no pending
+ * asynchronous cycle.  ig_run_cycle (parity mode, host-drawn neighbours) refuses to run while it is on.  Off (the default):
+ * every call behaves as without it.  ig_get_nuisance_records returns the per-step records of the last cycle. */
+int ig_set_device_nuisance(ig_handle* h, int32_t on);
+int ig_get_nuisance_records(ig_handle* h, int32_t n_steps, ig_nuisance_step* out);
 /* eval = score every mutation of one (A,B) pair without applying: extract_uniq_mutations +
  * perform_mutations + slice_sparse_mat + extract_current_sub_likelihood + eval_all_sub_likelihood
  * (CL:1417-1431).  Refreshes the coordinates / full likelihood like the head of step_sampler. */

@@ -25,6 +25,7 @@ EXPORTS = (
            "ig_run_cycle_device", "ig_get_cycle_plan", "ig_timeline_reset", "ig_timeline_get", "ig_timeline_blocks", "ig_timeline_phases",
     "ig_selftest_math", "ig_get_nuisance_stats", "ig_clone", "ig_run_cycles_device_multi", "ig_run_cycle_device_async", "ig_cycle_wait",
     "ig_bin_contacts", "ig_nccl_unique_id", "ig_nccl_init", "ig_allgather_best", "ig_get_gathered_state", "ig_nccl_finalize",
+    "ig_set_device_nuisance", "ig_get_nuisance_records",
 )
 
 
@@ -55,6 +56,10 @@ class ig_cycle_step(C.Structure):
 
 CYCLE_DTYPE = [("likelihood", "<f8"), ("lnz_full", "<f8"), ("dist", "<f8"), ("sum_l_cont", "<i8"), ("n_contigs", "<i4"),
                ("op_sampled", "<i4"), ("id_f_sampled", "<i4"), ("cand_index", "<i4"), ("n_proposals", "<i4"), ("q4_hits", "<i4")]
+
+# ig_nuisance_step (80 B): one device nuisance step of a production-mode cycle
+NUIS_DTYPE = [("likelihood_nuis", "<f8"), ("likelihood_t_after", "<f8"), ("u", "<f8"), ("draw", "<f8"), ("p_test", "<f4", (8,)),
+              ("id_modif", "<i4"), ("accepted", "<i4"), ("valid", "<i4"), ("pad", "<i4")]
 
 _lib = None
 
@@ -114,6 +119,8 @@ def lib():
         L.ig_get_gathered_state.argtypes = [vp, i32, vp]
         L.ig_nccl_finalize.argtypes = [vp]
         L.ig_selftest_math.argtypes = [vp, i32, C.c_float, C.c_float, C.c_float, vp]
+        L.ig_set_device_nuisance.argtypes = [vp, i32]
+        L.ig_get_nuisance_records.argtypes = [vp, i32, vp]
         for name in EXPORTS:
             if name not in ("ig_destroy", "ig_last_error"):
                 getattr(L, name).restype = C.c_int

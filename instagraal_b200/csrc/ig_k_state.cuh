@@ -9,7 +9,8 @@ __global__ void __launch_bounds__(IG_THREADS)
 k_coords(const FragRec* __restrict__ live, const SubRec* __restrict__ sub, CoordRec* __restrict__ coord,
          int* __restrict__ clen, int ns, const DevScalars* __restrict__ sc, float mbar, int use_test,
          double* __restrict__ part_z, int* __restrict__ part_n, int write_coords, SubX* __restrict__ subx,
-         unsigned char* __restrict__ row_dirty) {
+         unsigned char* __restrict__ row_dirty, const int* __restrict__ pred = nullptr) {
+    if (pred && !*pred) return;   // step kind 3: only after an accepted nuisance proposal
     TL(13);
     __shared__ double sm[32];
     __shared__ int sn;
@@ -192,7 +193,8 @@ __global__ void __launch_bounds__(IG_THREADS)
 k_lnz_refresh(const long long* __restrict__ row_ptr, const int2* __restrict__ cv, const CoordRec* __restrict__ coord,
               const int* __restrict__ clen, int ns, const DevScalars* __restrict__ sc, float mbar, int use_test,
               const float* __restrict__ exz_tab, int2* __restrict__ rec, unsigned char* __restrict__ row_dirty, int dp_bits,
-              double* __restrict__ part) {
+              double* __restrict__ part, const int* __restrict__ pred = nullptr) {
+    if (pred && !*pred) return;
     TL(14);
     __shared__ double sm[32];
     const Params p = use_test ? sc->p_test : sc->p;
@@ -244,7 +246,9 @@ k_lnz_refresh(const long long* __restrict__ row_ptr, const int2* __restrict__ cv
 
 __global__ void __launch_bounds__(IG_THREADS, 4)
 k_lnz_stream(const int4* __restrict__ rec2, long long n_pairs, int n_pad, double val_total, const DevScalars* __restrict__ sc,
-             int use_test, const float* __restrict__ exz_tab, int dp_bits, double* __restrict__ part) {
+             int use_test, const float* __restrict__ exz_tab, int dp_bits, double* __restrict__ part,
+             const int* __restrict__ pred = nullptr) {
+    if (pred && !*pred) return;
     TL(14);
     __shared__ double sm[32];
     __shared__ LnzQ queue[IG_WARPS_PER_BLOCK][IG_LNZ_QCAP];
@@ -306,7 +310,10 @@ k_lnz_stream(const int4* __restrict__ rec2, long long n_pairs, int n_pad, double
 }
 
 // generic deterministic final reduction of `n` doubles (and optionally ints) by one block
-__global__ void k_reduce(const double* __restrict__ part, int n, double* out, const int* __restrict__ ipart, int* iout) {
+// pred (all four kernels above too): when given, the kernel returns at once while *pred == 0
+__global__ void k_reduce(const double* __restrict__ part, int n, double* out, const int* __restrict__ ipart, int* iout,
+                         const int* __restrict__ pred = nullptr) {
+    if (pred && !*pred) return;
     __shared__ double sm[32];
     __shared__ int smi;
     if (threadIdx.x == 0) smi = 0;

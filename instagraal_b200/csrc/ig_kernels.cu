@@ -95,6 +95,11 @@ struct DevScalars {
     // streaming scoring path of large levels: which candidates take it, overflow of a pick list
     int use_stream[IG_MAX_CANDS];
     int list_overflow, pad2_;
+    // production-mode nuisance step (ig_k_nuis.cuh): the key and cycle of the cycle being run, the proposal in flight, and
+    // the flag that tells the next step (kind 3) that its likelihood sums are stale (the proposal was accepted)
+    unsigned nuis_key_lo, nuis_key_hi, nuis_cycle;
+    int nuis_id, nuis_valid, nuis_stale;
+    double nuis_u, nuis_draw;
 };
 
 struct CycleOut {  // compact per-step record of ig_run_cycle (128 B)
@@ -112,6 +117,8 @@ struct CycleOut {  // compact per-step record of ig_run_cycle (128 B)
 #include "ig_k_flat.cuh"   // flat scoring path of small levels: k_pick + k_eval_flat
 #include "ig_k_finish.cuh"   // finalisation, move selection, incremental maintenance, apply, contig bookkeeping, histogram, thumbnail
 #include "ig_k_rng.cuh"   // production RNG mode: Philox4x32-10 neighbour draws of a whole cycle
+#include "ig_k_nuis.cuh"   // production RNG mode: the nuisance-parameter step after every step of a cycle
+static_assert(sizeof(ig_nuisance_step) == 80, "ig_nuisance_step is 80 bytes (NUIS_DTYPE in _lib.py)");
 
 // ================================================================================================
 // host side
@@ -174,7 +181,12 @@ struct ig_handle {
     double* part_out;
     int gs_div, sparse_div, grid_split;
     long long last_n_full;
-    cudaGraphExec_t graph[6][IG_MAX_CANDS + 1];   // [step kind + 3 * cycle][candidates in the grid]
+    cudaGraphExec_t graph[8][IG_MAX_CANDS + 1];   // [step kind + 4 * cycle][candidates in the grid]
+    // production-mode nuisance step (ig_set_device_nuisance): one graph per handle replayed after every plan step, the
+    // per-step records (cyc_cap of them), and whether a nuisance step was enqueued since the plan began
+    bool nuis_on = false, nuis_enqueued = false, nuis_graph_dev_failed = false;
+    cudaGraphExec_t graph_nuis_dev = nullptr;
+    ig_nuisance_step* nuis_rec = nullptr;
     int* cyc_in; CycleOut* cyc_out; int cyc_cap; bool graph_failed, capturing, use_graph; long long n_full;
     int pending_steps;   // steps enqueued by an asynchronous cycle call and not collected yet
     // measurement (CUDA events on the launching stream)
@@ -498,9 +510,11 @@ extern "C" void ig_destroy(ig_handle* h) {
     if (h->h_p8) cudaFreeHost(h->h_p8);
     if (h->d_p8) cudaFree(h->d_p8);
     if (h->graph_nuis) cudaGraphExecDestroy(h->graph_nuis);
+    if (h->graph_nuis_dev) cudaGraphExecDestroy(h->graph_nuis_dev);
+    if (h->nuis_rec) cudaFree(h->nuis_rec);
     for (int i = 0; i < 6; i++) if (h->ev[i]) cudaEventDestroy(h->ev[i]);
     for (int i = 0; i < 16; i++) if (h->evk[i]) cudaEventDestroy(h->evk[i]);
-    for (int i = 0; i < 6; i++) for (int j = 0; j <= IG_MAX_CANDS; j++) if (h->graph[i][j]) cudaGraphExecDestroy(h->graph[i][j]);
+    for (int i = 0; i < 8; i++) for (int j = 0; j <= IG_MAX_CANDS; j++) if (h->graph[i][j]) cudaGraphExecDestroy(h->graph[i][j]);
     if (h->cyc_in) cudaFree(h->cyc_in);
     if (h->cyc_out) cudaFree(h->cyc_out);
     if (h->side) cudaStreamDestroy(h->side);
@@ -787,23 +801,26 @@ static int enqueue_step(ig_handle* h, int full, int n_grid_cands, int cycle = 0)
         L.cnt = c;
         k_prefetch_l2<<<h->n_part_zc, 256, 0, h->pf>>>(L);
     }
-    if (full == 2) {
+    if (full == 2 || full == 3) {
         // parameters changed, scaffold bookkeeping intact (an accepted nuisance proposal): coordinates as in the incremental
         // step (k_commit_coords flags the rows of the previous move), zero terms and the full non-zero likelihood recomputed
-        // under the new parameters -- the latter from the cached per-contact records (k_lnz_refresh + k_lnz_stream)
+        // under the new parameters -- the latter from the cached per-contact records (k_lnz_refresh + k_lnz_stream).
+        // Kind 3 (production-mode nuisance step): the same launches, but the recomputation only runs when the previous
+        // step's nuisance proposal was accepted (sc->nuis_stale); otherwise it is the incremental step, kind 0
+        const int* pred = full == 3 ? &h->sc->nuis_stale : nullptr;
         k_commit_coords<<<std::min(h->n_part_zc, (h->ns + 255) / 256), 256, 0, h->side>>>(h->coord, h->clen, h->sc, h->rows, h->ns,
                                                                                          h->table, h->table_len, h->live, h->sub, h->subx, h->row_dirty);
         k_coords<<<h->n_part_zc, IG_THREADS, 0, h->side>>>(h->live, h->sub, h->coord, h->clen, h->ns, h->sc, mbar, 0, h->part_zc,
-                                                          h->part_nc, 0, h->subx, nullptr);
-        k_reduce<<<1, 256, 0, h->side>>>(h->part_zc, h->n_part_zc, &h->sc->z_cur, h->part_nc, &h->sc->nintra_cur);
+                                                          h->part_nc, 0, h->subx, nullptr, pred);
+        k_reduce<<<1, 256, 0, h->side>>>(h->part_zc, h->n_part_zc, &h->sc->z_cur, h->part_nc, &h->sc->nintra_cur, pred);
         cudaEventRecord(h->ev_coords, h->side);
         if (h->profile && !h->capturing) cudaEventRecord(h->ev[2], h->side);
         k_lnz_refresh<<<h->grid_lnz, IG_THREADS, 0, h->side>>>(h->row_ptr, h->cv, h->coord, h->clen, h->ns, h->sc, mbar, 0, h->exz,
-                                                               h->lnz_rec, h->row_dirty, h->dp_bits, h->part_full + h->grid_lnz);
+                                                               h->lnz_rec, h->row_dirty, h->dp_bits, h->part_full + h->grid_lnz, pred);
         k_lnz_stream<<<h->grid_lnz, IG_THREADS, 0, h->side>>>(reinterpret_cast<const int4*>(h->lnz_rec), h->lnz_pairs, h->lnz_pad,
-                                                              h->lvl->val_total, h->sc, 0, h->exz, h->dp_bits, h->part_full);
+                                                              h->lvl->val_total, h->sc, 0, h->exz, h->dp_bits, h->part_full, pred);
         if (h->profile && !h->capturing) cudaEventRecord(h->ev[3], h->side);
-        k_reduce<<<1, 256, 0, h->side>>>(h->part_full, 2 * h->grid_lnz, &h->sc->lnz_full, nullptr, nullptr);
+        k_reduce<<<1, 256, 0, h->side>>>(h->part_full, 2 * h->grid_lnz, &h->sc->lnz_full, nullptr, nullptr, pred);
         cudaEventRecord(h->ev_lnz, h->side);
     } else if (full) {
         k_coords<<<h->n_part_zc, IG_THREADS, 0, h->side>>>(h->live, h->sub, h->coord, h->clen, h->ns, h->sc, mbar, 0, h->part_zc,
@@ -866,18 +883,19 @@ static int enqueue_step(ig_handle* h, int full, int n_grid_cands, int cycle = 0)
 #define IG_LAUNCHES_INCR 12
 #define IG_LAUNCHES_LITE 17
 // 0: incremental step; 1: coordinates and likelihood sums from scratch (scaffold replaced from outside, periodic refresh);
-// 2: likelihood sums only (parameters changed; needs the per-contact records and v_inter > 0, which the records assume)
+// 2: likelihood sums only (parameters changed; needs the per-contact records and v_inter > 0, which the records assume);
+// 3: kind 2 decided on the device (a step after a production-mode nuisance step: see enqueue_plan_step)
 static int step_kind(const ig_handle* h) {
     if (!h->incr_valid || (h->refresh_every > 0 && h->steps_since_full >= h->refresh_every)) return 1;
     if (h->lnz_stale) return (h->lnz_cache && h->vinter_pos) ? 2 : 1;
     return 0;
 }
 static int step_launches(const ig_handle* h, int kind) {
-    return (kind == 2 ? IG_LAUNCHES_LITE : kind ? IG_LAUNCHES_FULL : IG_LAUNCHES_INCR) - (h->rigid ? 1 : 0) + (h->prefetch ? 1 : 0) - (h->rows_small ? 1 : 0) + (h->flat ? 1 : 0) + (h->streaming ? 2 : 0);
+    return (kind >= 2 ? IG_LAUNCHES_LITE : kind ? IG_LAUNCHES_FULL : IG_LAUNCHES_INCR) - (h->rigid ? 1 : 0) + (h->prefetch ? 1 : 0) - (h->rows_small ? 1 : 0) + (h->flat ? 1 : 0) + (h->streaming ? 2 : 0);
 }
 
 static int get_graph(ig_handle* h, int full, cudaGraphExec_t* out, int cycle, int n) {
-    cudaGraphExec_t& ge = h->graph[full + 3 * cycle][n];
+    cudaGraphExec_t& ge = h->graph[full + 4 * cycle][n];
     if (!ge && !h->graph_failed) {
         cudaGraph_t g = nullptr;
         h->capturing = true;
@@ -947,10 +965,12 @@ static int cycle_buffers(ig_handle* h, int n_steps) {
         if (h->cyc_in) cudaFree(h->cyc_in);
         if (h->cyc_out) cudaFree(h->cyc_out);
         if (h->cyc_frags) cudaFree(h->cyc_frags);
-        h->cyc_in = nullptr; h->cyc_out = nullptr; h->cyc_frags = nullptr; h->cyc_cap = 0;
-        for (int i = 3; i < 6; i++) for (int j = 0; j <= IG_MAX_CANDS; j++) if (h->graph[i][j]) { cudaGraphExecDestroy(h->graph[i][j]); h->graph[i][j] = nullptr; }  // pointers are baked in
+        if (h->nuis_rec) cudaFree(h->nuis_rec);
+        h->cyc_in = nullptr; h->cyc_out = nullptr; h->cyc_frags = nullptr; h->nuis_rec = nullptr; h->cyc_cap = 0;
+        for (int i = 4; i < 8; i++) for (int j = 0; j <= IG_MAX_CANDS; j++) if (h->graph[i][j]) { cudaGraphExecDestroy(h->graph[i][j]); h->graph[i][j] = nullptr; }  // pointers are baked in
+        if (h->graph_nuis_dev) { cudaGraphExecDestroy(h->graph_nuis_dev); h->graph_nuis_dev = nullptr; }
         if (dev_alloc(h, &h->cyc_in, (size_t)n_steps * (2 + IG_MAX_CANDS)) || dev_alloc(h, &h->cyc_out, (size_t)n_steps) ||
-            dev_alloc(h, &h->cyc_frags, (size_t)n_steps)) return -2;
+            dev_alloc(h, &h->cyc_frags, (size_t)n_steps) || dev_alloc(h, &h->nuis_rec, (size_t)n_steps)) return -2;
         h->cyc_cap = n_steps;
     }
     return 0;
@@ -960,17 +980,59 @@ static int cycle_buffers(ig_handle* h, int n_steps) {
 // the stream); grid_n(t) = number of candidate slots the step's grid is built for
 // one step of the plan in h->cyc_in enqueued on the handle's stream (CUDA-graph replay); grid_n = number of candidate
 // slots the step's grid is built for
+// the nuisance step of the production mode (ig_k_nuis.cuh) after the step just enqueued: propose, evaluate the proposal
+// with exactly the launches of ig_full_likelihood(p_test, use_stale_coords = 1), decide, promote, record
+static void enqueue_nuisance(ig_handle* h) {
+    const float mbar = h->cfg.mean_sub_len_kb;
+    k_nuis_propose<<<1, 1, 0, h->stream>>>(h->sc);
+    k_exz_table<<<std::min(1024, (h->ns + 256) / 256), 256, 0, h->stream>>>(h->exz_test, h->ns + 1, h->sc, mbar, 1);
+    k_coords<<<h->n_part_zc, IG_THREADS, 0, h->stream>>>(h->live, h->sub, h->coord, h->clen, h->ns, h->sc, mbar, 1,
+                                                        h->part_zc, h->part_nc, 0, h->subx, h->row_dirty);
+    k_reduce<<<1, 256, 0, h->stream>>>(h->part_zc, h->n_part_zc, &h->sc->full_out[1], h->part_nc, &h->sc->full_nintra);
+    k_lnz_refresh<<<h->grid_lnz, IG_THREADS, 0, h->stream>>>(h->row_ptr, h->cv, h->coord, h->clen, h->ns, h->sc, mbar, 1, h->exz_test,
+                                                             h->lnz_rec, h->row_dirty, h->dp_bits, h->part_full + h->grid_lnz);
+    k_lnz_stream<<<h->grid_lnz, IG_THREADS, 0, h->stream>>>(reinterpret_cast<const int4*>(h->lnz_rec), h->lnz_pairs, h->lnz_pad,
+                                                            h->lvl->val_total, h->sc, 1, h->exz_test, h->dp_bits, h->part_full);
+    k_reduce<<<1, 256, 0, h->stream>>>(h->part_full, 2 * h->grid_lnz, &h->sc->full_out[0], nullptr, nullptr);
+    k_nuis_accept<<<1, 1, 0, h->stream>>>(h->sc, h->nuis_rec, h->cfg.n_pix);
+    k_nuis_copy_exz<<<std::min(1024, (h->ns + 258) / 256), 256, 0, h->stream>>>(h->exz, h->exz_test, h->ns + 3, h->sc);
+}
+#define IG_LAUNCHES_NUIS 9
+static int launch_nuisance(ig_handle* h) {
+    if (h->use_graph && !h->graph_nuis_dev && !h->nuis_graph_dev_failed) {
+        cudaGraph_t g = nullptr;
+        cudaError_t e = cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal);
+        if (e == cudaSuccess) {
+            enqueue_nuisance(h);
+            e = cudaStreamEndCapture(h->stream, &g);
+        }
+        if (e == cudaSuccess && g) e = cudaGraphInstantiate(&h->graph_nuis_dev, g, 0);
+        if (g) cudaGraphDestroy(g);
+        if (e != cudaSuccess || !h->graph_nuis_dev) { h->graph_nuis_dev = nullptr; h->nuis_graph_dev_failed = true; cudaGetLastError(); }
+    }
+    if (h->use_graph && h->graph_nuis_dev) { CK(cudaGraphLaunch(h->graph_nuis_dev, h->stream)); }
+    else enqueue_nuisance(h);
+    h->n_launches += IG_LAUNCHES_NUIS;
+    return launch_ok(h, "nuisance step");
+}
 static int enqueue_plan_step(ig_handle* h, int grid_n) {
     if (int rc = labels_guard(h)) return rc;
-    const int full = step_kind(h);
+    int full = step_kind(h);
+    // after a nuisance step of this plan the host cannot know whether the parameters changed: kind 3 decides on the device
+    if (full == 0 && h->nuis_on && h->nuis_enqueued) full = 3;
     cudaGraphExec_t ge = nullptr;
     if (h->use_graph) get_graph(h, full, &ge, 1, grid_n);
     if (ge) { CK(cudaGraphLaunch(ge, h->stream)); }
     else if (enqueue_step(h, full, grid_n, 1)) return -2;
-    h->steps_since_full = full ? 1 : h->steps_since_full + 1;
-    h->n_full += full ? 1 : 0;
+    const bool refresh = full == 1 || full == 2;
+    h->steps_since_full = refresh ? 1 : h->steps_since_full + 1;
+    h->n_full += refresh ? 1 : 0;
     h->incr_valid = true; h->lnz_stale = false;
     h->n_launches += step_launches(h, full);
+    if (h->nuis_on) {
+        if (int rc = launch_nuisance(h)) return rc;
+        h->nuis_enqueued = true;
+    }
     return 0;
 }
 static int begin_plan(ig_handle* h) {
@@ -990,6 +1052,18 @@ static int collect_plan(ig_handle* h, int n_steps, ig_cycle_step* out) {
     CK(cudaStreamSynchronize(h->stream));
     h->coords_fresh = false; h->coords_ever = true;
     h->pending_steps = 0;
+    if (h->nuis_on && h->nuis_enqueued) {
+        // the last step's nuisance decision: an accepted proposal leaves the sums stale for the next step (ig_step or the
+        // first step of the next cycle, both decided on the host: kind 2)
+        int stale = 0; Params p;
+        CK(cudaMemcpyAsync(&stale, &h->sc->nuis_stale, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaMemcpyAsync(&p, &h->sc->p, sizeof(Params), cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaMemsetAsync(&h->sc->nuis_stale, 0, sizeof(int), h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+        if (stale) h->lnz_stale = true;
+        h->vinter_pos = p.v_inter > 0.0f;   // (always: a proposal with v_inter <= 0 is never accepted)
+    }
+    h->nuis_enqueued = false;
     if (overflow) { h->err = "pick list of the streaming scoring path overflowed (IG_PICK_CAP)"; return -4; }
     float ms = 0.f;
     if (cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]) == cudaSuccess) h->ms_step += ms;
@@ -1018,6 +1092,8 @@ extern "C" int ig_run_cycle(ig_handle* h, int32_t n_steps, const int32_t* frags,
                             ig_cycle_step* out) {
     if (use(h)) return -1;
     if (!h->params_set) { h->err = "ig_run_cycle: parameters not set"; return -1; }
+    if (h->nuis_on) { h->err = "ig_run_cycle: the device nuisance step is on (it needs the seeded production mode, ig_run_cycle_device); "
+                                "turn it off with ig_set_device_nuisance(h, 0)"; return -1; }
     if (n_steps <= 0) return 0;
     std::vector<int> plan((size_t)n_steps * (2 + IG_MAX_CANDS), 0);
     for (int t = 0; t < n_steps; t++) {
@@ -1067,8 +1143,15 @@ static int prepare_device_plan(ig_handle* h, int32_t n_steps, const int32_t* fra
     if (h->nf < 2) { h->err = "ig_run_cycle_device: needs at least two fragments"; return -1; }
     if (h->pending_steps) { h->err = "ig_run_cycle_device: an asynchronous cycle is still pending (ig_cycle_wait)"; return -1; }
     for (int t = 0; t < n_steps; t++) if (frags[t] < 0 || frags[t] >= h->nf) { h->err = "ig_run_cycle_device: fragment out of range"; return -1; }
+    if (h->nuis_on && !(h->lnz_cache && h->vinter_pos)) {
+        h->err = "ig_run_cycle_device: the device nuisance step needs the per-contact likelihood records and v_inter > 0"; return -1;
+    }
     if (cycle_buffers(h, n_steps)) return -2;
     CK(cudaMemcpyAsync(h->cyc_frags, frags, sizeof(int) * (size_t)n_steps, cudaMemcpyHostToDevice, h->stream));
+    if (h->nuis_on) {
+        k_nuis_begin<<<1, 1, 0, h->stream>>>(h->sc, (unsigned)(seed & 0xffffffffu), (unsigned)(seed >> 32), cycle);
+        h->n_launches += 1;
+    }
     k_draw_plan<<<(n_steps + 127) / 128, 128, 0, h->stream>>>(h->cyc_in, h->cyc_frags, n_steps, n_neighbours, h->nf, h->lvl->nb_ptr, h->lvl->nb_idx,
                                                             h->lvl->nb_cdf, h->lvl->nb_nnz, (unsigned)(seed & 0xffffffffu), (unsigned)(seed >> 32), cycle);
     if (launch_ok(h, "draw_plan")) return -2;
@@ -1132,6 +1215,30 @@ extern "C" int ig_get_cycle_plan(ig_handle* h, int32_t n_steps, int32_t* out) {
     return 0;
 }
 
+extern "C" int ig_set_device_nuisance(ig_handle* h, int32_t on) {
+    if (use(h)) return -1;
+    if (h->pending_steps) { h->err = "ig_set_device_nuisance: an asynchronous cycle is still pending (ig_cycle_wait)"; return -1; }
+    if (on) {
+        if (!h->lnz_cache) {
+            h->err = "ig_set_device_nuisance: this handle has no per-contact likelihood records (IG_LNZ_CACHE=0, or a level whose "
+                     "counts / size do not fit them); the device nuisance step evaluates its proposals from them";
+            return -1;
+        }
+        if (!h->params_set) { h->err = "ig_set_device_nuisance: parameters not set (ig_set_params)"; return -1; }
+        if (!h->vinter_pos) { h->err = "ig_set_device_nuisance: the live v_inter must be > 0"; return -1; }
+    }
+    h->nuis_on = on != 0;
+    return 0;
+}
+extern "C" int ig_get_nuisance_records(ig_handle* h, int32_t n_steps, ig_nuisance_step* out) {
+    if (use(h)) return -1;
+    if (n_steps == 0) return 0;
+    if (n_steps < 0 || n_steps > h->cyc_cap || !h->nuis_rec) { h->err = "ig_get_nuisance_records: no such records"; return -1; }
+    CK(cudaMemcpyAsync(out, h->nuis_rec, sizeof(ig_nuisance_step) * (size_t)n_steps, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return 0;
+}
+
 // measurement / parity knobs: refresh_every = N -> recompute the coordinates and the full likelihood
 // over every contact at least every N steps (1 = every step, exactly the reference's schedule;
 // 0 = only when the state was changed from outside); use_graph = replay the step as one CUDA graph.
@@ -1151,7 +1258,8 @@ extern "C" int ig_set_gpu_share(ig_handle* h, int32_t share) {
     if (share < 1) { h->err = "ig_set_gpu_share: share must be >= 1"; return -1; }
     if (h->pending_steps) { h->err = "ig_set_gpu_share: an asynchronous cycle is still pending"; return -1; }
     CK(cudaStreamSynchronize(h->stream));
-    for (int i = 0; i < 6; i++) for (int j = 0; j <= IG_MAX_CANDS; j++) if (h->graph[i][j]) { cudaGraphExecDestroy(h->graph[i][j]); h->graph[i][j] = nullptr; }
+    for (int i = 0; i < 8; i++) for (int j = 0; j <= IG_MAX_CANDS; j++) if (h->graph[i][j]) { cudaGraphExecDestroy(h->graph[i][j]); h->graph[i][j] = nullptr; }
+    if (h->graph_nuis_dev) { cudaGraphExecDestroy(h->graph_nuis_dev); h->graph_nuis_dev = nullptr; }
     h->grid_score = std::max(8, h->grid_score_full / share);
     h->grid_flat = std::max(1, h->grid_score / 5);
     return 0;

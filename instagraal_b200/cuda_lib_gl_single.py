@@ -5,7 +5,8 @@ attributes, implemented over the C ABI of ``libinstagraal_b200.so`` through ctyp
 Mirrors (reference file:line):
   sampler.__init__            CL:92-319    -> ig_create (+ host-side neighbour pmfs, CL:3053-3101)
   step_sampler                CL:1401-1465 -> ig_step
-  step_nuisance_parameters    CL:2961-3051 -> ig_full_likelihood (+ host RNG / fsolve as in the reference)
+  step_nuisance_parameters    CL:2961-3051 -> ig_full_likelihood (+ host RNG / fsolve as in the reference);
+                              production RNG mode: run_cycle_device(nuisance=True) -> ig_set_device_nuisance (on the device)
   bomb_the_genome             CL:1925-1948 -> ig_bomb
   estimate_parameters_rippe   CL:2239-2372 -> ig_distance_histogram (+ scipy fit as in the reference)
   eval_likelihood / eval_all_sub_likelihood / test_copy_struct (step / eval / apply entry points)
@@ -37,6 +38,11 @@ ALL17 = ("pos", "sub_pos", "id_c", "start_bp", "len_bp", "sub_len", "circ", "id"
 PARAM_SIMU_RIPPE = np.dtype([("kuhn", np.float32), ("lm", np.float32), ("c1", np.float32), ("slope", np.float32),
                              ("d", np.float32), ("d_max", np.float32), ("fact", np.float32), ("v_inter", np.float32)],
                             align=True)  # CL:235-247
+# run_cycle_device(nuisance=True): the device record of every nuisance step, followed by the tuple step_nuisance_parameters
+# returns (IG:252; the list_* feeds of IG:291-330): the live parameters after the step, likelihood_t and success
+NUIS_STEP_DTYPE = np.dtype(L.NUIS_DTYPE[:-1] + [("fact", np.float32), ("d", np.float32), ("d_max", np.float32),
+                                                ("d_nuc", np.float32), ("slope", np.float32), ("likelihood_t", np.float64),
+                                                ("success", np.int32)])
 
 
 def _ptr(a):
@@ -182,6 +188,7 @@ class sampler:
         self._twin = None
         self._twin_synced = False
         self.n_nuis_overlapped = 0
+        self._nuis_device = False   # ig_set_device_nuisance state of the handle
         self.modification_str = [  # CL:1601-1620
             "eject frag", "flip frag", "pop out split insert @ left or 1", "pop out split insert @ left or -1",
             "pop out split insert @ right or 1", "pop out split insert @ right or -1", "pop out insert @ right or 1",
@@ -216,6 +223,7 @@ class sampler:
         s.n_proposals_scored = 0
         s.likelihood_t = None
         s._nuis_follows, s._spec, s._spec_pool, s._twin, s._twin_synced = False, None, None, None, False
+        s._nuis_device = False
         s._res = L.ig_step_result()
         s._res_scores = np.frombuffer(s._res, dtype=np.float64, count=L.IG_MAX_CANDS * L.IG_N_OPS, offset=L.ig_step_result.scores.offset)
         s._res_nuniq = np.frombuffer(s._res, dtype=np.int32, count=L.IG_MAX_CANDS, offset=L.ig_step_result.n_uniq.offset)
@@ -486,17 +494,61 @@ class sampler:
         cdf = np.ascontiguousarray(np.concatenate(cdf) if cdf else np.zeros(0, np.float64), dtype=np.float64)
         return ptr, idx, cdf, nnz
 
-    def run_cycle_device(self, list_frags, n_neighbours=5, seed=0, cycle=0):
+    def run_cycle_device(self, list_frags, n_neighbours=5, seed=0, cycle=0, nuisance=False):
         """Production RNG mode: like run_cycle, but every step's neighbours are drawn ON THE DEVICE (Philox4x32-10
         keyed by (seed, cycle, step, draw); same distribution as return_neighbours, a different random stream than
-        NumPy's).  The host only provides the visiting order (np.random.shuffle in full_em, IG:213)."""
+        NumPy's).  The host only provides the visiting order (np.random.shuffle in full_em, IG:213).
+
+        nuisance=True: every step is followed by step_nuisance_parameters (full_em from cycle 5 on, IG:242-252), also on
+        the device (ig_set_device_nuisance: Philox draws with the same seed, d_max by root finding, DESIGN.md D3).  Returns
+        (steps, nuis) with nuis a NUIS_STEP_DTYPE record per step; param_simu, param_simu_test and likelihood_t are left
+        where the device left them."""
         self._upload_neighbour_weights()
+        self.set_device_nuisance(nuisance)
         n = len(list_frags)
         frags = np.ascontiguousarray(list_frags, dtype=np.int32)
         out = np.zeros(n, dtype=L.CYCLE_DTYPE)
         L.check(self._h, L.lib().ig_run_cycle_device(self._h, n, _ptr(frags), int(n_neighbours), int(seed), int(cycle), _ptr(out)),
                 "ig_run_cycle_device")
         self._after_cycle(out)
+        if not nuisance:
+            return out
+        return out, self._after_nuisance(n)
+
+    def set_device_nuisance(self, on):
+        """ig_set_device_nuisance: run the nuisance step on the device after every step of run_cycle_device (and of
+        ReplicaSet.run_cycle)."""
+        on = bool(on)
+        if on != self._nuis_device:
+            L.check(self._h, L.lib().ig_set_device_nuisance(self._h, int(on)), "ig_set_device_nuisance")
+            self._nuis_device = on
+
+    def last_nuisance_records(self, n_steps):
+        """the raw ig_nuisance_step records of the last production-mode cycle (L.NUIS_DTYPE)"""
+        rec = np.zeros(int(n_steps), dtype=L.NUIS_DTYPE)
+        assert rec.dtype.itemsize == 80
+        L.check(self._h, L.lib().ig_get_nuisance_records(self._h, int(n_steps), _ptr(rec)), "ig_get_nuisance_records")
+        return rec
+
+    def _after_nuisance(self, n_steps):
+        """the records of the last cycle's device nuisance steps + the per-step tuple of step_nuisance_parameters; the host
+        copies of the parameters follow the device (no upload: the device already holds them)"""
+        rec = self.last_nuisance_records(n_steps)
+        out = np.zeros(len(rec), dtype=NUIS_STEP_DTYPE)
+        for k in rec.dtype.names[:-1]:
+            out[k] = rec[k]
+        p0 = np.array(list(self.param_simu[0]), dtype=np.float32)
+        acc = rec["accepted"] != 0
+        last = np.maximum.accumulate(np.where(acc, np.arange(len(rec)), -1))
+        live = np.where((last >= 0)[:, None], rec["p_test"][np.maximum(last, 0)], p0[None, :])
+        for k, i in (("fact", 6), ("d", 4), ("d_max", 5), ("d_nuc", 7), ("slope", 3)):
+            out[k] = live[:, i]
+        out["likelihood_t"] = rec["likelihood_t_after"]
+        out["success"] = rec["accepted"]
+        if len(rec):
+            self.param_simu = np.array([tuple(live[-1].tolist())], dtype=PARAM_SIMU_RIPPE)
+            self.param_simu_test = np.array([tuple(rec["p_test"][-1].tolist())], dtype=PARAM_SIMU_RIPPE)
+            self.likelihood_t = self.o = np.float64(rec["likelihood_t_after"][-1])
         return out
 
     def _upload_neighbour_weights(self):

@@ -66,13 +66,16 @@ class ReplicaSet:
             np.random.seed(int(seed0) + i)
             c.bomb_the_genome()
 
-    def run_cycle(self, frags_per_chain, n_neighbours=5, cycle=0):
+    def run_cycle(self, frags_per_chain, n_neighbours=5, cycle=0, nuisance=False):
         """frags_per_chain: int32[n_chains, n_steps] visiting orders.  Returns the structured per-step records
-        [n_chains, n_steps] (same fields as sampler.run_cycle_device)."""
+        [n_chains, n_steps] (same fields as sampler.run_cycle_device).  nuisance=True: every chain samples the p(s)
+        parameters after every step, on the device with its own seed (sampler.run_cycle_device(nuisance=True)); returns
+        (steps, nuis) with nuis [n_chains, n_steps] of sampler.NUIS_STEP_DTYPE."""
         frags = np.ascontiguousarray(frags_per_chain, dtype=np.int32)
         assert frags.ndim == 2 and frags.shape[0] == self.n
         for c in self.chains:
             c._upload_neighbour_weights()
+            c.set_device_nuisance(nuisance)
         n_steps = frags.shape[1]
         out = np.zeros((self.n, n_steps), dtype=L.CYCLE_DTYPE)
         rc = L.lib().ig_run_cycles_device_multi(self._handles, self.n, n_steps, _ptr(frags), int(n_neighbours), _ptr(self.seeds),
@@ -80,7 +83,9 @@ class ReplicaSet:
         L.check(None, rc, "ig_run_cycles_device_multi")
         for i, c in enumerate(self.chains):
             c._after_cycle(out[i])
-        return out
+        if not nuisance:
+            return out
+        return out, np.stack([c._after_nuisance(n_steps) for c in self.chains])
 
     def allgather(self):
         """-> (best global chain index, likelihood[n_ranks * n], n_contigs[n_ranks * n]); device ms accumulated in gather_ms"""
