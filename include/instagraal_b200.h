@@ -18,7 +18,9 @@ extern "C" {
 #define IG_N_FIELDS 13 /* pos, sub_pos, id_c, start_bp, len_bp, sub_len, circ, prev, next, l_cont,
                           sub_l_cont, l_cont_bp, ori  (struct frag, kernel_sparse_adapt.cu:40-58, minus
                           the inert id/rep/activ/id_d which the facade synthesises) */
-#define IG_MAX_CANDS 8
+#define IG_MAX_CANDS 8        /* candidates of one scoring pass (ig_step_result, ig_run_cycle plans) */
+#define IG_MAX_NEIGHBOURS 64  /* candidates of one step: steps of more than IG_MAX_CANDS are scored in passes of
+                                 IG_MAX_CANDS (ig_step_wide, ig_run_cycle_wide, ig_run_cycle_device) */
 #define IG_N_OPS 24
 
 typedef struct ig_handle ig_handle;
@@ -119,6 +121,20 @@ int ig_step(ig_handle* h, int32_t id_frag, const int32_t* cands, int32_t n_cands
  * synchronisation in between; cands8 = [n_steps][IG_MAX_CANDS] sorted candidates, n_cands = [n_steps]. */
 int ig_run_cycle(ig_handle* h, int32_t n_steps, const int32_t* frags, const int32_t* cands8, const int32_t* n_cands,
                  ig_cycle_step* out);
+/* Steps of up to IG_MAX_NEIGHBOURS candidates (the reference takes any --neighborhood).  The candidates are scored in
+ * passes of IG_MAX_CANDS; the move is the first index of the maximum over all of them (CL:1435-1446), as in ig_step.
+ * ig_step_wide: scores = [24 * n_cands] all_scores, n_uniq / n_sub = [n_cands]; the scalar fields of `out` are filled,
+ * cand_index is the index into the whole candidate list, and out->scores / n_uniq / n_sub hold the first IG_MAX_CANDS
+ * candidates' values.  n_cands <= IG_MAX_CANDS is ig_step.
+ * ig_run_cycle_wide: ig_run_cycle with cands = [n_steps][width] (width >= every n_cands[t], <= IG_MAX_NEIGHBOURS);
+ * ig_run_cycle is this call with width = IG_MAX_CANDS.
+ * ig_get_cycle_plan_wide: the plan of the last cycle as [n_steps][2 + width] (n_cands, fragment, candidates); fails when
+ * a step had more than width candidates. */
+int ig_step_wide(ig_handle* h, int32_t id_frag, const int32_t* cands, int32_t n_cands, ig_step_result* out, double* scores,
+                 int32_t* n_uniq, int32_t* n_sub);
+int ig_run_cycle_wide(ig_handle* h, int32_t n_steps, const int32_t* frags, const int32_t* cands, int32_t width,
+                      const int32_t* n_cands, ig_cycle_step* out);
+int ig_get_cycle_plan_wide(ig_handle* h, int32_t n_steps, int32_t width, int32_t* out /* [n_steps][2 + width] */);
 /* Production RNG mode (SURVEY 8b "RNG contract"): the neighbour draws of return_neighbours (CL:3103-3141) on the
  * device.  ig_set_neighbour_weights uploads setup_distri_frags (CL:3053-3101) as a CSR: for fragment f the
  * candidates idx[ptr[f]..ptr[f+1]) (f itself excluded), the running sum cdf of their probabilities pk and the
@@ -127,7 +143,7 @@ int ig_run_cycle(ig_handle* h, int32_t n_steps, const int32_t* frags, const int3
  * sorted, A dropped): no per-step host work at all.  ig_get_cycle_plan returns what was drawn. */
 int ig_set_neighbour_weights(ig_handle* h, const int64_t* ptr, const int32_t* idx, const double* cdf, const int32_t* n_nonzero);
 int ig_run_cycle_device(ig_handle* h, int32_t n_steps, const int32_t* frags, int32_t n_neighbours, uint64_t seed,
-                        uint32_t cycle, ig_cycle_step* out);
+                        uint32_t cycle, ig_cycle_step* out);   /* n_neighbours <= IG_MAX_NEIGHBOURS */
 int ig_get_cycle_plan(ig_handle* h, int32_t n_steps, int32_t* out /* [n_steps][2 + IG_MAX_CANDS] */);
 /* The nuisance-parameter step of the production RNG mode (step_nuisance_parameters, CL:2961-3051; full_em runs it after
  * every step_sampler from cycle 5 on, IG:242-252).  While on, ig_run_cycle_device, ig_run_cycles_device_multi and

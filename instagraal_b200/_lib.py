@@ -11,7 +11,8 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("IG_B200_LIB", os.path.join(_HERE, "libinstagraal_b200.so"))
 
-IG_MAX_CANDS = 8
+IG_MAX_CANDS = 8         # candidates of one scoring pass
+IG_MAX_NEIGHBOURS = 64   # candidates of one step (ig_step_wide, ig_run_cycle_wide, ig_run_cycle_device)
 IG_N_OPS = 24
 IG_N_FIELDS = 13
 FIELDS13 = ("pos", "sub_pos", "id_c", "start_bp", "len_bp", "sub_len", "circ", "prev", "next",
@@ -25,7 +26,7 @@ EXPORTS = (
            "ig_run_cycle_device", "ig_get_cycle_plan", "ig_timeline_reset", "ig_timeline_get", "ig_timeline_blocks", "ig_timeline_phases",
     "ig_selftest_math", "ig_get_nuisance_stats", "ig_clone", "ig_run_cycles_device_multi", "ig_run_cycle_device_async", "ig_cycle_wait",
     "ig_bin_contacts", "ig_nccl_unique_id", "ig_nccl_init", "ig_allgather_best", "ig_get_gathered_state", "ig_nccl_finalize",
-    "ig_set_device_nuisance", "ig_get_nuisance_records",
+    "ig_set_device_nuisance", "ig_get_nuisance_records", "ig_step_wide", "ig_run_cycle_wide", "ig_get_cycle_plan_wide",
 )
 
 
@@ -121,6 +122,9 @@ def lib():
         L.ig_selftest_math.argtypes = [vp, i32, C.c_float, C.c_float, C.c_float, vp]
         L.ig_set_device_nuisance.argtypes = [vp, i32]
         L.ig_get_nuisance_records.argtypes = [vp, i32, vp]
+        L.ig_step_wide.argtypes = [vp, i32, vp, i32, C.POINTER(ig_step_result), vp, vp, vp]
+        L.ig_run_cycle_wide.argtypes = [vp, i32, vp, vp, i32, vp, vp]
+        L.ig_get_cycle_plan_wide.argtypes = [vp, i32, i32, vp]
         for name in EXPORTS:
             if name not in ("ig_destroy", "ig_last_error"):
                 getattr(L, name).restype = C.c_int

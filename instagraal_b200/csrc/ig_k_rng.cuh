@@ -25,16 +25,19 @@ __device__ __forceinline__ double philox_uniform(unsigned step, unsigned cycle, 
     const unsigned long long bits = ((unsigned long long)r.x << 32) | r.y;
     return (double)(bits >> 11) * (1.0 / 9007199254740992.0);  // 53 bits -> [0, 1)
 }
-__global__ void k_draw_plan(int* __restrict__ plan, const int* __restrict__ frags, int n_steps, int delta, int nf,
-                            const long long* __restrict__ nb_ptr, const int* __restrict__ nb_idx, const double* __restrict__ nb_cdf,
-                            const int* __restrict__ nb_nnz, unsigned seed_lo, unsigned seed_hi, unsigned cycle) {
+// MAXC = the most draws a plan entry can hold, width = its number of candidate slots (plan stride 2 + width)
+template <int MAXC>
+__device__ __forceinline__ void draw_plan_step(int* __restrict__ plan, int width, const int* __restrict__ frags, int n_steps, int delta, int nf,
+                                               const long long* __restrict__ nb_ptr, const int* __restrict__ nb_idx,
+                                               const double* __restrict__ nb_cdf, const int* __restrict__ nb_nnz, unsigned seed_lo,
+                                               unsigned seed_hi, unsigned cycle) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n_steps) return;
     const uint2 key = make_uint2(seed_lo, seed_hi);
     const int a = frags[t];
     const long long b = nb_ptr[a], e = nb_ptr[a + 1];
     const int len = (int)(e - b);
-    int got[IG_MAX_CANDS];
+    int got[MAXC];
     int n = 0;
     if (len > 0) {
         const int n_max = min(delta, nb_nnz[a]);
@@ -76,9 +79,21 @@ __global__ void k_draw_plan(int* __restrict__ plan, const int* __restrict__ frag
     }
     // sorted, without A itself
     for (int i = 1; i < n; i++) { const int v = got[i]; int j = i - 1; while (j >= 0 && got[j] > v) { got[j + 1] = got[j]; j--; } got[j + 1] = v; }
-    int* p = plan + (size_t)t * (2 + IG_MAX_CANDS);
+    int* p = plan + (size_t)t * (2 + width);
     int m = 0;
     for (int i = 0; i < n; i++) if (got[i] != a) p[2 + m++] = got[i];
-    for (int i = m; i < IG_MAX_CANDS; i++) p[2 + i] = 0;
+    for (int i = m; i < width; i++) p[2 + i] = 0;
     p[0] = m; p[1] = a;
+}
+__global__ void k_draw_plan(int* __restrict__ plan, const int* __restrict__ frags, int n_steps, int delta, int nf,
+                            const long long* __restrict__ nb_ptr, const int* __restrict__ nb_idx, const double* __restrict__ nb_cdf,
+                            const int* __restrict__ nb_nnz, unsigned seed_lo, unsigned seed_hi, unsigned cycle) {
+    draw_plan_step<IG_MAX_CANDS>(plan, IG_MAX_CANDS, frags, n_steps, delta, nf, nb_ptr, nb_idx, nb_cdf, nb_nnz, seed_lo, seed_hi, cycle);
+}
+// plans of more than IG_MAX_CANDS neighbours (stride 2 + width, width <= IG_MAX_NEIGHBOURS): draw i has the counter
+// (t, cycle, i, attempt) of the narrow kernel, so a wide plan's first IG_MAX_CANDS draws are the narrow plan's
+__global__ void k_draw_plan_wide(int* __restrict__ plan, int width, const int* __restrict__ frags, int n_steps, int delta, int nf,
+                                 const long long* __restrict__ nb_ptr, const int* __restrict__ nb_idx, const double* __restrict__ nb_cdf,
+                                 const int* __restrict__ nb_nnz, unsigned seed_lo, unsigned seed_hi, unsigned cycle) {
+    draw_plan_step<IG_MAX_NEIGHBOURS>(plan, width, frags, n_steps, delta, nf, nb_ptr, nb_idx, nb_cdf, nb_nnz, seed_lo, seed_hi, cycle);
 }

@@ -118,6 +118,7 @@ struct CycleOut {  // compact per-step record of ig_run_cycle (128 B)
 #include "ig_k_finish.cuh"   // finalisation, move selection, incremental maintenance, apply, contig bookkeeping, histogram, thumbnail
 #include "ig_k_rng.cuh"   // production RNG mode: Philox4x32-10 neighbour draws of a whole cycle
 #include "ig_k_nuis.cuh"   // production RNG mode: the nuisance-parameter step after every step of a cycle
+#include "ig_k_wide.cuh"   // steps of more than IG_MAX_CANDS candidates: batch staging, running maximum, fix-ups
 static_assert(sizeof(ig_nuisance_step) == 80, "ig_nuisance_step is 80 bytes (NUIS_DTYPE in _lib.py)");
 
 // ================================================================================================
@@ -189,6 +190,12 @@ struct ig_handle {
     ig_nuisance_step* nuis_rec = nullptr;
     int* cyc_in; CycleOut* cyc_out; int cyc_cap; bool graph_failed, capturing, use_graph; long long n_full;
     int pending_steps;   // steps enqueued by an asynchronous cycle call and not collected yet
+    // steps of more than IG_MAX_CANDS candidates (ig_k_wide.cuh), allocated on first use: the wide record + its pinned mirror,
+    // the wide cycle plan ([cap][2 + plan_width]), and one graph per [step kind + 4 * cycle][number of batches]
+    WideStep *wide = nullptr, *h_wide = nullptr;
+    int* cyc_wide = nullptr; size_t cyc_wide_cap = 0;
+    int plan_width = IG_MAX_CANDS;   // candidate slots per entry of the last cycle's plan (> IG_MAX_CANDS: cyc_wide)
+    cudaGraphExec_t graph_wide[8][IG_MAX_BATCHES + 1] = {};
     // measurement (CUDA events on the launching stream)
     cudaEvent_t ev[6];
     cudaEvent_t evk[16]; double ms_k[16];  // per-kernel event timing of the main stream (profiling mode)
@@ -512,6 +519,10 @@ extern "C" void ig_destroy(ig_handle* h) {
     if (h->graph_nuis) cudaGraphExecDestroy(h->graph_nuis);
     if (h->graph_nuis_dev) cudaGraphExecDestroy(h->graph_nuis_dev);
     if (h->nuis_rec) cudaFree(h->nuis_rec);
+    if (h->wide) cudaFree(h->wide);
+    if (h->h_wide) cudaFreeHost(h->h_wide);
+    if (h->cyc_wide) cudaFree(h->cyc_wide);
+    for (int i = 0; i < 8; i++) for (int j = 0; j <= IG_MAX_BATCHES; j++) if (h->graph_wide[i][j]) cudaGraphExecDestroy(h->graph_wide[i][j]);
     for (int i = 0; i < 6; i++) if (h->ev[i]) cudaEventDestroy(h->ev[i]);
     for (int i = 0; i < 16; i++) if (h->evk[i]) cudaEventDestroy(h->evk[i]);
     for (int i = 0; i < 8; i++) for (int j = 0; j <= IG_MAX_CANDS; j++) if (h->graph[i][j]) cudaGraphExecDestroy(h->graph[i][j]);
@@ -781,10 +792,10 @@ static int fetch_result(ig_handle* h, int n, const int32_t* cands, ig_step_resul
 //             overlapped with the candidate setup on the main stream;
 //   full = 0: incremental refresh from the previous step's mutation table (same values up to f64
 //             summation order), O(rows of the last move).
-static int enqueue_step(ig_handle* h, int full, int n_grid_cands, int cycle = 0) {
+// head of a step: the side streams fork from the main stream, then the refresh or incremental commit of `full` runs on the
+// side stream (ev_coords / ev_lnz mark its coordinates and its likelihood sums)
+static void enqueue_head(ig_handle* h, int full) {
     const float mbar = h->cfg.mean_sub_len_kb;
-    const int n = n_grid_cands;
-    if (!cycle) cudaMemcpyAsync(&h->sc->n_cands, h->h_small, (2 + IG_MAX_CANDS) * sizeof(int), cudaMemcpyHostToDevice, h->stream);
     cudaEventRecord(h->ev_fork, h->stream);
     cudaStreamWaitEvent(h->side, h->ev_fork, 0);
     cudaStreamWaitEvent(h->pf, h->ev_fork, 0);
@@ -839,9 +850,15 @@ static int enqueue_step(ig_handle* h, int full, int n_grid_cands, int cycle = 0)
         cudaEventRecord(h->ev_coords, h->side);
         cudaEventRecord(h->ev_lnz, h->side);
     }
+}
+// one scoring pass over the candidates in sc (or in the cycle plan cyc_in): setup, row list, precompute, scoring, k_finalize
+// (do_select: with the move selection); wide_rescore: the re-score of a wide step's winning batch (k_wide_flip)
+static void enqueue_pass(ig_handle* h, int n, int first_flip_eject, const int* cyc_in, int do_select, bool wide_rescore = false) {
+    const float mbar = h->cfg.mean_sub_len_kb;
     const FragRec* live = h->live;
     IG_MARK(0);
-    k_cand_setup<<<1, 32, 0, h->stream>>>(live, h->sc, h->desc, h->cfg.max_bounds_insert, 1, cycle ? h->cyc_in : nullptr, h->streaming ? h->stream_rows_max : 0);
+    k_cand_setup<<<1, 32, 0, h->stream>>>(live, h->sc, h->desc, h->cfg.max_bounds_insert, first_flip_eject, cyc_in, h->streaming ? h->stream_rows_max : 0);
+    if (wide_rescore) k_wide_flip<<<1, 32, 0, h->stream>>>(h->sc, h->desc, h->wide);
     IG_MARK(1);
     k_find_cuts<<<(h->nf + 255) / 256, 256, 0, h->stream>>>(live, h->nf, h->sc, h->desc, h->clstab);
     cudaEventRecord(h->ev_cuts, h->stream);
@@ -856,8 +873,12 @@ static int enqueue_step(ig_handle* h, int full, int n_grid_cands, int cycle = 0)
     IG_MARK(6);
     k_finalize<<<n, 1024, 0, h->stream>>>(h->row_ptr, h->cv, h->coord, h->sc, h->desc, h->rows, h->rowidx, h->ns, h->row_cnt, h->table,
                                          h->table_len, mbar, h->exz, h->part_nz, h->part_c, h->flat ? h->grid_score : gsx, h->part_z, h->part_i,
-                                         h->grid_pre, h->cfg.n_pix, h->cfg.compat_last_block, h->d_nuniq, h->d_nsub, 1, gsx, h->flat ? 1 : 0);
+                                         h->grid_pre, h->cfg.n_pix, h->cfg.compat_last_block, h->d_nuniq, h->d_nsub, do_select, gsx, h->flat ? 1 : 0);
     IG_MARK(7);
+}
+// the move selected by the last pass: incremental maintenance beside it, apply, contig bookkeeping (+ the cycle record)
+static void enqueue_tail(ig_handle* h, int cycle) {
+    const float mbar = h->cfg.mean_sub_len_kb;
     IG_MARK(8);
     // independent of apply/post: runs beside them on the side stream, joined before the result copy
     cudaEventRecord(h->ev_sel, h->stream);
@@ -874,10 +895,40 @@ static int enqueue_step(ig_handle* h, int full, int n_grid_cands, int cycle = 0)
                                                        cycle ? h->cyc_out : nullptr, h->d_nuniq, h->d_nsub);
     IG_MARK(11);
     cudaStreamWaitEvent(h->stream, h->ev_out, 0);
+}
+static int enqueue_step(ig_handle* h, int full, int n_grid_cands, int cycle = 0) {
+    if (!cycle) cudaMemcpyAsync(&h->sc->n_cands, h->h_small, (2 + IG_MAX_CANDS) * sizeof(int), cudaMemcpyHostToDevice, h->stream);
+    enqueue_head(h, full);
+    enqueue_pass(h, n_grid_cands, 1, cycle ? h->cyc_in : nullptr, 1);
+    enqueue_tail(h, cycle);
     if (!cycle) {
         cudaMemcpyAsync(h->h_sc, h->sc, sizeof(DevScalars), cudaMemcpyDeviceToHost, h->stream);
     }
     return launch_ok(h, "enqueue_step");
+}
+// A step of n_batches * IG_MAX_CANDS candidate slots (ig_k_wide.cuh): the head once, one score-only pass per batch, the
+// winning batch scored again with the selecting tail.  Every pass is launched for a full batch (the grid of IG_MAX_CANDS
+// candidates, whatever the batch holds), so the re-score repeats its batch's pass launch for launch and its scores, hence
+// its selection, are bit-identical to that pass's.  The candidates come from the cycle plan cyc_wide (cycle) or h->wide->in.
+static int enqueue_wide_step(ig_handle* h, int full, int n_batches, int cycle) {
+    const int* plan = cycle ? h->cyc_wide : nullptr;
+    const int width = h->plan_width;
+    if (!cycle) cudaMemcpyAsync(h->wide->in, h->h_wide->in, sizeof(h->wide->in), cudaMemcpyHostToDevice, h->stream);
+    enqueue_head(h, full);
+    for (int b = 0; b < n_batches; b++) {
+        k_wide_stage<<<1, 32, 0, h->stream>>>(h->sc, h->wide, plan, width, b);
+        enqueue_pass(h, IG_MAX_CANDS, b == 0 ? 1 : 0, nullptr, 0);
+        k_wide_stash<<<1, 256, 0, h->stream>>>(h->sc, h->wide, b);
+    }
+    k_wide_pick<<<1, 32, 0, h->stream>>>(h->sc, h->wide, plan, width);
+    enqueue_pass(h, IG_MAX_CANDS, 1, nullptr, 1, true);
+    enqueue_tail(h, cycle);
+    k_wide_finish<<<1, 32, 0, h->stream>>>(h->sc, h->wide, cycle ? h->cyc_out : nullptr);
+    if (!cycle) {
+        cudaMemcpyAsync(h->h_sc, h->sc, sizeof(DevScalars), cudaMemcpyDeviceToHost, h->stream);
+        cudaMemcpyAsync(h->h_wide, h->wide, sizeof(WideStep), cudaMemcpyDeviceToHost, h->stream);
+    }
+    return launch_ok(h, "enqueue_wide_step");
 }
 #define IG_LAUNCHES_FULL 15
 #define IG_LAUNCHES_INCR 12
@@ -911,6 +962,44 @@ static int get_graph(ig_handle* h, int full, cudaGraphExec_t* out, int cycle, in
     }
     *out = ge;
     return 0;
+}
+
+// wide steps: one graph per (kind, cycle, number of batches), in a cache of their own
+static int get_wide_graph(ig_handle* h, int full, cudaGraphExec_t* out, int cycle, int n_batches) {
+    cudaGraphExec_t& ge = h->graph_wide[full + 4 * cycle][n_batches];
+    if (!ge && !h->graph_failed) {
+        cudaGraph_t g = nullptr;
+        h->capturing = true;
+        cudaError_t e = cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal);
+        if (e == cudaSuccess) {
+            enqueue_wide_step(h, full, n_batches, cycle);
+            e = cudaStreamEndCapture(h->stream, &g);
+        }
+        h->capturing = false;
+        if (e == cudaSuccess && g) e = cudaGraphInstantiate(&ge, g, 0);
+        if (g) cudaGraphDestroy(g);
+        if (e != cudaSuccess || !ge) { ge = nullptr; h->graph_failed = true; cudaGetLastError(); }
+    }
+    *out = ge;
+    return 0;
+}
+static void destroy_wide_graphs(ig_handle* h, int first_kind_slot) {
+    for (int i = first_kind_slot; i < 8; i++)
+        for (int j = 0; j <= IG_MAX_BATCHES; j++) if (h->graph_wide[i][j]) { cudaGraphExecDestroy(h->graph_wide[i][j]); h->graph_wide[i][j] = nullptr; }
+}
+static int wide_alloc(ig_handle* h) {
+    if (h->wide) return 0;
+    if (dev_alloc(h, &h->wide, 1)) return -2;
+    CK(cudaMallocHost((void**)&h->h_wide, sizeof(WideStep)));
+    memset(h->h_wide, 0, sizeof(WideStep));
+    return 0;
+}
+static int n_batches_of(int n) { return (n + IG_MAX_CANDS - 1) / IG_MAX_CANDS; }
+// launches of a wide step: the narrow step's, plus one pass and the two wide kernels around it per batch, plus the re-score's
+// k_wide_pick / k_wide_flip and k_wide_finish
+static int wide_step_launches(const ig_handle* h, int kind, int n_batches) {
+    const int pass = step_launches(h, 0) - 3 - (h->rigid ? 0 : 1) - (h->prefetch ? 1 : 0);   // minus k_commit_coords, tail, prefetch
+    return step_launches(h, kind) + n_batches * (pass + 2) + 3;
 }
 
 extern "C" int ig_step(ig_handle* h, int32_t id_frag, const int32_t* cands, int32_t n_cands, ig_step_result* out) {
@@ -955,6 +1044,64 @@ extern "C" int ig_step(ig_handle* h, int32_t id_frag, const int32_t* cands, int3
     return 0;
 }
 
+// step_sampler with more than IG_MAX_CANDS candidates (enqueue_wide_step); up to IG_MAX_CANDS it is ig_step
+extern "C" int ig_step_wide(ig_handle* h, int32_t id_frag, const int32_t* cands, int32_t n_cands, ig_step_result* out, double* scores,
+                            int32_t* n_uniq, int32_t* n_sub) {
+    if (use(h)) return -1;
+    if (!out || !cands) { h->err = "ig_step_wide: null argument"; return -1; }
+    if (n_cands <= 0 || n_cands > IG_MAX_NEIGHBOURS) { h->err = "ig_step_wide: n_cands out of range (1 .. IG_MAX_NEIGHBOURS = 64)"; return -1; }
+    if (n_cands <= IG_MAX_CANDS) {
+        if (int rc = ig_step(h, id_frag, cands, n_cands, out)) return rc;
+        for (int i = 0; i < n_cands * IG_N_OPS; i++) if (scores) scores[i] = out->scores[i];
+        for (int i = 0; i < n_cands; i++) { if (n_uniq) n_uniq[i] = out->n_uniq[i]; if (n_sub) n_sub[i] = out->n_sub[i]; }
+        return 0;
+    }
+    if (!h->params_set) { h->err = "ig_step_wide: parameters not set (ig_set_params)"; return -1; }
+    if (id_frag < 0 || id_frag >= h->nf) { h->err = "id_frag out of range"; return -1; }
+    for (int i = 0; i < n_cands; i++) if (cands[i] < 0 || cands[i] >= h->nf) { h->err = "candidate out of range"; return -1; }
+    for (int i = 0; i < n_cands; i++) if (cands[i] == id_frag) { h->err = "candidate equals the visited fragment (reference quirk Q4; see DESIGN.md D1)"; return -1; }
+    if (int rc = wide_alloc(h)) return rc;
+    if (int rc = labels_guard(h)) return rc;
+    int* in = h->h_wide->in;
+    in[0] = n_cands; in[1] = id_frag;
+    for (int i = 0; i < IG_MAX_NEIGHBOURS; i++) in[2 + i] = i < n_cands ? cands[i] : 0;
+    const int full = step_kind(h);
+    const int nb = n_batches_of(n_cands);
+    cudaGraphExec_t ge = nullptr;
+    if (h->use_graph && !h->profile) get_wide_graph(h, full, &ge, 0, nb);
+    cudaEventRecord(h->ev[0], h->stream);
+    if (ge) {
+        CK(cudaGraphLaunch(ge, h->stream));
+    } else {
+        if (enqueue_wide_step(h, full, nb, 0)) return -2;
+    }
+    cudaEventRecord(h->ev[1], h->stream);
+    CK(cudaStreamSynchronize(h->stream));
+    h->n_launches += wide_step_launches(h, full, nb);
+    h->steps_since_full = full ? 1 : h->steps_since_full + 1;
+    h->n_full += full ? 1 : 0;
+    h->incr_valid = true; h->lnz_stale = false;
+    h->coords_fresh = false; h->coords_ever = true;
+    const DevScalars& sres = *h->h_sc;
+    const WideStep& w = *h->h_wide;
+    if (sres.list_overflow) { h->err = "pick list of the streaming scoring path overflowed (IG_PICK_CAP)"; return -4; }
+    memset(out, 0, sizeof *out);
+    for (int i = 0; i < IG_MAX_CANDS * IG_N_OPS; i++) out->scores[i] = w.scores[i];
+    for (int i = 0; i < IG_MAX_CANDS; i++) { out->n_uniq[i] = w.n_uniq[i]; out->n_sub[i] = w.n_sub[i]; }
+    if (scores) for (int i = 0; i < n_cands * IG_N_OPS; i++) scores[i] = w.scores[i];
+    for (int i = 0; i < n_cands; i++) { if (n_uniq) n_uniq[i] = w.n_uniq[i]; if (n_sub) n_sub[i] = w.n_sub[i]; }
+    out->lnz_full = sres.lnz_full; out->q4_hits = sres.q4_hits;
+    out->likelihood = sres.likelihood;
+    out->cand_index = w.win_cand; out->op_sampled = sres.win_op;
+    out->id_f_sampled = cands[w.win_cand];
+    out->n_contigs = sres.n_heads; out->sum_l_cont = sres.sum_l_cont;
+    out->dist = (3.0 * h->nf - 0.5 * (double)sres.dist_half) / (3.0 * h->nf);
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]) == cudaSuccess) h->ms_step += ms;
+    h->n_steps++;
+    return 0;
+}
+
 // A whole MCMC cycle (or any run of steps) enqueued without a single host synchronisation in between:
 // the host uploads the plan {fragment, sorted candidates} of every step (drawn with the reference's own
 // RNG calls, which do not depend on the chain state), every step is one CUDA-graph replay that reads its
@@ -968,11 +1115,26 @@ static int cycle_buffers(ig_handle* h, int n_steps) {
         if (h->nuis_rec) cudaFree(h->nuis_rec);
         h->cyc_in = nullptr; h->cyc_out = nullptr; h->cyc_frags = nullptr; h->nuis_rec = nullptr; h->cyc_cap = 0;
         for (int i = 4; i < 8; i++) for (int j = 0; j <= IG_MAX_CANDS; j++) if (h->graph[i][j]) { cudaGraphExecDestroy(h->graph[i][j]); h->graph[i][j] = nullptr; }  // pointers are baked in
+        destroy_wide_graphs(h, 4);
         if (h->graph_nuis_dev) { cudaGraphExecDestroy(h->graph_nuis_dev); h->graph_nuis_dev = nullptr; }
         if (dev_alloc(h, &h->cyc_in, (size_t)n_steps * (2 + IG_MAX_CANDS)) || dev_alloc(h, &h->cyc_out, (size_t)n_steps) ||
             dev_alloc(h, &h->cyc_frags, (size_t)n_steps) || dev_alloc(h, &h->nuis_rec, (size_t)n_steps)) return -2;
         h->cyc_cap = n_steps;
     }
+    return 0;
+}
+// the plan of a wide cycle: [n_steps][2 + width] (the stride is baked into the cycle graphs of wide steps)
+static int wide_plan_buffers(ig_handle* h, int n_steps, int width) {
+    if (int rc = wide_alloc(h)) return rc;
+    const size_t need = (size_t)n_steps * (2 + width);
+    if (need > h->cyc_wide_cap || width != h->plan_width) destroy_wide_graphs(h, 4);
+    if (need > h->cyc_wide_cap) {
+        if (h->cyc_wide) cudaFree(h->cyc_wide);
+        h->cyc_wide = nullptr; h->cyc_wide_cap = 0;
+        if (dev_alloc(h, &h->cyc_wide, need)) return -2;
+        h->cyc_wide_cap = need;
+    }
+    h->plan_width = width;
     return 0;
 }
 
@@ -1015,20 +1177,29 @@ static int launch_nuisance(ig_handle* h) {
     h->n_launches += IG_LAUNCHES_NUIS;
     return launch_ok(h, "nuisance step");
 }
+// grid_n > IG_MAX_CANDS: a wide step of n_batches_of(grid_n) batches from the wide plan
 static int enqueue_plan_step(ig_handle* h, int grid_n) {
     if (int rc = labels_guard(h)) return rc;
     int full = step_kind(h);
     // after a nuisance step of this plan the host cannot know whether the parameters changed: kind 3 decides on the device
     if (full == 0 && h->nuis_on && h->nuis_enqueued) full = 3;
     cudaGraphExec_t ge = nullptr;
-    if (h->use_graph) get_graph(h, full, &ge, 1, grid_n);
-    if (ge) { CK(cudaGraphLaunch(ge, h->stream)); }
-    else if (enqueue_step(h, full, grid_n, 1)) return -2;
+    if (grid_n > IG_MAX_CANDS) {
+        const int nb = n_batches_of(grid_n);
+        if (h->use_graph) get_wide_graph(h, full, &ge, 1, nb);
+        if (ge) { CK(cudaGraphLaunch(ge, h->stream)); }
+        else if (enqueue_wide_step(h, full, nb, 1)) return -2;
+        h->n_launches += wide_step_launches(h, full, nb);
+    } else {
+        if (h->use_graph) get_graph(h, full, &ge, 1, grid_n);
+        if (ge) { CK(cudaGraphLaunch(ge, h->stream)); }
+        else if (enqueue_step(h, full, grid_n, 1)) return -2;
+        h->n_launches += step_launches(h, full);
+    }
     const bool refresh = full == 1 || full == 2;
     h->steps_since_full = refresh ? 1 : h->steps_since_full + 1;
     h->n_full += refresh ? 1 : 0;
     h->incr_valid = true; h->lnz_stale = false;
-    h->n_launches += step_launches(h, full);
     if (h->nuis_on) {
         if (int rc = launch_nuisance(h)) return rc;
         h->nuis_enqueued = true;
@@ -1044,10 +1215,12 @@ static int begin_plan(ig_handle* h) {
 static int collect_plan(ig_handle* h, int n_steps, ig_cycle_step* out) {
     cudaEventRecord(h->ev[1], h->stream);
     std::vector<CycleOut> res(n_steps);
-    std::vector<int> plan((size_t)n_steps * (2 + IG_MAX_CANDS));
+    const int stride = 2 + h->plan_width;   // wide cycles: the wide plan holds every step
+    std::vector<int> plan((size_t)n_steps * stride);
     int overflow = 0;
     CK(cudaMemcpyAsync(res.data(), h->cyc_out, sizeof(CycleOut) * n_steps, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaMemcpyAsync(plan.data(), h->cyc_in, plan.size() * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(plan.data(), h->plan_width > IG_MAX_CANDS ? h->cyc_wide : h->cyc_in, plan.size() * sizeof(int),
+                       cudaMemcpyDeviceToHost, h->stream));
     CK(cudaMemcpyAsync(&overflow, &h->sc->list_overflow, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     h->coords_fresh = false; h->coords_ever = true;
@@ -1070,14 +1243,15 @@ static int collect_plan(ig_handle* h, int n_steps, ig_cycle_step* out) {
     h->n_steps += n_steps;
     for (int t = 0; t < n_steps; t++) {
         const CycleOut& r = res[t];
-        const int* pl = &plan[(size_t)t * (2 + IG_MAX_CANDS)];
+        const int* pl = &plan[(size_t)t * stride];
         ig_cycle_step& o = out[t];
         o.likelihood = r.likelihood; o.lnz_full = r.lnz_full;
         o.dist = (3.0 * h->nf - 0.5 * (double)r.dist_half) / (3.0 * h->nf);
         o.sum_l_cont = r.sum_l_cont; o.n_contigs = r.n_heads; o.op_sampled = r.win_op; o.cand_index = r.win_cand;
         o.id_f_sampled = pl[2 + r.win_cand];
         o.q4_hits = r.q4_hits; o.n_proposals = 0;
-        for (int i = 0; i < pl[0]; i++) o.n_proposals += r.n_uniq[i];
+        if (r.pad[1]) o.n_proposals = r.pad[0];   // a wide step (k_wide_finish): every batch's proposals
+        else for (int i = 0; i < pl[0]; i++) o.n_proposals += r.n_uniq[i];
     }
     return 0;
 }
@@ -1090,25 +1264,54 @@ static int run_plan(ig_handle* h, int n_steps, GridN grid_n, ig_cycle_step* out)
 
 extern "C" int ig_run_cycle(ig_handle* h, int32_t n_steps, const int32_t* frags, const int32_t* cands8, const int32_t* n_cands,
                             ig_cycle_step* out) {
+    return ig_run_cycle_wide(h, n_steps, frags, cands8, IG_MAX_CANDS, n_cands, out);
+}
+// cands = [n_steps][width].  A cycle whose steps all have at most IG_MAX_CANDS candidates runs from the narrow plan (cyc_in);
+// otherwise the wide plan (stride 2 + width) holds every step, steps of more than IG_MAX_CANDS candidates run as wide steps and
+// the others as narrow steps from the narrow plan, which then holds their entries (both plans are read at entry step_idx)
+extern "C" int ig_run_cycle_wide(ig_handle* h, int32_t n_steps, const int32_t* frags, const int32_t* cands, int32_t width,
+                                 const int32_t* n_cands, ig_cycle_step* out) {
     if (use(h)) return -1;
     if (!h->params_set) { h->err = "ig_run_cycle: parameters not set"; return -1; }
     if (h->nuis_on) { h->err = "ig_run_cycle: the device nuisance step is on (it needs the seeded production mode, ig_run_cycle_device); "
                                 "turn it off with ig_set_device_nuisance(h, 0)"; return -1; }
+    if (width <= 0 || width > IG_MAX_NEIGHBOURS) { h->err = "ig_run_cycle: width out of range (1 .. IG_MAX_NEIGHBOURS = 64)"; return -1; }
     if (n_steps <= 0) return 0;
+    int n_max = 0;
+    for (int t = 0; t < n_steps; t++) {
+        const int n = n_cands[t];
+        if (n > width) { h->err = "ig_run_cycle: a step has more candidates than the width of the candidate array"; return -1; }
+        if (n <= 0 || frags[t] < 0 || frags[t] >= h->nf) { h->err = "ig_run_cycle: bad plan entry"; return -1; }
+        for (int i = 0; i < n; i++) {
+            const int c = cands[(size_t)t * width + i];
+            if (c < 0 || c >= h->nf || c == frags[t]) { h->err = "ig_run_cycle: candidate out of range or equal to the visited fragment"; return -1; }
+        }
+        n_max = std::max(n_max, n);
+    }
+    const bool wide = n_max > IG_MAX_CANDS;
     std::vector<int> plan((size_t)n_steps * (2 + IG_MAX_CANDS), 0);
     for (int t = 0; t < n_steps; t++) {
         const int n = n_cands[t];
-        if (n <= 0 || n > IG_MAX_CANDS || frags[t] < 0 || frags[t] >= h->nf) { h->err = "ig_run_cycle: bad plan entry"; return -1; }
+        if (n > IG_MAX_CANDS) continue;
         int* p = &plan[(size_t)t * (2 + IG_MAX_CANDS)];
         p[0] = n; p[1] = frags[t];
-        for (int i = 0; i < n; i++) {
-            const int c = cands8[(size_t)t * IG_MAX_CANDS + i];
-            if (c < 0 || c >= h->nf || c == frags[t]) { h->err = "ig_run_cycle: candidate out of range or equal to the visited fragment"; return -1; }
-            p[2 + i] = c;
-        }
+        for (int i = 0; i < n; i++) p[2 + i] = cands[(size_t)t * width + i];
     }
     if (cycle_buffers(h, n_steps)) return -2;
     CK(cudaMemcpyAsync(h->cyc_in, plan.data(), plan.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    if (wide) {
+        if (wide_plan_buffers(h, n_steps, width)) return -2;
+        std::vector<int> wp((size_t)n_steps * (2 + width), 0);
+        for (int t = 0; t < n_steps; t++) {
+            int* p = &wp[(size_t)t * (2 + width)];
+            p[0] = n_cands[t]; p[1] = frags[t];
+            for (int i = 0; i < n_cands[t]; i++) p[2 + i] = cands[(size_t)t * width + i];
+        }
+        CK(cudaMemcpyAsync(h->cyc_wide, wp.data(), wp.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+        CK(cudaStreamSynchronize(h->stream));   // (pageable source)
+    } else {
+        h->plan_width = IG_MAX_CANDS;
+    }
     return run_plan(h, n_steps, [&](int t) { return n_cands[t]; }, out);
 }
 
@@ -1139,7 +1342,7 @@ extern "C" int ig_set_neighbour_weights(ig_handle* h, const int64_t* ptr, const 
 static int prepare_device_plan(ig_handle* h, int32_t n_steps, const int32_t* frags, int32_t n_neighbours, uint64_t seed, uint32_t cycle) {
     if (!h->params_set) { h->err = "ig_run_cycle_device: parameters not set"; return -1; }
     if (!h->lvl->nb_ptr) { h->err = "ig_run_cycle_device: neighbour weights not set (ig_set_neighbour_weights)"; return -1; }
-    if (n_neighbours <= 0 || n_neighbours > IG_MAX_CANDS) { h->err = "ig_run_cycle_device: n_neighbours out of range"; return -1; }
+    if (n_neighbours <= 0 || n_neighbours > IG_MAX_NEIGHBOURS) { h->err = "ig_run_cycle_device: n_neighbours out of range (1 .. IG_MAX_NEIGHBOURS = 64)"; return -1; }
     if (h->nf < 2) { h->err = "ig_run_cycle_device: needs at least two fragments"; return -1; }
     if (h->pending_steps) { h->err = "ig_run_cycle_device: an asynchronous cycle is still pending (ig_cycle_wait)"; return -1; }
     for (int t = 0; t < n_steps; t++) if (frags[t] < 0 || frags[t] >= h->nf) { h->err = "ig_run_cycle_device: fragment out of range"; return -1; }
@@ -1152,8 +1355,16 @@ static int prepare_device_plan(ig_handle* h, int32_t n_steps, const int32_t* fra
         k_nuis_begin<<<1, 1, 0, h->stream>>>(h->sc, (unsigned)(seed & 0xffffffffu), (unsigned)(seed >> 32), cycle);
         h->n_launches += 1;
     }
-    k_draw_plan<<<(n_steps + 127) / 128, 128, 0, h->stream>>>(h->cyc_in, h->cyc_frags, n_steps, n_neighbours, h->nf, h->lvl->nb_ptr, h->lvl->nb_idx,
-                                                            h->lvl->nb_cdf, h->lvl->nb_nnz, (unsigned)(seed & 0xffffffffu), (unsigned)(seed >> 32), cycle);
+    if (n_neighbours > IG_MAX_CANDS) {   // every step a wide step (enqueue_plan_step), candidates from the wide plan
+        if (wide_plan_buffers(h, n_steps, n_neighbours)) return -2;
+        k_draw_plan_wide<<<(n_steps + 127) / 128, 128, 0, h->stream>>>(h->cyc_wide, n_neighbours, h->cyc_frags, n_steps, n_neighbours, h->nf,
+                                                                     h->lvl->nb_ptr, h->lvl->nb_idx, h->lvl->nb_cdf, h->lvl->nb_nnz,
+                                                                     (unsigned)(seed & 0xffffffffu), (unsigned)(seed >> 32), cycle);
+    } else {
+        h->plan_width = IG_MAX_CANDS;
+        k_draw_plan<<<(n_steps + 127) / 128, 128, 0, h->stream>>>(h->cyc_in, h->cyc_frags, n_steps, n_neighbours, h->nf, h->lvl->nb_ptr, h->lvl->nb_idx,
+                                                                h->lvl->nb_cdf, h->lvl->nb_nnz, (unsigned)(seed & 0xffffffffu), (unsigned)(seed >> 32), cycle);
+    }
     if (launch_ok(h, "draw_plan")) return -2;
     h->n_launches += 1;
     return 0;
@@ -1209,9 +1420,29 @@ extern "C" int ig_cycle_wait(ig_handle* h, int32_t n_steps, ig_cycle_step* out) 
 
 // download the plan of the last cycle ([n_steps][2 + IG_MAX_CANDS]: n_cands, fragment, candidates) -- tests / logging
 extern "C" int ig_get_cycle_plan(ig_handle* h, int32_t n_steps, int32_t* out) {
+    return ig_get_cycle_plan_wide(h, n_steps, IG_MAX_CANDS, out);
+}
+// the same as [n_steps][2 + width], from the plan the last cycle ran (narrow, or wide of stride 2 + plan_width)
+extern "C" int ig_get_cycle_plan_wide(ig_handle* h, int32_t n_steps, int32_t width, int32_t* out) {
     if (use(h)) return -1;
     if (n_steps > h->cyc_cap) { h->err = "ig_get_cycle_plan: no such plan"; return -1; }
-    CK(cudaMemcpy(out, h->cyc_in, sizeof(int) * (size_t)n_steps * (2 + IG_MAX_CANDS), cudaMemcpyDeviceToHost));
+    if (width <= 0 || width > IG_MAX_NEIGHBOURS) { h->err = "ig_get_cycle_plan: width out of range (1 .. IG_MAX_NEIGHBOURS = 64)"; return -1; }
+    if (n_steps <= 0) return 0;
+    if (h->plan_width == IG_MAX_CANDS && width == IG_MAX_CANDS) {
+        CK(cudaMemcpy(out, h->cyc_in, sizeof(int) * (size_t)n_steps * (2 + IG_MAX_CANDS), cudaMemcpyDeviceToHost));
+        return 0;
+    }
+    const int src_w = h->plan_width;
+    if (src_w > IG_MAX_CANDS && (size_t)n_steps * (2 + src_w) > h->cyc_wide_cap) { h->err = "ig_get_cycle_plan: no such plan"; return -1; }
+    std::vector<int> src((size_t)n_steps * (2 + src_w));
+    CK(cudaMemcpy(src.data(), src_w > IG_MAX_CANDS ? h->cyc_wide : h->cyc_in, src.size() * sizeof(int), cudaMemcpyDeviceToHost));
+    for (int t = 0; t < n_steps; t++) {
+        const int* p = &src[(size_t)t * (2 + src_w)];
+        int* q = out + (size_t)t * (2 + width);
+        if (p[0] > width) { h->err = "ig_get_cycle_plan: a step of the last cycle has more candidates than width"; return -1; }
+        q[0] = p[0]; q[1] = p[1];
+        for (int i = 0; i < width; i++) q[2 + i] = i < p[0] ? p[2 + i] : 0;
+    }
     return 0;
 }
 
@@ -1259,6 +1490,7 @@ extern "C" int ig_set_gpu_share(ig_handle* h, int32_t share) {
     if (h->pending_steps) { h->err = "ig_set_gpu_share: an asynchronous cycle is still pending"; return -1; }
     CK(cudaStreamSynchronize(h->stream));
     for (int i = 0; i < 8; i++) for (int j = 0; j <= IG_MAX_CANDS; j++) if (h->graph[i][j]) { cudaGraphExecDestroy(h->graph[i][j]); h->graph[i][j] = nullptr; }
+    destroy_wide_graphs(h, 0);
     if (h->graph_nuis_dev) { cudaGraphExecDestroy(h->graph_nuis_dev); h->graph_nuis_dev = nullptr; }
     h->grid_score = std::max(8, h->grid_score_full / share);
     h->grid_flat = std::max(1, h->grid_score / 5);

@@ -389,12 +389,11 @@ class sampler:
     # ------------------------------------------------------------------ the hot path
     def _usable_candidates(self, id_frag, candidates):
         """Sorted candidate list of one step: deviation D1 (B == A dropped, see step_sampler) and the library's limit of
-        IG_MAX_CANDS candidates per step (the reference has no limit; its CLI default is 5)."""
+        IG_MAX_NEIGHBOURS candidates per step (the reference has no limit; its CLI default is 5)."""
         cs = sorted(int(c) for c in candidates if int(c) != int(id_frag))
-        if len(cs) > L.IG_MAX_CANDS:
+        if len(cs) > L.IG_MAX_NEIGHBOURS:
             raise ValueError("instagraal_b200 scores at most %d candidate neighbours per step (got %d: lower "
-                             "--neighborhood / n_neighbours, or rebuild the library with a larger IG_MAX_CANDS)"
-                             % (L.IG_MAX_CANDS, len(cs)))
+                             "--neighborhood / n_neighbours)" % (L.IG_MAX_NEIGHBOURS, len(cs)))
         return cs
 
     def step_sampler(self, id_frag, n_neighbours, dt, candidates=None):
@@ -413,7 +412,8 @@ class sampler:
             self.all_scores = np.zeros(0)
             self.n_uniq, self.n_sub_vals = [], []
             return (self.likelihood_t, self._last_dist, -1, int(id_frag), self.mean_length_contigs, self.n_contigs)
-        self._cand_buf[:n] = self.candidates
+        if n <= L.IG_MAX_CANDS:
+            self._cand_buf[:n] = self.candidates
         res = self._res
         fut = None
         if self._nuis_follows and self.param_simu is not None:   # the previous call was a nuisance step: expect the next one
@@ -422,13 +422,24 @@ class sampler:
                 self._spec_pool = ThreadPoolExecutor(max_workers=1, thread_name_prefix="ig-nuisance")
             fut = self._spec_pool.submit(self._speculate_nuisance)
         self._nuis_follows = False
-        rc = self._ig_step(self._h, int(id_frag), self._cand_ptr, n, self._res_ref)
+        if n <= L.IG_MAX_CANDS:
+            rc = self._ig_step(self._h, int(id_frag), self._cand_ptr, n, self._res_ref)
+        else:   # more candidates than one scoring pass takes: ig_step_wide (batches of IG_MAX_CANDS)
+            wide = self._wide_buffers()
+            wide["cands"][:n] = self.candidates
+            rc = L.lib().ig_step_wide(self._h, int(id_frag), _ptr(wide["cands"]), n, self._res_ref, _ptr(wide["scores"]),
+                                      _ptr(wide["n_uniq"]), _ptr(wide["n_sub"]))
         self._spec = fut.result() if fut is not None else None
         if rc != 0:
             L.check(self._h, rc, "ig_step")
-        self.all_scores = self._res_scores[:self.n_tmp_struct * n].copy()
-        self.n_uniq = self._res_nuniq[:n].tolist()
-        self.n_sub_vals = self._res_nsub[:n].tolist()
+        if n <= L.IG_MAX_CANDS:
+            self.all_scores = self._res_scores[:self.n_tmp_struct * n].copy()
+            self.n_uniq = self._res_nuniq[:n].tolist()
+            self.n_sub_vals = self._res_nsub[:n].tolist()
+        else:
+            self.all_scores = wide["scores"][:self.n_tmp_struct * n].copy()
+            self.n_uniq = wide["n_uniq"][:n].tolist()
+            self.n_sub_vals = wide["n_sub"][:n].tolist()
         self.n_proposals_scored += sum(self.n_uniq)
         self.q4_hits = res.q4_hits
         global_id = np.int64(res.cand_index * self.n_tmp_struct + res.op_sampled)
@@ -443,6 +454,16 @@ class sampler:
         self._last_dist = res.dist
         return (o, res.dist, op_sampled, id_f_sampled, self.mean_length_contigs, self.n_contigs)
 
+    def _wide_buffers(self):
+        """host buffers of ig_step_wide (made on first use, per handle)"""
+        w = getattr(self, "_wide", None)
+        if w is None or w["owner"] is not self._h:
+            w = {"owner": self._h, "cands": np.zeros(L.IG_MAX_NEIGHBOURS, dtype=np.int32),
+                 "scores": np.zeros(L.IG_MAX_NEIGHBOURS * L.IG_N_OPS, dtype=np.float64),
+                 "n_uniq": np.zeros(L.IG_MAX_NEIGHBOURS, dtype=np.int32), "n_sub": np.zeros(L.IG_MAX_NEIGHBOURS, dtype=np.int32)}
+            self._wide = w
+        return w
+
     def run_cycle(self, list_frags, n_neighbours=5, candidates=None):
         """The inner loop of full_em (IG:217-241) for the fragments in ``list_frags`` as ONE library call:
         candidates are drawn here with the reference's own RNG calls in the reference's order (they do not
@@ -451,19 +472,25 @@ class sampler:
         (likelihood, dist, op_sampled, id_f_sampled, sum_l_cont, n_contigs, n_proposals)."""
         n = len(list_frags)
         frags = np.ascontiguousarray(list_frags, dtype=np.int32)
-        c8 = np.zeros((n, L.IG_MAX_CANDS), dtype=np.int32)
-        nc = np.zeros(n, dtype=np.int32)
+        lists = []
         for t in range(n):
             cs = candidates[t] if candidates is not None else self.return_neighbours(int(frags[t]), n_neighbours)
             cs = self._usable_candidates(frags[t], cs)  # deviation D1, see step_sampler
             if not cs:
                 raise ValueError("run_cycle: step %d (fragment %d) has no candidate but the visited fragment itself; "
                                  "use step_sampler (which skips such a step) or n_neighbours >= 2" % (t, int(frags[t])))
+            lists.append(cs)
+        # candidate array of IG_MAX_CANDS columns, or as wide as the longest list (ig_run_cycle_wide)
+        width = max([L.IG_MAX_CANDS] + [len(cs) for cs in lists])
+        c8 = np.zeros((n, width), dtype=np.int32)
+        nc = np.zeros(n, dtype=np.int32)
+        for t, cs in enumerate(lists):
             nc[t] = len(cs)
             c8[t, :len(cs)] = cs
         out = np.zeros(n, dtype=L.CYCLE_DTYPE)
         assert out.dtype.itemsize == C.sizeof(L.ig_cycle_step)
-        L.check(self._h, L.lib().ig_run_cycle(self._h, n, _ptr(frags), _ptr(c8), _ptr(nc), _ptr(out)), "ig_run_cycle")
+        L.check(self._h, L.lib().ig_run_cycle_wide(self._h, n, _ptr(frags), _ptr(c8), int(width), _ptr(nc), _ptr(out)), "ig_run_cycle")
+        self._plan_width = width
         if n:
             last = out[-1]
             self.n_contigs = np.int32(last["n_contigs"])
@@ -510,6 +537,7 @@ class sampler:
         out = np.zeros(n, dtype=L.CYCLE_DTYPE)
         L.check(self._h, L.lib().ig_run_cycle_device(self._h, n, _ptr(frags), int(n_neighbours), int(seed), int(cycle), _ptr(out)),
                 "ig_run_cycle_device")
+        self._plan_width = max(L.IG_MAX_CANDS, int(n_neighbours))
         self._after_cycle(out)
         if not nuisance:
             return out
@@ -567,10 +595,12 @@ class sampler:
             self.likelihood_t = self.o = np.float64(last["likelihood"])
             self.n_proposals_scored += int(out["n_proposals"].sum())
 
-    def last_cycle_plan(self, n_steps):
-        """(n_cands, fragment, candidates[8]) per step of the last run_cycle / run_cycle_device call."""
-        plan = np.zeros((int(n_steps), 2 + L.IG_MAX_CANDS), dtype=np.int32)
-        L.check(self._h, L.lib().ig_get_cycle_plan(self._h, int(n_steps), _ptr(plan)), "ig_get_cycle_plan")
+    def last_cycle_plan(self, n_steps, width=None):
+        """(n_cands, fragment, candidates[width]) per step of the last run_cycle / run_cycle_device call; width defaults to
+        that call's (IG_MAX_CANDS, or its number of neighbours / longest candidate list when larger)."""
+        width = int(width if width is not None else getattr(self, "_plan_width", L.IG_MAX_CANDS))
+        plan = np.zeros((int(n_steps), 2 + width), dtype=np.int32)
+        L.check(self._h, L.lib().ig_get_cycle_plan_wide(self._h, int(n_steps), width, _ptr(plan)), "ig_get_cycle_plan")
         return plan
 
     def eval_likelihood(self):

@@ -67,7 +67,7 @@ class ReplicaSet:
             c.bomb_the_genome()
 
     def run_cycle(self, frags_per_chain, n_neighbours=5, cycle=0, nuisance=False):
-        """frags_per_chain: int32[n_chains, n_steps] visiting orders.  Returns the structured per-step records
+        """frags_per_chain: int32[n_chains, n_steps] visiting orders, n_neighbours <= IG_MAX_NEIGHBOURS (64).  Returns the structured per-step records
         [n_chains, n_steps] (same fields as sampler.run_cycle_device).  nuisance=True: every chain samples the p(s)
         parameters after every step, on the device with its own seed (sampler.run_cycle_device(nuisance=True)); returns
         (steps, nuis) with nuis [n_chains, n_steps] of sampler.NUIS_STEP_DTYPE."""
@@ -82,6 +82,7 @@ class ReplicaSet:
                                                 int(cycle), _ptr(out))
         L.check(None, rc, "ig_run_cycles_device_multi")
         for i, c in enumerate(self.chains):
+            c._plan_width = max(L.IG_MAX_CANDS, int(n_neighbours))
             c._after_cycle(out[i])
         if not nuisance:
             return out
