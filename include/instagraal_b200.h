@@ -238,12 +238,19 @@ int ig_cycle_wait(ig_handle* h, int32_t n_steps, ig_cycle_step* out);
  * ig_nccl_init: one communicator per process / GPU, owned by `lead`; n_ranks == 1 needs no id and no NCCL.
  * ig_allgather_best: lik / n_contigs = [n_ranks * n_local] (rank-major); best = index of the highest likelihood (lowest index
  * on ties; the same on every rank); ms = device time of pack + all-gather (CUDA events).
- * ig_get_gathered_state: scaffold [13][NF] of chain `index` as of the last all-gather. */
+ * ig_get_gathered_state: scaffold [13][NF] of chain `index` as of the last all-gather.
+ * ig_adopt_gathered: every local chain whose global index differs from `index` restarts from chain `index` of the last
+ * all-gather, on the device: scaffold, live parameters, validity list (quirk Q3) and contig-label counter; its next step is a
+ * full refresh and it keeps its own seed.  Chain `index`, if local, is not touched.  Asynchronous: enqueued on the lead's
+ * stream, each adopting chain's stream waits for it.  p8_out / valid_out / likelihood_out (each may be NULL) receive the
+ * adopted chain's parameters, validity list and likelihood. */
 int ig_nccl_unique_id(char id_out[128]);
 int ig_nccl_init(ig_handle* lead, int32_t rank, int32_t n_ranks, int32_t n_local_chains, const char id[128]);
 int ig_allgather_best(ig_handle* lead, ig_handle** local_chains, int32_t n_local, double* lik, int32_t* n_contigs, int32_t* best,
                       float* ms);
 int ig_get_gathered_state(ig_handle* lead, int32_t index, int32_t* out13xNF);
+int ig_adopt_gathered(ig_handle* lead, ig_handle** local_chains, int32_t n_local, int32_t index, float p8_out[8], int32_t valid_out[12],
+                      double* likelihood_out);
 int ig_nccl_finalize(ig_handle* lead);
 /* ---- pyramid build (SURVEY 8f N2; pyramid_sparse.py:331-397 fill_sparse_pyramid_level, :686-722 the contact part of
  * subsample_data_set): bin n contacts (fa, fb 0-based, count nc) of one level.  old2new (may be NULL = identity) maps an

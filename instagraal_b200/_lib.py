@@ -27,6 +27,7 @@ EXPORTS = (
     "ig_selftest_math", "ig_get_nuisance_stats", "ig_clone", "ig_run_cycles_device_multi", "ig_run_cycle_device_async", "ig_cycle_wait",
     "ig_bin_contacts", "ig_nccl_unique_id", "ig_nccl_init", "ig_allgather_best", "ig_get_gathered_state", "ig_nccl_finalize",
     "ig_set_device_nuisance", "ig_get_nuisance_records", "ig_step_wide", "ig_run_cycle_wide", "ig_get_cycle_plan_wide",
+    "ig_adopt_gathered",
 )
 
 
@@ -118,6 +119,7 @@ def lib():
         L.ig_nccl_init.argtypes = [vp, i32, i32, i32, vp]
         L.ig_allgather_best.argtypes = [vp, vp, i32, vp, vp, C.POINTER(i32), C.POINTER(C.c_float)]
         L.ig_get_gathered_state.argtypes = [vp, i32, vp]
+        L.ig_adopt_gathered.argtypes = [vp, vp, i32, i32, vp, vp, C.POINTER(dbl)]
         L.ig_nccl_finalize.argtypes = [vp]
         L.ig_selftest_math.argtypes = [vp, i32, C.c_float, C.c_float, C.c_float, vp]
         L.ig_set_device_nuisance.argtypes = [vp, i32]

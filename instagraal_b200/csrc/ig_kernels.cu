@@ -611,13 +611,17 @@ extern "C" int ig_set_state(ig_handle* h, const int32_t* in13) {
     h->incr_valid = false;
     return 0;
 }
+// (the handle's stream is drained first: ig_adopt_gathered writes the list asynchronously, and these copies run on the
+// legacy stream, which is not ordered with the handle's non-blocking one)
 extern "C" int ig_get_valid_insert(ig_handle* h, int32_t out12[12]) {
     if (use(h)) return -1;
+    CK(cudaStreamSynchronize(h->stream));
     CK(cudaMemcpy(out12, h->sc->valid, 12 * sizeof(int), cudaMemcpyDeviceToHost));
     return 0;
 }
 extern "C" int ig_set_valid_insert(ig_handle* h, const int32_t in12[12]) {
     if (use(h)) return -1;
+    CK(cudaStreamSynchronize(h->stream));
     CK(h2d_sync(h->sc->valid, in12, 12 * sizeof(int)));
     return 0;
 }

@@ -2,11 +2,12 @@
 // library (no PyTorch in the product).  Part of ig_kernels.cu (host side; included last).
 //
 // One process per GPU owns 1..n chains of the same level (ig_create + ig_clone).  Once per cycle (or every few hundred
-// steps) ig_allgather_best packs, per local chain, a 64-byte header {likelihood, n_contigs} + the live scaffold records
-// (64 B x NF) straight from device memory into one send buffer, all-gathers it over NVLink (ncclAllGather on the lead
-// handle's stream; NCCL is dlopen'ed, so the library loads without it), compacts the headers on the device and copies only
-// those to the host: every rank then takes the same decision (best chain = highest likelihood, lowest global index on
-// ties).  The winner's scaffold stays in the receive buffer of every rank (ig_get_gathered_state).
+// steps) ig_allgather_best packs, per local chain, a 128-byte header {likelihood, n_contigs, parameters, validity list,
+// label counter} + the live scaffold records (64 B x NF) straight from device memory into one send buffer, all-gathers it
+// over NVLink (ncclAllGather on the lead handle's stream; NCCL is dlopen'ed, so the library loads without it), compacts the
+// headers on the device and copies only those to the host: every rank then takes the same decision (best chain = highest
+// likelihood, lowest global index on ties).  The winner's record stays in the receive buffer of every rank
+// (ig_get_gathered_state), and ig_adopt_gathered restarts the local chains from it on the device.
 // The reference has no counterpart (single process, single GPU); a chain is inherently sequential, so there is no data-path
 // collective: replicas only (SURVEY 8e).
 #pragma once
@@ -38,10 +39,20 @@ static int nccl_load(std::string& err) {
     return 0;
 }
 
-struct ReplicaHeader { double likelihood; int n_contigs; int n_frags; long long pad[6]; };   // 64 B
+// Everything a chain carries besides its scaffold, so that another chain can take over its whole state (ig_adopt_gathered):
+// the live parameters (in the order of k_set_params_dev), the carried validity list (quirk Q3) and the label counter.
+struct ReplicaHeader {
+    double likelihood; int n_contigs; int n_frags;
+    float p8[8];
+    int valid[12];
+    int max_label;
+    int pad[7];
+};
+static_assert(sizeof(ReplicaHeader) == 128, "ReplicaHeader is 128 bytes (the scaffold records that follow it stay 64-B aligned)");
 struct ig_replica_state {
     void* comm;
     int rank, n_ranks, n_local;
+    bool gathered;             // an all-gather completed since ig_nccl_init (recv / h_heads hold its result)
     size_t rec_bytes;          // header + NF scaffold records
     char *send, *recv;         // [n_local] / [n_ranks * n_local] records
     ReplicaHeader* heads;      // compact headers on the device, [n_ranks * n_local]
@@ -52,8 +63,21 @@ struct ig_replica_state {
 __global__ void k_replica_header(const DevScalars* __restrict__ sc, int nf, ReplicaHeader* out) {
     ReplicaHeader r;
     r.likelihood = sc->likelihood; r.n_contigs = sc->n_heads; r.n_frags = nf;
-    for (int i = 0; i < 6; i++) r.pad[i] = 0;
+    const float* p = &sc->p.kuhn;
+    for (int i = 0; i < 8; i++) r.p8[i] = p[i];
+    for (int i = 0; i < 12; i++) r.valid[i] = sc->valid[i];
+    r.max_label = sc->max_label;
+    for (int i = 0; i < 7; i++) r.pad[i] = 0;
     *out = r;
+}
+// a chain takes over the gathered chain's parameters (as k_set_params_dev sets them), validity list and label counter
+__global__ void k_replica_adopt(const ReplicaHeader* __restrict__ src, DevScalars* sc) {
+    const ReplicaHeader& r = *src;
+    Params p;
+    p.kuhn = r.p8[0]; p.lm = r.p8[1]; p.c1 = r.p8[2]; p.slope = r.p8[3]; p.d = r.p8[4]; p.d_max = r.p8[5]; p.fact = r.p8[6]; p.v_inter = r.p8[7];
+    sc->p = p; sc->log10_vinter = log10((double)p.v_inter);
+    for (int i = 0; i < 12; i++) sc->valid[i] = r.valid[i];
+    sc->max_label = r.max_label;
 }
 __global__ void k_replica_compact(const char* __restrict__ recv, size_t rec_bytes, int n, ReplicaHeader* __restrict__ out) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -148,6 +172,7 @@ extern "C" int ig_allgather_best(ig_handle* h, ig_handle** local, int32_t n_loca
     CK(cudaStreamSynchronize(h->stream));
     if (launch_ok(h, "allgather_best")) return -2;
     h->n_launches += 2 * n_local + 1;
+    r->gathered = true;
     int b = 0;
     for (int i = 0; i < n_all; i++) {
         if (lik) lik[i] = r->h_heads[i].likelihood;
@@ -173,6 +198,60 @@ extern "C" int ig_get_gathered_state(ig_handle* h, int32_t index, int32_t* out13
         for (int k = 0; k < IG_N_FIELDS; k++) out13[(size_t)k * nf + i] = v[k];
     }
     canonical_labels(nf, out13);
+    return 0;
+}
+
+// Every local chain other than `index` restarts from chain `index` of the last all-gather, device to device: its scaffold
+// records (raw contig labels: labels are only compared for equality, see labels_guard), parameters, validity list and label
+// counter, then its live expected-contact table is rebuilt.  The host flags become those of ig_set_state + ig_set_params, so
+// the chain's next step is a full refresh (kind 1).  Always read from recv, never from the source handle: one rank and N
+// ranks run the same code, and a local source chain is left untouched.  Everything is enqueued on the lead's stream, which
+// the gather used (a later gather is ordered after these copies out of recv); each adopting chain's stream waits for it.
+extern "C" int ig_adopt_gathered(ig_handle* h, ig_handle** local, int32_t n_local, int32_t index, float p8_out[8], int32_t valid_out[12],
+                                 double* likelihood_out) {
+    if (use(h)) return -1;
+    ig_replica_state* r = h->rep;
+    if (!r) { h->err = "ig_adopt_gathered: ig_nccl_init not called"; return -1; }
+    if (!r->gathered) { h->err = "ig_adopt_gathered: no all-gather since ig_nccl_init (ig_allgather_best)"; return -1; }
+    if (index < 0 || index >= r->n_ranks * r->n_local) { h->err = "ig_adopt_gathered: no such chain"; return -1; }
+    if (n_local != r->n_local) { h->err = "ig_adopt_gathered: number of local chains differs from ig_nccl_init"; return -1; }
+    for (int c = 0; c < n_local; c++)
+        if (!local[c] || local[c]->nf != h->nf || local[c]->ns != h->ns || local[c]->cfg.device != h->cfg.device) {
+            h->err = "ig_adopt_gathered: chains must share level and device"; return -1;
+        }
+    for (int c = 0; c < n_local; c++)
+        if (local[c]->pending_steps) { h->err = "ig_adopt_gathered: an asynchronous cycle is still pending (ig_cycle_wait)"; return -1; }
+    const ReplicaHeader& src = r->h_heads[index];
+    const char* rec = r->recv + r->rec_bytes * index;
+    int n_adopt = 0;
+    for (int c = 0; c < n_local; c++) {   // the copies wait for everything the chain has enqueued so far
+        if (r->rank * n_local + c == index || local[c] == h) continue;
+        CK(cudaEventRecord(r->ev_chain, local[c]->stream));
+        CK(cudaStreamWaitEvent(h->stream, r->ev_chain, 0));
+    }
+    for (int c = 0; c < n_local; c++) {
+        if (r->rank * n_local + c == index) continue;
+        ig_handle* t = local[c];
+        CK(cudaMemcpyAsync(t->live, rec + sizeof(ReplicaHeader), sizeof(FragRec) * (size_t)h->nf, cudaMemcpyDeviceToDevice, h->stream));
+        k_replica_adopt<<<1, 1, 0, h->stream>>>(reinterpret_cast<const ReplicaHeader*>(rec), t->sc);
+        k_exz_table<<<std::min(1024, (t->ns + 256) / 256), 256, 0, h->stream>>>(t->exz, t->ns + 1, t->sc, t->cfg.mean_sub_len_kb, 0);
+        n_adopt++;
+    }
+    if (launch_ok(h, "adopt_gathered")) return -2;
+    h->n_launches += 2 * n_adopt;
+    CK(cudaEventRecord(r->ev_chain, h->stream));
+    for (int c = 0; c < n_local; c++) {
+        if (r->rank * n_local + c == index) continue;
+        ig_handle* t = local[c];
+        if (t != h) CK(cudaStreamWaitEvent(t->stream, r->ev_chain, 0));
+        t->label_hi = src.max_label;
+        t->coords_fresh = false; t->incr_valid = false;
+        t->lnz_stale = true; t->params_set = true;
+        t->vinter_pos = src.p8[7] > 0.0f;
+    }
+    if (p8_out) memcpy(p8_out, src.p8, sizeof src.p8);
+    if (valid_out) memcpy(valid_out, src.valid, sizeof src.valid);
+    if (likelihood_out) *likelihood_out = src.likelihood;
     return 0;
 }
 extern "C" int ig_nccl_finalize(ig_handle* h) {

@@ -4,8 +4,10 @@ independent chains with different seeds, one or more per GPU).
 ``ReplicaSet`` owns the chains of ONE process / GPU: the first one is a normal ``sampler`` (uploads the level), the others
 are ``ig_clone``s that share its contacts in device memory.  ``run_cycle`` advances all of them together
 (``ig_run_cycles_device_multi``: steps enqueued round-robin on the chains' streams, so a GPU that one yeast-scale chain
-keeps < 25 % busy is filled by eight); ``allgather`` is the per-cycle exchange of {likelihood, n_contigs, live scaffold}
-across the GPUs: ``ncclAllGather`` INSIDE the library, straight from device memory over NVLink (``ig_allgather_best``).
+keeps < 25 % busy is filled by eight); ``allgather`` is the per-cycle exchange of {likelihood, n_contigs, p(s) parameters,
+validity list, live scaffold} across the GPUs: ``ncclAllGather`` INSIDE the library, straight from device memory over NVLink
+(``ig_allgather_best``).  ``adopt`` / ``exchange`` restart every chain from the gathered best one on the device
+(``ig_adopt_gathered``), so the set searches as one population instead of N unrelated runs.
 No PyTorch here: the launcher only has to hand every rank the 128-byte NCCL id created by rank 0
 (``nccl_unique_id`` -> file / environment / any broadcast).
 The live path of the reference has no temperature (fragment moves are an argmax, CL:1435-1446), so the chains differ by
@@ -50,6 +52,7 @@ class ReplicaSet:
         self.nf = int(first_sampler.n_new_frags)
         self.gather_ms = 0.0
         self.n_gathers = 0
+        self._gathered_nc = None   # n_contigs of every chain in the last all-gather
         # several chains on this GPU: each takes a share of the SMs so that their (latency-bound) kernels overlap
         self.gpu_share = min(n_chains, 4)
         for c in self.chains:
@@ -101,7 +104,35 @@ class ReplicaSet:
                 "ig_allgather_best")
         self.gather_ms += float(ms.value)
         self.n_gathers += 1
+        self._gathered_nc = nc
         return int(best.value), lik, nc
+
+    def adopt(self, index):
+        """Every local chain other than global chain ``index`` restarts from that chain's state in the last all-gather, on the
+        device (ig_adopt_gathered): scaffold, p(s) parameters and validity list; each keeps its own seed, and its next step
+        is a full refresh.  Chain ``index``, if it is local, is not touched.  -> (p8, valid, likelihood) of chain ``index``."""
+        from .cuda_lib_gl_single import PARAM_SIMU_RIPPE
+        p8 = np.zeros(8, dtype=np.float32)
+        valid = np.zeros(12, dtype=np.int32)
+        lik = C.c_double(0.0)
+        lead = self.chains[0]
+        L.check(lead._h, L.lib().ig_adopt_gathered(lead._h, self._handles, self.n, int(index), _ptr(p8), _ptr(valid), C.byref(lik)),
+                "ig_adopt_gathered")
+        for c, ch in enumerate(self.chains):
+            if self.rank * self.n + c == int(index):
+                continue
+            ch.param_simu = np.array([tuple(p8.tolist())], dtype=PARAM_SIMU_RIPPE)
+            ch.param_simu_test = ch.param_simu
+            ch.likelihood_t = ch.o = np.float64(lik.value)
+            ch.n_contigs = np.int32(self._gathered_nc[int(index)])
+        return p8, valid, float(lik.value)
+
+    def exchange(self):
+        """allgather() followed by adopt(best): every chain continues from the best chain of the whole set.
+        -> (best, likelihood[n_ranks * n], n_contigs[n_ranks * n]) as allgather returns them."""
+        best, lik, nc = self.allgather()
+        self.adopt(best)
+        return best, lik, nc
 
     def gathered_state(self, index):
         out = np.zeros((13, self.nf), dtype=np.int32)
