@@ -146,8 +146,9 @@ k_full_lnz(const long long* __restrict__ row_ptr, const int2* __restrict__ cv, c
         }
     }
     if (lane < qn) acc += lnz_eval(myq[lane], p, l10v);
-    // floor contacts: ob * log10(v_inter) - v_inter each (KA:259-262 with ex == v_inter)
-    acc += l10v * (double)sob - (double)p.v_inter * (double)nfl + acc_exz * (double)LOG10E_F;
+    // floor contacts: ob * log10(v_inter) - v_inter each (KA:259-262 with ex == v_inter).  The generic routine has no floor
+    // sums (sob == nfl == acc_exz == 0), and with v_inter <= 0 log10(v_inter) is -inf or NaN: 0 * -inf would make it NaN
+    if (!generic) acc += l10v * (double)sob - (double)p.v_inter * (double)nfl + acc_exz * (double)LOG10E_F;
     double tot = block_sum(acc, sm);
     if (threadIdx.x == 0) part[blockIdx.x] = tot - (blockIdx.x == 0 ? sc->obc_total : 0.0);
 }

@@ -99,8 +99,10 @@ def dist_inter_genome(live, init_prev, init_next, orientable):
 def distance_histogram(sparse_matrix, soa, s2f, n_rows, max_dist_kb, size_bin_kb):
     """Histogram part of estimate_parameters_rippe CL:2247-2297: for the first ``n_rows`` rows of the
     SYMMETRIC level L-1 matrix, per-row contact sums per distance bin (intra-contig only), then the
-    mean over rows.  Returns (bins, mean_contacts float64, n_rows_used)."""
+    mean over rows.  Returns (bins, mean_contacts float64, n_rows_used).  Rows past the level's last do not exist: n_rows
+    is clamped to the number of sub-fragments."""
     sym = (sparse_matrix + sparse_matrix.transpose()).tocsr()
+    n_rows = min(int(n_rows), sym.shape[0])
     bins = np.arange(size_bin_kb, max_dist_kb + size_bin_kb, size_bin_kb)
     acc = np.zeros(len(bins), dtype=np.int64)
     used = 0

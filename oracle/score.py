@@ -97,8 +97,10 @@ def sub_tables(np_sub_frags_2_frags):
                 crick=a["z"].astype(np.float32), j=a["w"].astype(np.int64))
 
 
-def contact_terms(v, rows, cols, dat, p: Params, mbar, len_from="col"):
-    """Per-contact term of KA:4296-4354 / 4155-4208 / 4409-4464 for coordinates ``v``."""
+def contact_terms(v, rows, cols, dat, p: Params, mbar, len_from="col", return_parts=False):
+    """Per-contact term of KA:4296-4354 / 4155-4208 / 4409-4464 for coordinates ``v``.
+    return_parts=True: (terms, ex, exz), the float32 expected contacts of each contact and of its zero term
+    (error bounds on a device sum are built from them)."""
     ci, cj = v["id_c"][rows], v["id_c"][cols]
     si, sj = v["dist"][rows], v["dist"][cols]
     s = np.abs((si - sj).astype(np.float32))
@@ -118,7 +120,8 @@ def contact_terms(v, rows, cols, dat, p: Params, mbar, len_from="col"):
         ex_c, exz_c = ex_lin, exz_lin
     ex = np.where(same, np.where(lin, ex_lin, ex_c), p.v_inter).astype(np.float32)
     exz = np.where(same, np.where(lin, exz_lin, exz_c), p.v_inter).astype(np.float32)
-    return likelihood_pxl(ex, dat) + exz.astype(np.float64) * LOG10E_F
+    terms = likelihood_pxl(ex, dat) + exz.astype(np.float64) * LOG10E_F
+    return (terms, ex, exz) if return_parts else terms
 
 
 def full_likelihood_nz(v, coo, p, mbar):
@@ -127,9 +130,10 @@ def full_likelihood_nz(v, coo, p, mbar):
     return float(np.sum(contact_terms(v, rows, cols, dat, p, mbar, len_from="row")))
 
 
-def zeros_term_raw(v, p, mbar):
+def zeros_term_raw(v, p, mbar, return_parts=False):
     """eval_likelihood_on_zero / eval_all_likelihood_on_zero_1st (KA:3850-4002):
-    returns (Z = -sum ex*(len-pos), n_intra as wrapped int32)."""
+    returns (Z = -sum ex*(len-pos), n_intra as wrapped int32); return_parts=True appends the float64 terms
+    ex*(len-pos) of the sub-fragments that have one (pos > 0)."""
     pos, ln, s_tot = v["pos"], v["len"], v["s_tot"]
     heads = pos == 0
     lh = ln[heads].astype(np.int64)
@@ -142,8 +146,9 @@ def zeros_term_raw(v, p, mbar):
     lin = s_tot[m] == 0
     ex = np.where(lin, rippe_contacts(s, p), rippe_contacts_circ(s, s_tot_z, p) if np.any(~lin) else F32(0))
     ex = np.where(s < p.d_max, ex, p.v_inter).astype(np.float64)
-    z = -float(np.sum(ex * (ln[m] - pos[m]).astype(np.float64)))
-    return z, n_intra
+    terms = ex * (ln[m] - pos[m]).astype(np.float64)
+    z = -float(np.sum(terms))
+    return (z, n_intra, terms) if return_parts else (z, n_intra)
 
 
 def _wrap32(x):

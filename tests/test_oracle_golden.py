@@ -130,3 +130,31 @@ def test_yeast_toy_config0_oracle_cycle_sample():
         assert 0 <= int(r[2]) < 24 and 0 <= int(r[3]) < level.n_frags
         n_prop += int(sum(o.n_uniq_list))
     assert n_prop >= 4 * 10
+
+
+@pytest.mark.parametrize("d_exp", [2.0, 2.37])
+def test_contact_terms_return_parts_equal_the_plain_call(d_exp):
+    """contact_terms(..., return_parts=True) and zeros_term_raw(..., return_parts=True) return the same terms as the plain
+    calls bit for bit, plus float32 expected values the terms are rebuilt from; circular contigs included."""
+    from oracle.fuzz import random_state
+    level = make_level(WORKLOADS["micro"])
+    p8 = np.array([2.2354, 1.4933294, 0.06928191, -0.9384134, d_exp, 386.88467, 65.71848, 0.01698581], dtype=np.float32)
+    o = OracleSampler(level, p8)
+    from test_gpu_parity import _rebuild_offsets
+    st = random_state(level.n_frags, np.random.RandomState(4), p_circ=0.5)
+    for k in ("len_bp", "sub_len"):   # the level's fragment lengths, so that coordinates stay meaningful
+        st[k] = np.asarray(level.S_o_A_frags[k], dtype=np.int32).copy()
+    st = _rebuild_offsets(st)
+    assert st["circ"].any()
+    for live in (o.live, st):
+        v = sc.fill_vect_dist(live, o.sub)
+        for len_from in ("row", "col"):
+            t0 = sc.contact_terms(v, *o.coo, o.params, o.mbar, len_from=len_from)
+            t1, ex, exz = sc.contact_terms(v, *o.coo, o.params, o.mbar, len_from=len_from, return_parts=True)
+            assert ex.dtype == np.float32 and exz.dtype == np.float32 and ex.shape == exz.shape == t0.shape
+            assert np.array_equal(t0.view(np.int64), t1.view(np.int64))
+            t2 = sc.likelihood_pxl(ex, o.coo[2]) + exz.astype(np.float64) * sc.LOG10E_F
+            assert np.array_equal(t0.view(np.int64), t2.view(np.int64))
+        z0, n0 = sc.zeros_term_raw(v, o.params, o.mbar)
+        z1, n1, zt = sc.zeros_term_raw(v, o.params, o.mbar, return_parts=True)
+        assert np.isfinite(z0) and (z0, n0) == (z1, n1) and z0 == -float(np.sum(zt)) and zt.size == int((v["pos"] > 0).sum())
