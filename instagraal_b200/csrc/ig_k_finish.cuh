@@ -390,8 +390,7 @@ __global__ void k_post_scalars(DevScalars* sc, const IgDescriptor* __restrict__ 
 }
 __global__ void __launch_bounds__(256)
 k_post(const FragRec* __restrict__ live, int nf, const int* __restrict__ init_prev, const int* __restrict__ init_next,
-       const int* __restrict__ orientable, DevScalars* sc, CycleOut* __restrict__ cyc_out, const int* __restrict__ d_nuniq,
-       const int* __restrict__ d_nsub) {
+       const int* __restrict__ orientable, DevScalars* sc, CycleOut* __restrict__ cyc_out) {
     TL(10);
     __shared__ int s_heads;
     __shared__ long long s_len, s_half;
@@ -445,7 +444,9 @@ k_post(const FragRec* __restrict__ live, int nf, const int* __restrict__ init_pr
                 o.likelihood = sc->likelihood; o.lnz_full = sc->lnz_full;
                 o.dist_half = *(volatile long long*)&sc->dist_half; o.sum_l_cont = *(volatile long long*)&sc->sum_l_cont;
                 o.n_heads = *(volatile int*)&sc->n_heads; o.win_cand = sc->win_cand; o.win_op = sc->win_op; o.q4_hits = sc->q4_hits;
-                for (int i = 0; i < IG_MAX_CANDS; i++) { o.n_uniq[i] = d_nuniq[i]; o.n_sub[i] = d_nsub[i]; o.pad[i] = 0; }
+                o.n_proposals = 0;
+                for (int i = 0; i < sc->n_cands; i++) o.n_proposals += sc->res_nuniq[i];
+                o.id_f_sampled = sc->cands[sc->win_cand];
                 cyc_out[sc->step_idx] = o;
                 sc->step_idx += 1;
 #ifdef IG_TIMELINE

@@ -25,13 +25,16 @@ __device__ __forceinline__ double philox_uniform(unsigned step, unsigned cycle, 
     const unsigned long long bits = ((unsigned long long)r.x << 32) | r.y;
     return (double)(bits >> 11) * (1.0 / 9007199254740992.0);  // 53 bits -> [0, 1)
 }
-// MAXC = the most draws a plan entry can hold, width = its number of candidate slots (plan stride 2 + width)
+// MAXC = the most draws a plan entry can hold (IG_MAX_CANDS, or IG_MAX_NEIGHBOURS for wider plans), width = its number of
+// candidate slots (plan stride 2 + width, written to sc->plan_stride).  Draw i has the counter (t, cycle, i, attempt) in
+// both instantiations, so a wide plan's first IG_MAX_CANDS draws are the narrow plan's.
 template <int MAXC>
-__device__ __forceinline__ void draw_plan_step(int* __restrict__ plan, int width, const int* __restrict__ frags, int n_steps, int delta, int nf,
-                                               const long long* __restrict__ nb_ptr, const int* __restrict__ nb_idx,
-                                               const double* __restrict__ nb_cdf, const int* __restrict__ nb_nnz, unsigned seed_lo,
-                                               unsigned seed_hi, unsigned cycle) {
+__global__ void k_draw_plan(int* __restrict__ plan, int width, DevScalars* sc, const int* __restrict__ frags, int n_steps, int delta,
+                            int nf, const long long* __restrict__ nb_ptr, const int* __restrict__ nb_idx,
+                            const double* __restrict__ nb_cdf, const int* __restrict__ nb_nnz, unsigned seed_lo, unsigned seed_hi,
+                            unsigned cycle) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t == 0) sc->plan_stride = 2 + width;
     if (t >= n_steps) return;
     const uint2 key = make_uint2(seed_lo, seed_hi);
     const int a = frags[t];
@@ -84,16 +87,4 @@ __device__ __forceinline__ void draw_plan_step(int* __restrict__ plan, int width
     for (int i = 0; i < n; i++) if (got[i] != a) p[2 + m++] = got[i];
     for (int i = m; i < width; i++) p[2 + i] = 0;
     p[0] = m; p[1] = a;
-}
-__global__ void k_draw_plan(int* __restrict__ plan, const int* __restrict__ frags, int n_steps, int delta, int nf,
-                            const long long* __restrict__ nb_ptr, const int* __restrict__ nb_idx, const double* __restrict__ nb_cdf,
-                            const int* __restrict__ nb_nnz, unsigned seed_lo, unsigned seed_hi, unsigned cycle) {
-    draw_plan_step<IG_MAX_CANDS>(plan, IG_MAX_CANDS, frags, n_steps, delta, nf, nb_ptr, nb_idx, nb_cdf, nb_nnz, seed_lo, seed_hi, cycle);
-}
-// plans of more than IG_MAX_CANDS neighbours (stride 2 + width, width <= IG_MAX_NEIGHBOURS): draw i has the counter
-// (t, cycle, i, attempt) of the narrow kernel, so a wide plan's first IG_MAX_CANDS draws are the narrow plan's
-__global__ void k_draw_plan_wide(int* __restrict__ plan, int width, const int* __restrict__ frags, int n_steps, int delta, int nf,
-                                 const long long* __restrict__ nb_ptr, const int* __restrict__ nb_idx, const double* __restrict__ nb_cdf,
-                                 const int* __restrict__ nb_nnz, unsigned seed_lo, unsigned seed_hi, unsigned cycle) {
-    draw_plan_step<IG_MAX_NEIGHBOURS>(plan, width, frags, n_steps, delta, nf, nb_ptr, nb_idx, nb_cdf, nb_nnz, seed_lo, seed_hi, cycle);
 }

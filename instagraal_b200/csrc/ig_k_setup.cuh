@@ -6,10 +6,10 @@
 // K2: per-candidate setup.  Thread 0 walks the candidates IN ORDER because extract_uniq_mutations
 //     of candidate k reads the list_valid_insert left by get_bounds of candidate k-1 (quirk Q3).
 __global__ void k_cand_setup(const FragRec* __restrict__ live, DevScalars* sc, IgDescriptor* desc, int n_bounds,
-                             int first_flip_eject, const int* __restrict__ cyc_in, int stream_mode) {
+                             int first_flip_eject, const int* __restrict__ plan, int stream_mode) {
     TL(0);
-    if (cyc_in) {  // cycle mode: this step's {n_cands, fragment, candidates} come from the uploaded cycle plan
-        const int* src = cyc_in + (size_t)sc->step_idx * (2 + IG_MAX_CANDS);
+    if (plan) {  // cycle mode: this step's {n_cands, fragment, candidates} come from the cycle plan (a step of <= IG_MAX_CANDS)
+        const int* src = plan + (size_t)sc->step_idx * sc->plan_stride;
         if (threadIdx.x < 2 + IG_MAX_CANDS) (&sc->n_cands)[threadIdx.x] = src[threadIdx.x];
         __syncthreads();
     }

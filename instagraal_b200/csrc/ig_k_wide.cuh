@@ -8,6 +8,8 @@
 // below only move data between the step's scalar record and the wide record: they stage a batch's candidates where
 // k_cand_setup reads them, keep every pass's scores and the running maximum, and fix up what the re-scored batch cannot
 // know (its index in the whole list, the flip/eject proposal of a batch other than the first, the validity list).
+// Everything around the launch sequence (enqueue_wide_step in ig_kernels.cu) is the narrow step's: host step, cycle plan
+// (read here at the stride sc->plan_stride), graph cache and step record.
 #define IG_MAX_BATCHES ((IG_MAX_NEIGHBOURS + IG_MAX_CANDS - 1) / IG_MAX_CANDS)
 struct WideStep {
     int in[2 + IG_MAX_NEIGHBOURS];             // ig_step_wide: n_cands, fragment, sorted candidates
@@ -22,11 +24,11 @@ struct WideStep {
 };
 
 // before batch b: its candidates (8b .. 8b + n_b - 1 of the step's list) into sc, where k_cand_setup reads them, and the
-// validity list the batch starts from.  plan = the cycle plan (stride 2 + width, entry sc->step_idx) or nullptr (w->in).
+// validity list the batch starts from.  plan = the cycle plan (entry sc->step_idx, stride sc->plan_stride) or nullptr (w->in).
 // A batch past the step's candidates (a device-drawn plan with fewer neighbours than asked for) gets n_b = 0: every
 // kernel of the pass then does nothing.
-__global__ void k_wide_stage(DevScalars* sc, WideStep* w, const int* __restrict__ plan, int width, int b) {
-    const int* src = plan ? plan + (size_t)sc->step_idx * (2 + width) : w->in;
+__global__ void k_wide_stage(DevScalars* sc, WideStep* w, const int* __restrict__ plan, int b) {
+    const int* src = plan ? plan + (size_t)sc->step_idx * sc->plan_stride : w->in;
     const int n = src[0], i = threadIdx.x;
     const int nb = max(0, min(IG_MAX_CANDS, n - b * IG_MAX_CANDS));
     if (i < IG_MAX_CANDS) sc->cands[i] = i < nb ? src[2 + b * IG_MAX_CANDS + i] : 0;
@@ -63,8 +65,8 @@ __global__ void k_wide_stash(const DevScalars* __restrict__ sc, WideStep* w, int
 
 // before the re-score: the winning batch (batch 0 when nothing was scored, as np.argmax of an all -inf vector) staged
 // like k_wide_stage, from the validity list it started from
-__global__ void k_wide_pick(DevScalars* sc, WideStep* w, const int* __restrict__ plan, int width) {
-    const int* src = plan ? plan + (size_t)sc->step_idx * (2 + width) : w->in;
+__global__ void k_wide_pick(DevScalars* sc, WideStep* w, const int* __restrict__ plan) {
+    const int* src = plan ? plan + (size_t)sc->step_idx * sc->plan_stride : w->in;
     const int b = max(w->best_b, 0);
     const int nb = max(0, min(IG_MAX_CANDS, w->n - b * IG_MAX_CANDS));
     const int i = threadIdx.x;
@@ -83,7 +85,8 @@ __global__ void k_wide_flip(const DevScalars* __restrict__ sc, IgDescriptor* des
 }
 
 // after the tail: the candidate index in the whole list, the step's proposal count (score-only passes), and the validity
-// list the reference leaves -- the last batch's, unless the applied op re-ran get_bounds (op >= 12, select_step)
+// list the reference leaves -- the last batch's, unless the applied op re-ran get_bounds (op >= 12, select_step).  The
+// fragment k_post recorded is already right: sc->cands holds the re-scored winning batch.
 __global__ void k_wide_finish(DevScalars* sc, WideStep* w, CycleOut* __restrict__ cyc_out) {
     const int i = threadIdx.x;
     if (i < 12 && sc->win_op < 12) sc->valid[i] = w->valid_end[i];
@@ -91,6 +94,6 @@ __global__ void k_wide_finish(DevScalars* sc, WideStep* w, CycleOut* __restrict_
     w->win_cand = w->best_b * IG_MAX_CANDS + sc->win_cand;
     if (cyc_out) {   // the record k_post just published (it advanced step_idx)
         CycleOut& o = cyc_out[sc->step_idx - 1];
-        o.win_cand = w->win_cand; o.pad[0] = w->n_prop; o.pad[1] = 1;
+        o.win_cand = w->win_cand; o.n_proposals = w->n_prop;
     }
 }

@@ -3,6 +3,8 @@
 // One ig_step() = one reference step_sampler() (cuda_lib_gl_single.py:1401-1465, "CL") with the
 // ~700 host<->device crossings collapsed into 11-12 stream-ordered launches (one CUDA-graph replay) and
 // ONE blocking D2H of a 6 KB result record; ig_run_cycle / ig_run_cycle_device enqueue a whole sweep.
+// Steps of up to 64 candidates take the same host step (ig_step_wide), cycle plan, graph cache and plan step; only the
+// launch sequence differs beyond IG_MAX_CANDS (enqueue_step / enqueue_wide_step, ig_k_wide.cuh).
 // Design (DESIGN.md has the long form):
 //   * contacts: CSR by row sub-fragment of the strict upper triangle, (col,val) interleaved int2;
 //     a candidate touches only the rows of the <=2 affected contigs (ordered row list built on
@@ -81,7 +83,7 @@ struct DevScalars {
     double lnz_next, z_next; int nintra_next;
     int prev_k, prev_u, prev_windowed, prev_id_a, prev_n_rows;
     unsigned int ticket_out, ticket_post;
-    int step_idx;
+    int step_idx, plan_stride;   // entry of the cycle plan the next step reads; ints per entry (2 + W), set by whoever writes the plan
     double full_out[3];
     int full_nintra, pad_;
     double obc_total;   // sum over every stored contact of the observed-count-only part of its term (k_obc_sum)
@@ -102,12 +104,11 @@ struct DevScalars {
     double nuis_u, nuis_draw;
 };
 
-struct CycleOut {  // compact per-step record of ig_run_cycle (128 B)
+struct CycleOut {  // compact per-step record of a cycle (k_post; k_wide_finish fixes up a wide step's)
     double likelihood, lnz_full;
     long long dist_half, sum_l_cont;
     int n_heads, win_cand, win_op, q4_hits;
-    int n_uniq[IG_MAX_CANDS], n_sub[IG_MAX_CANDS];
-    int pad[8];
+    int n_proposals, id_f_sampled;   // proposals scored by the step, fragment of the applied move's candidate
 };
 
 #include "ig_k_common.cuh"   // optional device-side timeline, the reference's device math (textual twins), reduction helpers
@@ -182,20 +183,19 @@ struct ig_handle {
     double* part_out;
     int gs_div, sparse_div, grid_split;
     long long last_n_full;
-    cudaGraphExec_t graph[8][IG_MAX_CANDS + 1];   // [step kind + 4 * cycle][candidates in the grid]
+    // one graph per [step kind + 4 * cycle][shape]: shape = candidates in the grid (1 .. IG_MAX_CANDS) of a narrow step,
+    // IG_MAX_CANDS + number of batches of a wide step (get_graph)
+    cudaGraphExec_t graph[8][IG_MAX_CANDS + IG_MAX_BATCHES + 1];
     // production-mode nuisance step (ig_set_device_nuisance): one graph per handle replayed after every plan step, the
     // per-step records (cyc_cap of them), and whether a nuisance step was enqueued since the plan began
     bool nuis_on = false, nuis_enqueued = false, nuis_graph_dev_failed = false;
     cudaGraphExec_t graph_nuis_dev = nullptr;
     ig_nuisance_step* nuis_rec = nullptr;
-    int* cyc_in; CycleOut* cyc_out; int cyc_cap; bool graph_failed, capturing, use_graph; long long n_full;
+    // the cycle plan [cyc_cap][2 + W] (n_cands, fragment, candidates), W <= cyc_width; plan_width = W of the last cycle
+    int* cyc_plan; CycleOut* cyc_out; int cyc_cap, cyc_width, plan_width; bool graph_failed, capturing, use_graph; long long n_full;
     int pending_steps;   // steps enqueued by an asynchronous cycle call and not collected yet
-    // steps of more than IG_MAX_CANDS candidates (ig_k_wide.cuh), allocated on first use: the wide record + its pinned mirror,
-    // the wide cycle plan ([cap][2 + plan_width]), and one graph per [step kind + 4 * cycle][number of batches]
+    // steps of more than IG_MAX_CANDS candidates (ig_k_wide.cuh): the wide record + its pinned mirror
     WideStep *wide = nullptr, *h_wide = nullptr;
-    int* cyc_wide = nullptr; size_t cyc_wide_cap = 0;
-    int plan_width = IG_MAX_CANDS;   // candidate slots per entry of the last cycle's plan (> IG_MAX_CANDS: cyc_wide)
-    cudaGraphExec_t graph_wide[8][IG_MAX_BATCHES + 1] = {};
     // measurement (CUDA events on the launching stream)
     cudaEvent_t ev[6];
     cudaEvent_t evk[16]; double ms_k[16];  // per-kernel event timing of the main stream (profiling mode)
@@ -277,7 +277,8 @@ static int create_impl(const ig_config* cfg, const ig_level_data* data, ig_handl
     }
     if (const char* e = getenv("IG_GS_DIV")) h->gs_div = std::max(1, atoi(e));
     if (const char* e = getenv("IG_BLOCK_MODE")) if (atoi(e)) h->gs_div = -h->gs_div;
-    memset(h->graph, 0, sizeof h->graph); h->cyc_in = nullptr; h->cyc_out = nullptr; h->cyc_frags = nullptr; h->cyc_cap = 0;
+    memset(h->graph, 0, sizeof h->graph); h->cyc_plan = nullptr; h->cyc_out = nullptr; h->cyc_frags = nullptr;
+    h->cyc_cap = 0; h->cyc_width = 0; h->plan_width = IG_MAX_CANDS;
     h->graph_failed = false; h->capturing = false; h->use_graph = true; h->n_full = 0; h->pending_steps = 0; h->rep = nullptr;
     cudaError_t e0 = cudaSetDevice(cfg->device);
     if (e0 != cudaSuccess) { g_err = std::string("cudaSetDevice: ") + cudaGetErrorString(e0); delete h; return -2; }
@@ -391,7 +392,8 @@ static int create_impl(const ig_config* cfg, const ig_level_data* data, ig_handl
         CK(cudaMallocHost((void**)&h->h_sc, sizeof(DevScalars)));
         CK(cudaMallocHost((void**)&h->h_small, 64 * sizeof(int)));
         CK(cudaMallocHost((void**)&h->h_p8, sizeof(Params)));
-        if (dev_alloc(h, &h->d_p8, 8)) return -2;
+        if (dev_alloc(h, &h->d_p8, 8) || dev_alloc(h, &h->wide, 1)) return -2;
+        CK(cudaMallocHost((void**)&h->h_wide, sizeof(WideStep)));
         CK(cudaMemsetAsync(h->sc, 0, sizeof(DevScalars), h->stream));
         // uploads
         if (parent) {
@@ -494,6 +496,14 @@ extern "C" int ig_clone(ig_handle* parent, ig_handle** out) {
     return create_impl(&parent->cfg, nullptr, parent, out);
 }
 
+// the step graphs of slots first_slot .. 7 (4 and up: cycle graphs) and the device nuisance graph, which bake in the
+// cycle buffers and the scoring grids
+static void destroy_graphs(ig_handle* h, int first_slot) {
+    for (int i = first_slot; i < 8; i++)
+        for (cudaGraphExec_t& g : h->graph[i]) if (g) { cudaGraphExecDestroy(g); g = nullptr; }
+    if (h->graph_nuis_dev) { cudaGraphExecDestroy(h->graph_nuis_dev); h->graph_nuis_dev = nullptr; }
+}
+
 static void replica_free(ig_handle* h);
 extern "C" void ig_destroy(ig_handle* h) {
     if (!h) return;
@@ -517,16 +527,13 @@ extern "C" void ig_destroy(ig_handle* h) {
     if (h->h_p8) cudaFreeHost(h->h_p8);
     if (h->d_p8) cudaFree(h->d_p8);
     if (h->graph_nuis) cudaGraphExecDestroy(h->graph_nuis);
-    if (h->graph_nuis_dev) cudaGraphExecDestroy(h->graph_nuis_dev);
     if (h->nuis_rec) cudaFree(h->nuis_rec);
     if (h->wide) cudaFree(h->wide);
     if (h->h_wide) cudaFreeHost(h->h_wide);
-    if (h->cyc_wide) cudaFree(h->cyc_wide);
-    for (int i = 0; i < 8; i++) for (int j = 0; j <= IG_MAX_BATCHES; j++) if (h->graph_wide[i][j]) cudaGraphExecDestroy(h->graph_wide[i][j]);
     for (int i = 0; i < 6; i++) if (h->ev[i]) cudaEventDestroy(h->ev[i]);
     for (int i = 0; i < 16; i++) if (h->evk[i]) cudaEventDestroy(h->evk[i]);
-    for (int i = 0; i < 8; i++) for (int j = 0; j <= IG_MAX_CANDS; j++) if (h->graph[i][j]) cudaGraphExecDestroy(h->graph[i][j]);
-    if (h->cyc_in) cudaFree(h->cyc_in);
+    destroy_graphs(h, 0);
+    if (h->cyc_plan) cudaFree(h->cyc_plan);
     if (h->cyc_out) cudaFree(h->cyc_out);
     if (h->side) cudaStreamDestroy(h->side);
     if (h->pf) cudaStreamDestroy(h->pf);
@@ -650,26 +657,6 @@ static int labels_guard(ig_handle* h) {
     return ig_set_state(h, st.data());
 }
 
-// head of step_sampler: fill_dist_single + eval_likelihood (CL:1407-1409)
-static int refresh_current(ig_handle* h, cudaStream_t st, bool fork) {
-    const float mbar = h->cfg.mean_sub_len_kb;
-    if (fork) {  // side stream: starts after everything already queued on the main stream
-        cudaEventRecord(h->ev_fork, h->stream);
-        cudaStreamWaitEvent(st, h->ev_fork, 0);
-    }
-    k_coords<<<h->n_part_zc, IG_THREADS, 0, st>>>(h->live, h->sub, h->coord, h->clen, h->ns, h->sc, mbar, 0, h->part_zc, h->part_nc, 1, h->subx, h->row_dirty);
-    k_reduce<<<1, 256, 0, st>>>(h->part_zc, h->n_part_zc, &h->sc->z_cur, h->part_nc, &h->sc->nintra_cur);
-    if (fork) cudaEventRecord(h->ev_coords, st);
-    if (h->profile) cudaEventRecord(h->ev[2], st);
-    k_full_lnz<<<h->n_part_full, IG_THREADS, 0, st>>>(h->row_ptr, h->cv, h->coord, h->clen, h->ns, h->sc, mbar, 0, h->exz, h->part_full);
-    if (h->profile) cudaEventRecord(h->ev[3], st);
-    k_reduce<<<1, 256, 0, st>>>(h->part_full, h->n_part_full, &h->sc->lnz_full, nullptr, nullptr);
-    if (fork) cudaEventRecord(h->ev_lnz, st);
-    h->n_launches += 4;
-    h->coords_fresh = true; h->coords_ever = true;
-    return launch_ok(h, "refresh_current");
-}
-
 // k_score grid: the candidates of a step run side by side, so the resident capacity (3 CTAs per SM) is shared
 // between them -- one wave for the whole step instead of one (mostly latency) wave per candidate
 static int score_grid_x(const ig_handle* h, int n) {
@@ -677,28 +664,28 @@ static int score_grid_x(const ig_handle* h, int n) {
     return std::max(h->grid_score / std::max(n, 1), h->grid_score / 8) * h->grid_split;
 }
 
-// rows + precompute + scoring kernels of one step (after k_cand_setup / k_find_cuts / k_classes were enqueued);
-// in_step: event joins with the side streams and the profiling marks of enqueue_step
+// rows + precompute + scoring kernels of one pass (after k_cand_setup / k_find_cuts were enqueued, k_classes on h->pf)
 #define IG_MARK(i) do { if (h->profile && !h->capturing) cudaEventRecord(h->evk[i], h->stream); } while (0)
-static void enqueue_scoring(ig_handle* h, int n, bool in_step) {
+static void enqueue_scoring(ig_handle* h, int n) {
     const float mbar = h->cfg.mean_sub_len_kb;
     const FragRec* live = h->live;
     if (h->rows_small) {
-        if (in_step) IG_MARK(3);
+        IG_MARK(3);
         k_rows_small<<<n, IG_ROW_CHUNK, 0, h->stream>>>(h->coord, h->ns, h->sc, h->n_chunks, h->rows, h->rowidx, h->row_cnt, h->ns,
                                                         h->clstab, h->row_ptr, h->rinfo);
     } else {
         k_rows_count<<<h->n_chunks, IG_ROW_CHUNK, 0, h->stream>>>(h->coord, h->ns, h->sc, h->chunk_cnt, h->n_chunks);
-        if (in_step) IG_MARK(3);
+        IG_MARK(3);
         k_rows_write<<<h->n_chunks, IG_ROW_CHUNK, 0, h->stream>>>(h->coord, h->ns, h->sc, h->chunk_cnt, h->n_chunks, h->rows,
                                                                            h->rowidx, h->row_cnt, h->ns, h->clstab, h->row_ptr, h->rinfo,
                                                                            h->bitmap, h->bitmap_words, h->cls16);
     }
-    if (in_step) IG_MARK(4);
+    IG_MARK(4);
     k_precompute<<<dim3(h->grid_pre, n), IG_PRE_THREADS, 0, h->stream>>>(h->coord, h->clen, live, h->sub, h->sc, h->desc, h->rows, h->ns,
                                                                     h->table, h->table_len, mbar, h->part_z, h->part_i);
     if (h->profile && !h->capturing) cudaEventRecord(h->ev[4], h->stream);
-    if (in_step) { cudaStreamWaitEvent(h->stream, h->ev_cls, 0); IG_MARK(5); }
+    cudaStreamWaitEvent(h->stream, h->ev_cls, 0);
+    IG_MARK(5);
     const int gsx = h->flat ? h->grid_flat : score_grid_x(h, n);
     if (h->flat) {
         k_pick<<<dim3(gsx, n), IG_THREADS, 0, h->stream>>>(h->cv, h->coord, h->clen, h->sc, h->desc, h->rowidx, h->ns, h->row_cnt,
@@ -708,15 +695,13 @@ static void enqueue_scoring(ig_handle* h, int n, bool in_step) {
                                                                             h->flat_stride, h->table, h->table_len, mbar, h->exz, h->part_nz, h->clstab, h->flat_items);
     } else {
         // (streaming mode: k_score only works for the candidates k_stream leaves to it -- circular contigs, and in the
-        //  reference-faithful mode the candidates whose picks would not fit the list.  Inside a step it runs BESIDE the
-        //  streaming pair on the third stream -- different candidates, different partials -- and joins before k_finalize.)
+        //  reference-faithful mode the candidates whose picks would not fit the list.  It runs BESIDE the streaming pair on
+        //  the third stream -- different candidates, different partials -- and joins before k_finalize.)
         cudaStream_t ks = h->stream;
-        if (h->streaming && in_step) {
+        if (h->streaming) {
             ks = h->pf;   // (k_classes ran on it: already ordered)
             cudaEventRecord(h->ev_pre, h->stream);
             cudaStreamWaitEvent(ks, h->ev_pre, 0);
-        }
-        if (h->streaming) {
             k_stream<<<dim3(gsx, n), IG_THREADS, h->stream_smem, h->stream>>>(h->cv, h->coord, h->clen, h->sc, h->desc, h->rowidx, h->ns, h->row_cnt,
                                                                              h->bitmap, h->bitmap_words, h->cls16, h->part_c, h->pick_list, h->pick_cap,
                                                                              mbar, h->exz, h->clstab, h->subx, h->rinfo);
@@ -734,57 +719,45 @@ static void enqueue_scoring(ig_handle* h, int n, bool in_step) {
     if (h->profile && !h->capturing) cudaEventRecord(h->ev[5], h->stream);
 }
 
-static int score_candidates(ig_handle* h, int a, const int32_t* cands, int n, int first_flip_eject, bool overlap) {
-    if (n <= 0 || n > IG_MAX_CANDS) { h->err = "n_cands out of range"; return -1; }
-    if (a < 0 || a >= h->nf) { h->err = "id_frag out of range"; return -1; }
-    for (int i = 0; i < n; i++) if (cands[i] < 0 || cands[i] >= h->nf) { h->err = "candidate out of range"; return -1; }
-    const float mbar = h->cfg.mean_sub_len_kb;
-    int* hs = h->h_small;
-    hs[0] = n; hs[1] = a;
-    for (int i = 0; i < IG_MAX_CANDS; i++) hs[2 + i] = i < n ? cands[i] : 0;
-    CK(cudaMemcpyAsync(&h->sc->n_cands, hs, (2 + IG_MAX_CANDS) * sizeof(int), cudaMemcpyHostToDevice, h->stream));
-    const FragRec* live = h->live;
-    k_cand_setup<<<1, 32, 0, h->stream>>>(live, h->sc, h->desc, h->cfg.max_bounds_insert, first_flip_eject, nullptr, h->streaming ? h->stream_rows_max : 0);
-    k_find_cuts<<<(h->nf + 255) / 256, 256, 0, h->stream>>>(live, h->nf, h->sc, h->desc, h->clstab);
-    k_classes<<<n, IG_N_OPS * 32, 0, h->stream>>>(h->sc, h->desc, h->clstab, h->rigid, h->cfg.mean_sub_len_kb);
-    if (overlap) cudaStreamWaitEvent(h->stream, h->ev_coords, 0);
-    enqueue_scoring(h, n, false);
-    const int gsx = h->flat ? h->grid_flat : score_grid_x(h, n);
-    h->n_launches += 7;
-    if (overlap) cudaStreamWaitEvent(h->stream, h->ev_lnz, 0);
-    k_finalize<<<n, 1024, 0, h->stream>>>(h->row_ptr, h->cv, h->coord, h->sc, h->desc, h->rows, h->rowidx, h->ns, h->row_cnt, h->table,
-                                         h->table_len, mbar, h->exz, h->part_nz, h->part_c, h->flat ? h->grid_score : gsx, h->part_z, h->part_i,
-                                         h->grid_pre, h->cfg.n_pix, h->cfg.compat_last_block, h->d_nuniq, h->d_nsub, 0, gsx, h->flat ? 1 : 0);
-    return launch_ok(h, "score_candidates");
-}
-
 static int apply_and_post(ig_handle* h, int forced_cand, int forced_op) {
     const int nf = h->nf;
     h->label_hi += 2;
     k_apply<<<(nf + 255) / 256, 256, 0, h->stream>>>(h->live, nf, h->sc, h->desc, forced_cand, forced_op);
     k_post_scalars<<<1, 1, 0, h->stream>>>(h->sc, h->desc, forced_cand, forced_op);
-    k_post<<<(nf + 255) / 256, 256, 0, h->stream>>>(h->live, nf, h->init_prev, h->init_next, h->orientable, h->sc, nullptr, nullptr, nullptr);
+    k_post<<<(nf + 255) / 256, 256, 0, h->stream>>>(h->live, nf, h->init_prev, h->init_next, h->orientable, h->sc, nullptr);
     h->coords_fresh = false;
     h->n_launches += 3;
     return launch_ok(h, "apply");
 }
 
-static int fetch_result(ig_handle* h, int n, const int32_t* cands, ig_step_result* out, bool applied, bool copy = true) {
+// the result of the last step or scoring pass of n candidates from the scalar record (and the wide record beyond
+// IG_MAX_CANDS): `out` holds the first IG_MAX_CANDS candidates' values (applied: and the move), scores / n_uniq / n_sub
+// (where given) all n.  copy: download the scalar record first (a step enqueues that copy itself)
+static int fetch_result(ig_handle* h, int n, const int32_t* cands, ig_step_result* out, bool applied, bool copy = true,
+                        double* scores = nullptr, int32_t* n_uniq = nullptr, int32_t* n_sub = nullptr) {
     if (copy) {
         CK(cudaMemcpyAsync(h->h_sc, h->sc, sizeof(DevScalars), cudaMemcpyDeviceToHost, h->stream));
         CK(cudaStreamSynchronize(h->stream));
     }
     const DevScalars& s = *h->h_sc;
     if (s.list_overflow) { h->err = "pick list of the streaming scoring path overflowed (IG_PICK_CAP)"; return -4; }
+    const bool wide = n > IG_MAX_CANDS;
+    const double* sv = wide ? h->h_wide->scores : s.scores;
+    const int* nu = wide ? h->h_wide->n_uniq : s.res_nuniq;
+    const int* nsub = wide ? h->h_wide->n_sub : s.res_nsub;
+    const int m = std::min(n, IG_MAX_CANDS);
     memset(out, 0, sizeof *out);
-    for (int i = 0; i < n * IG_N_OPS; i++) out->scores[i] = s.scores[i];
+    for (int i = 0; i < m * IG_N_OPS; i++) out->scores[i] = sv[i];
+    for (int i = 0; i < m; i++) { out->n_uniq[i] = nu[i]; out->n_sub[i] = nsub[i]; }
+    if (scores) for (int i = 0; i < n * IG_N_OPS; i++) scores[i] = sv[i];
+    for (int i = 0; i < n; i++) { if (n_uniq) n_uniq[i] = nu[i]; if (n_sub) n_sub[i] = nsub[i]; }
     out->lnz_full = s.lnz_full;
-    for (int i = 0; i < n; i++) { out->n_uniq[i] = s.res_nuniq[i]; out->n_sub[i] = s.res_nsub[i]; }
     out->q4_hits = s.q4_hits;
     if (applied) {
+        const int win = wide ? h->h_wide->win_cand : s.win_cand;
         out->likelihood = s.likelihood;
-        out->cand_index = s.win_cand; out->op_sampled = s.win_op;
-        out->id_f_sampled = cands ? cands[s.win_cand] : -1;
+        out->cand_index = win; out->op_sampled = s.win_op;
+        out->id_f_sampled = cands[win];
         out->n_contigs = s.n_heads; out->sum_l_cont = s.sum_l_cont;
         out->dist = (3.0 * h->nf - 0.5 * (double)s.dist_half) / (3.0 * h->nf);
     }
@@ -855,13 +828,14 @@ static void enqueue_head(ig_handle* h, int full) {
         cudaEventRecord(h->ev_lnz, h->side);
     }
 }
-// one scoring pass over the candidates in sc (or in the cycle plan cyc_in): setup, row list, precompute, scoring, k_finalize
-// (do_select: with the move selection); wide_rescore: the re-score of a wide step's winning batch (k_wide_flip)
-static void enqueue_pass(ig_handle* h, int n, int first_flip_eject, const int* cyc_in, int do_select, bool wide_rescore = false) {
+// one scoring pass over the candidates in sc (or, plan != nullptr, in the cycle plan's entry sc->step_idx): setup, row list,
+// precompute, scoring, k_finalize (do_select: with the move selection); wide_rescore: the re-score of a wide step's winning
+// batch (k_wide_flip)
+static void enqueue_pass(ig_handle* h, int n, int first_flip_eject, const int* plan, int do_select, bool wide_rescore = false) {
     const float mbar = h->cfg.mean_sub_len_kb;
     const FragRec* live = h->live;
     IG_MARK(0);
-    k_cand_setup<<<1, 32, 0, h->stream>>>(live, h->sc, h->desc, h->cfg.max_bounds_insert, first_flip_eject, cyc_in, h->streaming ? h->stream_rows_max : 0);
+    k_cand_setup<<<1, 32, 0, h->stream>>>(live, h->sc, h->desc, h->cfg.max_bounds_insert, first_flip_eject, plan, h->streaming ? h->stream_rows_max : 0);
     if (wide_rescore) k_wide_flip<<<1, 32, 0, h->stream>>>(h->sc, h->desc, h->wide);
     IG_MARK(1);
     k_find_cuts<<<(h->nf + 255) / 256, 256, 0, h->stream>>>(live, h->nf, h->sc, h->desc, h->clstab);
@@ -871,7 +845,7 @@ static void enqueue_pass(ig_handle* h, int n, int first_flip_eject, const int* c
     cudaEventRecord(h->ev_cls, h->pf);
     cudaStreamWaitEvent(h->stream, h->ev_coords, 0);
     IG_MARK(2);
-    enqueue_scoring(h, n, true);
+    enqueue_scoring(h, n);
     const int gsx = h->flat ? h->grid_flat : score_grid_x(h, n);
     cudaStreamWaitEvent(h->stream, h->ev_lnz, 0);
     IG_MARK(6);
@@ -896,35 +870,34 @@ static void enqueue_tail(ig_handle* h, int cycle) {
     k_apply<<<(h->nf + 255) / 256, 256, 0, h->stream>>>(h->live, h->nf, h->sc, h->desc, -1, -1);
     IG_MARK(10);
     k_post<<<(h->nf + 255) / 256, 256, 0, h->stream>>>(h->live, h->nf, h->init_prev, h->init_next, h->orientable, h->sc,
-                                                       cycle ? h->cyc_out : nullptr, h->d_nuniq, h->d_nsub);
+                                                       cycle ? h->cyc_out : nullptr);
     IG_MARK(11);
     cudaStreamWaitEvent(h->stream, h->ev_out, 0);
 }
-static int enqueue_step(ig_handle* h, int full, int n_grid_cands, int cycle = 0) {
+// Everything one step enqueues (no host synchronisation): used directly and under graph capture.  The candidates come from
+// the cycle plan (cycle: the step also writes its record) or from the pinned staging of the host step (h_small, h_wide->in).
+// A step of up to IG_MAX_CANDS candidates: one selecting pass over its grid_n candidate slots.
+static void enqueue_step(ig_handle* h, int full, int grid_n, int cycle) {
     if (!cycle) cudaMemcpyAsync(&h->sc->n_cands, h->h_small, (2 + IG_MAX_CANDS) * sizeof(int), cudaMemcpyHostToDevice, h->stream);
     enqueue_head(h, full);
-    enqueue_pass(h, n_grid_cands, 1, cycle ? h->cyc_in : nullptr, 1);
+    enqueue_pass(h, grid_n, 1, cycle ? h->cyc_plan : nullptr, 1);
     enqueue_tail(h, cycle);
-    if (!cycle) {
-        cudaMemcpyAsync(h->h_sc, h->sc, sizeof(DevScalars), cudaMemcpyDeviceToHost, h->stream);
-    }
-    return launch_ok(h, "enqueue_step");
+    if (!cycle) cudaMemcpyAsync(h->h_sc, h->sc, sizeof(DevScalars), cudaMemcpyDeviceToHost, h->stream);
 }
 // A step of n_batches * IG_MAX_CANDS candidate slots (ig_k_wide.cuh): the head once, one score-only pass per batch, the
 // winning batch scored again with the selecting tail.  Every pass is launched for a full batch (the grid of IG_MAX_CANDS
 // candidates, whatever the batch holds), so the re-score repeats its batch's pass launch for launch and its scores, hence
-// its selection, are bit-identical to that pass's.  The candidates come from the cycle plan cyc_wide (cycle) or h->wide->in.
-static int enqueue_wide_step(ig_handle* h, int full, int n_batches, int cycle) {
-    const int* plan = cycle ? h->cyc_wide : nullptr;
-    const int width = h->plan_width;
+// its selection, are bit-identical to that pass's.
+static void enqueue_wide_step(ig_handle* h, int full, int n_batches, int cycle) {
+    const int* plan = cycle ? h->cyc_plan : nullptr;
     if (!cycle) cudaMemcpyAsync(h->wide->in, h->h_wide->in, sizeof(h->wide->in), cudaMemcpyHostToDevice, h->stream);
     enqueue_head(h, full);
     for (int b = 0; b < n_batches; b++) {
-        k_wide_stage<<<1, 32, 0, h->stream>>>(h->sc, h->wide, plan, width, b);
+        k_wide_stage<<<1, 32, 0, h->stream>>>(h->sc, h->wide, plan, b);
         enqueue_pass(h, IG_MAX_CANDS, b == 0 ? 1 : 0, nullptr, 0);
         k_wide_stash<<<1, 256, 0, h->stream>>>(h->sc, h->wide, b);
     }
-    k_wide_pick<<<1, 32, 0, h->stream>>>(h->sc, h->wide, plan, width);
+    k_wide_pick<<<1, 32, 0, h->stream>>>(h->sc, h->wide, plan);
     enqueue_pass(h, IG_MAX_CANDS, 1, nullptr, 1, true);
     enqueue_tail(h, cycle);
     k_wide_finish<<<1, 32, 0, h->stream>>>(h->sc, h->wide, cycle ? h->cyc_out : nullptr);
@@ -932,11 +905,15 @@ static int enqueue_wide_step(ig_handle* h, int full, int n_batches, int cycle) {
         cudaMemcpyAsync(h->h_sc, h->sc, sizeof(DevScalars), cudaMemcpyDeviceToHost, h->stream);
         cudaMemcpyAsync(h->h_wide, h->wide, sizeof(WideStep), cudaMemcpyDeviceToHost, h->stream);
     }
-    return launch_ok(h, "enqueue_wide_step");
 }
-#define IG_LAUNCHES_FULL 15
-#define IG_LAUNCHES_INCR 12
-#define IG_LAUNCHES_LITE 17
+static int n_batches_of(int n) { return (n + IG_MAX_CANDS - 1) / IG_MAX_CANDS; }
+// the launches of a step of grid_n candidate slots
+static int enqueue_any_step(ig_handle* h, int full, int grid_n, int cycle) {
+    if (grid_n > IG_MAX_CANDS) enqueue_wide_step(h, full, n_batches_of(grid_n), cycle);
+    else enqueue_step(h, full, grid_n, cycle);
+    return launch_ok(h, "enqueue_step");
+}
+
 // 0: incremental step; 1: coordinates and likelihood sums from scratch (scaffold replaced from outside, periodic refresh);
 // 2: likelihood sums only (parameters changed; needs the per-contact records and v_inter > 0, which the records assume);
 // 3: kind 2 decided on the device (a step after a production-mode nuisance step: see enqueue_plan_step)
@@ -945,97 +922,83 @@ static int step_kind(const ig_handle* h) {
     if (h->lnz_stale) return (h->lnz_cache && h->vinter_pos) ? 2 : 1;
     return 0;
 }
-static int step_launches(const ig_handle* h, int kind) {
-    return (kind >= 2 ? IG_LAUNCHES_LITE : kind ? IG_LAUNCHES_FULL : IG_LAUNCHES_INCR) - (h->rigid ? 1 : 0) + (h->prefetch ? 1 : 0) - (h->rows_small ? 1 : 0) + (h->flat ? 1 : 0) + (h->streaming ? 2 : 0);
+// kernel launches of enqueue_head (per kind) and of one enqueue_pass
+static int head_launches(const ig_handle* h, int kind) { return (h->prefetch ? 1 : 0) + (kind >= 2 ? 6 : kind ? 4 : 1); }
+static int pass_launches(const ig_handle* h) { return 8 - (h->rows_small ? 1 : 0) + (h->flat ? 1 : 0) + (h->streaming ? 2 : 0); }
+// ... of a step of grid_n candidate slots: head, pass, tail (k_lnz_outside unless rigid, k_apply, k_post); a wide step adds
+// one pass with k_wide_stage and k_wide_stash per batch, and k_wide_pick, k_wide_flip, k_wide_finish
+static int step_launches(const ig_handle* h, int kind, int grid_n) {
+    const int wide = grid_n > IG_MAX_CANDS ? n_batches_of(grid_n) * (pass_launches(h) + 2) + 3 : 0;
+    return head_launches(h, kind) + pass_launches(h) + (h->rigid ? 2 : 3) + wide;
 }
 
-static int get_graph(ig_handle* h, int full, cudaGraphExec_t* out, int cycle, int n) {
-    cudaGraphExec_t& ge = h->graph[full + 4 * cycle][n];
-    if (!ge && !h->graph_failed) {
-        cudaGraph_t g = nullptr;
-        h->capturing = true;
-        cudaError_t e = cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal);
-        if (e == cudaSuccess) {
-            enqueue_step(h, full, n, cycle);
-            e = cudaStreamEndCapture(h->stream, &g);
-        }
-        h->capturing = false;
-        if (e == cudaSuccess && g) e = cudaGraphInstantiate(&ge, g, 0);
-        if (g) cudaGraphDestroy(g);
-        if (e != cudaSuccess || !ge) { ge = nullptr; h->graph_failed = true; cudaGetLastError(); }
+// capture what `enqueue` launches on the handle's stream into `exec`; a failed capture leaves it null and sets `failed`
+// (the caller then launches directly)
+template <class F>
+static void capture(ig_handle* h, cudaGraphExec_t& exec, bool& failed, F enqueue) {
+    cudaGraph_t g = nullptr;
+    h->capturing = true;
+    cudaError_t e = cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal);
+    if (e == cudaSuccess) {
+        enqueue();
+        e = cudaStreamEndCapture(h->stream, &g);
     }
-    *out = ge;
+    h->capturing = false;
+    if (e == cudaSuccess && g) e = cudaGraphInstantiate(&exec, g, 0);
+    if (g) cudaGraphDestroy(g);
+    if (e != cudaSuccess || !exec) { exec = nullptr; failed = true; cudaGetLastError(); }
+}
+// the graph of a step of grid_n candidate slots (captured on first use; nullptr once a capture failed)
+static cudaGraphExec_t get_graph(ig_handle* h, int full, int grid_n, int cycle) {
+    cudaGraphExec_t& ge = h->graph[full + 4 * cycle][grid_n <= IG_MAX_CANDS ? grid_n : IG_MAX_CANDS + n_batches_of(grid_n)];
+    if (!ge && !h->graph_failed) capture(h, ge, h->graph_failed, [&] { enqueue_any_step(h, full, grid_n, cycle); });
+    return ge;
+}
+// one step on the handle's stream: the graph ge (get_graph), or its launches when there is none
+static int launch_step(ig_handle* h, cudaGraphExec_t ge, int full, int grid_n, int cycle) {
+    if (ge) { CK(cudaGraphLaunch(ge, h->stream)); }
+    else if (enqueue_any_step(h, full, grid_n, cycle)) return -2;
+    h->n_launches += step_launches(h, full, grid_n);
     return 0;
 }
-
-// wide steps: one graph per (kind, cycle, number of batches), in a cache of their own
-static int get_wide_graph(ig_handle* h, int full, cudaGraphExec_t* out, int cycle, int n_batches) {
-    cudaGraphExec_t& ge = h->graph_wide[full + 4 * cycle][n_batches];
-    if (!ge && !h->graph_failed) {
-        cudaGraph_t g = nullptr;
-        h->capturing = true;
-        cudaError_t e = cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal);
-        if (e == cudaSuccess) {
-            enqueue_wide_step(h, full, n_batches, cycle);
-            e = cudaStreamEndCapture(h->stream, &g);
-        }
-        h->capturing = false;
-        if (e == cudaSuccess && g) e = cudaGraphInstantiate(&ge, g, 0);
-        if (g) cudaGraphDestroy(g);
-        if (e != cudaSuccess || !ge) { ge = nullptr; h->graph_failed = true; cudaGetLastError(); }
-    }
-    *out = ge;
-    return 0;
-}
-static void destroy_wide_graphs(ig_handle* h, int first_kind_slot) {
-    for (int i = first_kind_slot; i < 8; i++)
-        for (int j = 0; j <= IG_MAX_BATCHES; j++) if (h->graph_wide[i][j]) { cudaGraphExecDestroy(h->graph_wide[i][j]); h->graph_wide[i][j] = nullptr; }
-}
-static int wide_alloc(ig_handle* h) {
-    if (h->wide) return 0;
-    if (dev_alloc(h, &h->wide, 1)) return -2;
-    CK(cudaMallocHost((void**)&h->h_wide, sizeof(WideStep)));
-    memset(h->h_wide, 0, sizeof(WideStep));
-    return 0;
-}
-static int n_batches_of(int n) { return (n + IG_MAX_CANDS - 1) / IG_MAX_CANDS; }
-// launches of a wide step: the narrow step's, plus one pass and the two wide kernels around it per batch, plus the re-score's
-// k_wide_pick / k_wide_flip and k_wide_finish
-static int wide_step_launches(const ig_handle* h, int kind, int n_batches) {
-    const int pass = step_launches(h, 0) - 3 - (h->rigid ? 0 : 1) - (h->prefetch ? 1 : 0);   // minus k_commit_coords, tail, prefetch
-    return step_launches(h, kind) + n_batches * (pass + 2) + 3;
+// the handle's bookkeeping after a step of kind `kind` (host step or plan step; kind 3 counts as incremental)
+static void after_step(ig_handle* h, int kind) {
+    const bool refresh = kind == 1 || kind == 2;
+    h->steps_since_full = refresh ? 1 : h->steps_since_full + 1;
+    h->n_full += refresh ? 1 : 0;
+    h->incr_valid = true; h->lnz_stale = false;
+    h->coords_fresh = false; h->coords_ever = true;
 }
 
 extern "C" int ig_step(ig_handle* h, int32_t id_frag, const int32_t* cands, int32_t n_cands, ig_step_result* out) {
     if (use(h)) return -1;
-    if (!h->params_set) { h->err = "ig_step: parameters not set (ig_set_params)"; return -1; }
-    if (!out) { h->err = "ig_step: null result"; return -1; }
     if (n_cands <= 0 || n_cands > IG_MAX_CANDS) { h->err = "n_cands out of range"; return -1; }
+    return ig_step_wide(h, id_frag, cands, n_cands, out, nullptr, nullptr, nullptr);
+}
+
+// step_sampler: enqueue_step up to IG_MAX_CANDS candidates, enqueue_wide_step beyond
+extern "C" int ig_step_wide(ig_handle* h, int32_t id_frag, const int32_t* cands, int32_t n_cands, ig_step_result* out, double* scores,
+                            int32_t* n_uniq, int32_t* n_sub) {
+    if (use(h)) return -1;
+    if (!out || !cands) { h->err = "ig_step_wide: null argument"; return -1; }
+    if (n_cands <= 0 || n_cands > IG_MAX_NEIGHBOURS) { h->err = "ig_step_wide: n_cands out of range (1 .. IG_MAX_NEIGHBOURS = 64)"; return -1; }
+    if (!h->params_set) { h->err = "ig_step: parameters not set (ig_set_params)"; return -1; }
     if (id_frag < 0 || id_frag >= h->nf) { h->err = "id_frag out of range"; return -1; }
     for (int i = 0; i < n_cands; i++) if (cands[i] < 0 || cands[i] >= h->nf) { h->err = "candidate out of range"; return -1; }
     for (int i = 0; i < n_cands; i++) if (cands[i] == id_frag) { h->err = "candidate equals the visited fragment (reference quirk Q4; see DESIGN.md D1)"; return -1; }
     if (int rc = labels_guard(h)) return rc;
-    int* hs = h->h_small;
-    hs[0] = n_cands; hs[1] = id_frag;
-    for (int i = 0; i < IG_MAX_CANDS; i++) hs[2 + i] = i < n_cands ? cands[i] : 0;
+    const bool wide = n_cands > IG_MAX_CANDS;
+    int* in = wide ? h->h_wide->in : h->h_small;
+    in[0] = n_cands; in[1] = id_frag;
+    for (int i = 0; i < (wide ? IG_MAX_NEIGHBOURS : IG_MAX_CANDS); i++) in[2 + i] = i < n_cands ? cands[i] : 0;
     const int full = step_kind(h);
-    cudaGraphExec_t ge = nullptr;
-    if (h->use_graph && !h->profile) get_graph(h, full, &ge, 0, n_cands);
+    cudaGraphExec_t ge = (h->use_graph && !h->profile) ? get_graph(h, full, n_cands, 0) : nullptr;   // (profiling: per-kernel marks)
     cudaEventRecord(h->ev[0], h->stream);
-    if (ge) {
-        CK(cudaGraphLaunch(ge, h->stream));
-    } else {
-        if (enqueue_step(h, full, n_cands)) return -2;
-    }
+    if (int rc = launch_step(h, ge, full, n_cands, 0)) return rc;
     cudaEventRecord(h->ev[1], h->stream);
     CK(cudaStreamSynchronize(h->stream));
-    h->n_launches += step_launches(h, full);
-    h->steps_since_full = full ? 1 : h->steps_since_full + 1;
-    h->n_full += full ? 1 : 0;
-    h->incr_valid = true; h->lnz_stale = false;
-    h->coords_fresh = false; h->coords_ever = true;
-    int rc = fetch_result(h, n_cands, cands, out, true, false);
-    if (rc) return rc;
+    after_step(h, full);
+    if (int rc = fetch_result(h, n_cands, cands, out, true, false, scores, n_uniq, n_sub)) return rc;
     float ms = 0.f;
     if (cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]) == cudaSuccess) h->ms_step += ms;
     if (h->profile) {
@@ -1048,104 +1011,28 @@ extern "C" int ig_step(ig_handle* h, int32_t id_frag, const int32_t* cands, int3
     return 0;
 }
 
-// step_sampler with more than IG_MAX_CANDS candidates (enqueue_wide_step); up to IG_MAX_CANDS it is ig_step
-extern "C" int ig_step_wide(ig_handle* h, int32_t id_frag, const int32_t* cands, int32_t n_cands, ig_step_result* out, double* scores,
-                            int32_t* n_uniq, int32_t* n_sub) {
-    if (use(h)) return -1;
-    if (!out || !cands) { h->err = "ig_step_wide: null argument"; return -1; }
-    if (n_cands <= 0 || n_cands > IG_MAX_NEIGHBOURS) { h->err = "ig_step_wide: n_cands out of range (1 .. IG_MAX_NEIGHBOURS = 64)"; return -1; }
-    if (n_cands <= IG_MAX_CANDS) {
-        if (int rc = ig_step(h, id_frag, cands, n_cands, out)) return rc;
-        for (int i = 0; i < n_cands * IG_N_OPS; i++) if (scores) scores[i] = out->scores[i];
-        for (int i = 0; i < n_cands; i++) { if (n_uniq) n_uniq[i] = out->n_uniq[i]; if (n_sub) n_sub[i] = out->n_sub[i]; }
-        return 0;
-    }
-    if (!h->params_set) { h->err = "ig_step_wide: parameters not set (ig_set_params)"; return -1; }
-    if (id_frag < 0 || id_frag >= h->nf) { h->err = "id_frag out of range"; return -1; }
-    for (int i = 0; i < n_cands; i++) if (cands[i] < 0 || cands[i] >= h->nf) { h->err = "candidate out of range"; return -1; }
-    for (int i = 0; i < n_cands; i++) if (cands[i] == id_frag) { h->err = "candidate equals the visited fragment (reference quirk Q4; see DESIGN.md D1)"; return -1; }
-    if (int rc = wide_alloc(h)) return rc;
-    if (int rc = labels_guard(h)) return rc;
-    int* in = h->h_wide->in;
-    in[0] = n_cands; in[1] = id_frag;
-    for (int i = 0; i < IG_MAX_NEIGHBOURS; i++) in[2 + i] = i < n_cands ? cands[i] : 0;
-    const int full = step_kind(h);
-    const int nb = n_batches_of(n_cands);
-    cudaGraphExec_t ge = nullptr;
-    if (h->use_graph && !h->profile) get_wide_graph(h, full, &ge, 0, nb);
-    cudaEventRecord(h->ev[0], h->stream);
-    if (ge) {
-        CK(cudaGraphLaunch(ge, h->stream));
-    } else {
-        if (enqueue_wide_step(h, full, nb, 0)) return -2;
-    }
-    cudaEventRecord(h->ev[1], h->stream);
-    CK(cudaStreamSynchronize(h->stream));
-    h->n_launches += wide_step_launches(h, full, nb);
-    h->steps_since_full = full ? 1 : h->steps_since_full + 1;
-    h->n_full += full ? 1 : 0;
-    h->incr_valid = true; h->lnz_stale = false;
-    h->coords_fresh = false; h->coords_ever = true;
-    const DevScalars& sres = *h->h_sc;
-    const WideStep& w = *h->h_wide;
-    if (sres.list_overflow) { h->err = "pick list of the streaming scoring path overflowed (IG_PICK_CAP)"; return -4; }
-    memset(out, 0, sizeof *out);
-    for (int i = 0; i < IG_MAX_CANDS * IG_N_OPS; i++) out->scores[i] = w.scores[i];
-    for (int i = 0; i < IG_MAX_CANDS; i++) { out->n_uniq[i] = w.n_uniq[i]; out->n_sub[i] = w.n_sub[i]; }
-    if (scores) for (int i = 0; i < n_cands * IG_N_OPS; i++) scores[i] = w.scores[i];
-    for (int i = 0; i < n_cands; i++) { if (n_uniq) n_uniq[i] = w.n_uniq[i]; if (n_sub) n_sub[i] = w.n_sub[i]; }
-    out->lnz_full = sres.lnz_full; out->q4_hits = sres.q4_hits;
-    out->likelihood = sres.likelihood;
-    out->cand_index = w.win_cand; out->op_sampled = sres.win_op;
-    out->id_f_sampled = cands[w.win_cand];
-    out->n_contigs = sres.n_heads; out->sum_l_cont = sres.sum_l_cont;
-    out->dist = (3.0 * h->nf - 0.5 * (double)sres.dist_half) / (3.0 * h->nf);
-    float ms = 0.f;
-    if (cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]) == cudaSuccess) h->ms_step += ms;
-    h->n_steps++;
-    return 0;
-}
-
 // A whole MCMC cycle (or any run of steps) enqueued without a single host synchronisation in between:
 // the host uploads the plan {fragment, sorted candidates} of every step (drawn with the reference's own
 // RNG calls, which do not depend on the chain state), every step is one CUDA-graph replay that reads its
 // plan entry and writes a compact record on the device, and the host synchronises once at the end.
 // Semantically identical to n_steps calls of ig_step (IG.full_em inner loop, instagraal.py:217-241).
-static int cycle_buffers(ig_handle* h, int n_steps) {
-    if (n_steps > h->cyc_cap) {
-        if (h->cyc_in) cudaFree(h->cyc_in);
-        if (h->cyc_out) cudaFree(h->cyc_out);
-        if (h->cyc_frags) cudaFree(h->cyc_frags);
-        if (h->nuis_rec) cudaFree(h->nuis_rec);
-        h->cyc_in = nullptr; h->cyc_out = nullptr; h->cyc_frags = nullptr; h->nuis_rec = nullptr; h->cyc_cap = 0;
-        for (int i = 4; i < 8; i++) for (int j = 0; j <= IG_MAX_CANDS; j++) if (h->graph[i][j]) { cudaGraphExecDestroy(h->graph[i][j]); h->graph[i][j] = nullptr; }  // pointers are baked in
-        destroy_wide_graphs(h, 4);
-        if (h->graph_nuis_dev) { cudaGraphExecDestroy(h->graph_nuis_dev); h->graph_nuis_dev = nullptr; }
-        if (dev_alloc(h, &h->cyc_in, (size_t)n_steps * (2 + IG_MAX_CANDS)) || dev_alloc(h, &h->cyc_out, (size_t)n_steps) ||
-            dev_alloc(h, &h->cyc_frags, (size_t)n_steps) || dev_alloc(h, &h->nuis_rec, (size_t)n_steps)) return -2;
-        h->cyc_cap = n_steps;
-    }
-    return 0;
-}
-// the plan of a wide cycle: [n_steps][2 + width] (the stride is baked into the cycle graphs of wide steps)
-static int wide_plan_buffers(ig_handle* h, int n_steps, int width) {
-    if (int rc = wide_alloc(h)) return rc;
-    const size_t need = (size_t)n_steps * (2 + width);
-    if (need > h->cyc_wide_cap || width != h->plan_width) destroy_wide_graphs(h, 4);
-    if (need > h->cyc_wide_cap) {
-        if (h->cyc_wide) cudaFree(h->cyc_wide);
-        h->cyc_wide = nullptr; h->cyc_wide_cap = 0;
-        if (dev_alloc(h, &h->cyc_wide, need)) return -2;
-        h->cyc_wide_cap = need;
+
+// The buffers of a cycle of n_steps steps whose plan entries hold `width` candidate slots: the plan [n_steps][2 + width],
+// the step records, the visiting order, the nuisance records.  They only grow; the cycle graphs bake them in.
+static int cycle_buffers(ig_handle* h, int n_steps, int width) {
+    if (n_steps > h->cyc_cap || width > h->cyc_width) {
+        const int cap = std::max(n_steps, h->cyc_cap), w = std::max(width, h->cyc_width);
+        for (void* q : {(void*)h->cyc_plan, (void*)h->cyc_out, (void*)h->cyc_frags, (void*)h->nuis_rec}) if (q) cudaFree(q);
+        h->cyc_plan = nullptr; h->cyc_out = nullptr; h->cyc_frags = nullptr; h->nuis_rec = nullptr; h->cyc_cap = 0; h->cyc_width = 0;
+        destroy_graphs(h, 4);
+        if (dev_alloc(h, &h->cyc_plan, (size_t)cap * (2 + w)) || dev_alloc(h, &h->cyc_out, (size_t)cap) ||
+            dev_alloc(h, &h->cyc_frags, (size_t)cap) || dev_alloc(h, &h->nuis_rec, (size_t)cap)) return -2;
+        h->cyc_cap = cap; h->cyc_width = w;
     }
     h->plan_width = width;
     return 0;
 }
 
-// replay n_steps steps from the plan in h->cyc_in (already on the device, or being written by an earlier kernel of
-// the stream); grid_n(t) = number of candidate slots the step's grid is built for
-// one step of the plan in h->cyc_in enqueued on the handle's stream (CUDA-graph replay); grid_n = number of candidate
-// slots the step's grid is built for
 // the nuisance step of the production mode (ig_k_nuis.cuh) after the step just enqueued: propose, evaluate the proposal
 // with exactly the launches of ig_full_likelihood(p_test, use_stale_coords = 1), decide, promote, record
 static void enqueue_nuisance(ig_handle* h) {
@@ -1165,45 +1052,22 @@ static void enqueue_nuisance(ig_handle* h) {
 }
 #define IG_LAUNCHES_NUIS 9
 static int launch_nuisance(ig_handle* h) {
-    if (h->use_graph && !h->graph_nuis_dev && !h->nuis_graph_dev_failed) {
-        cudaGraph_t g = nullptr;
-        cudaError_t e = cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal);
-        if (e == cudaSuccess) {
-            enqueue_nuisance(h);
-            e = cudaStreamEndCapture(h->stream, &g);
-        }
-        if (e == cudaSuccess && g) e = cudaGraphInstantiate(&h->graph_nuis_dev, g, 0);
-        if (g) cudaGraphDestroy(g);
-        if (e != cudaSuccess || !h->graph_nuis_dev) { h->graph_nuis_dev = nullptr; h->nuis_graph_dev_failed = true; cudaGetLastError(); }
-    }
+    if (h->use_graph && !h->graph_nuis_dev && !h->nuis_graph_dev_failed)
+        capture(h, h->graph_nuis_dev, h->nuis_graph_dev_failed, [&] { enqueue_nuisance(h); });
     if (h->use_graph && h->graph_nuis_dev) { CK(cudaGraphLaunch(h->graph_nuis_dev, h->stream)); }
     else enqueue_nuisance(h);
     h->n_launches += IG_LAUNCHES_NUIS;
     return launch_ok(h, "nuisance step");
 }
-// grid_n > IG_MAX_CANDS: a wide step of n_batches_of(grid_n) batches from the wide plan
+// the plan's next step (entry sc->step_idx) on the handle's stream, its grid built for grid_n candidate slots (a wide step
+// beyond IG_MAX_CANDS), then the production-mode nuisance step when it is on
 static int enqueue_plan_step(ig_handle* h, int grid_n) {
     if (int rc = labels_guard(h)) return rc;
     int full = step_kind(h);
     // after a nuisance step of this plan the host cannot know whether the parameters changed: kind 3 decides on the device
     if (full == 0 && h->nuis_on && h->nuis_enqueued) full = 3;
-    cudaGraphExec_t ge = nullptr;
-    if (grid_n > IG_MAX_CANDS) {
-        const int nb = n_batches_of(grid_n);
-        if (h->use_graph) get_wide_graph(h, full, &ge, 1, nb);
-        if (ge) { CK(cudaGraphLaunch(ge, h->stream)); }
-        else if (enqueue_wide_step(h, full, nb, 1)) return -2;
-        h->n_launches += wide_step_launches(h, full, nb);
-    } else {
-        if (h->use_graph) get_graph(h, full, &ge, 1, grid_n);
-        if (ge) { CK(cudaGraphLaunch(ge, h->stream)); }
-        else if (enqueue_step(h, full, grid_n, 1)) return -2;
-        h->n_launches += step_launches(h, full);
-    }
-    const bool refresh = full == 1 || full == 2;
-    h->steps_since_full = refresh ? 1 : h->steps_since_full + 1;
-    h->n_full += refresh ? 1 : 0;
-    h->incr_valid = true; h->lnz_stale = false;
+    if (int rc = launch_step(h, h->use_graph ? get_graph(h, full, grid_n, 1) : nullptr, full, grid_n, 1)) return rc;
+    after_step(h, full);
     if (h->nuis_on) {
         if (int rc = launch_nuisance(h)) return rc;
         h->nuis_enqueued = true;
@@ -1219,15 +1083,10 @@ static int begin_plan(ig_handle* h) {
 static int collect_plan(ig_handle* h, int n_steps, ig_cycle_step* out) {
     cudaEventRecord(h->ev[1], h->stream);
     std::vector<CycleOut> res(n_steps);
-    const int stride = 2 + h->plan_width;   // wide cycles: the wide plan holds every step
-    std::vector<int> plan((size_t)n_steps * stride);
     int overflow = 0;
     CK(cudaMemcpyAsync(res.data(), h->cyc_out, sizeof(CycleOut) * n_steps, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaMemcpyAsync(plan.data(), h->plan_width > IG_MAX_CANDS ? h->cyc_wide : h->cyc_in, plan.size() * sizeof(int),
-                       cudaMemcpyDeviceToHost, h->stream));
     CK(cudaMemcpyAsync(&overflow, &h->sc->list_overflow, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    h->coords_fresh = false; h->coords_ever = true;
     h->pending_steps = 0;
     if (h->nuis_on && h->nuis_enqueued) {
         // the last step's nuisance decision: an accepted proposal leaves the sums stale for the next step (ig_step or the
@@ -1247,15 +1106,12 @@ static int collect_plan(ig_handle* h, int n_steps, ig_cycle_step* out) {
     h->n_steps += n_steps;
     for (int t = 0; t < n_steps; t++) {
         const CycleOut& r = res[t];
-        const int* pl = &plan[(size_t)t * stride];
         ig_cycle_step& o = out[t];
         o.likelihood = r.likelihood; o.lnz_full = r.lnz_full;
         o.dist = (3.0 * h->nf - 0.5 * (double)r.dist_half) / (3.0 * h->nf);
         o.sum_l_cont = r.sum_l_cont; o.n_contigs = r.n_heads; o.op_sampled = r.win_op; o.cand_index = r.win_cand;
-        o.id_f_sampled = pl[2 + r.win_cand];
-        o.q4_hits = r.q4_hits; o.n_proposals = 0;
-        if (r.pad[1]) o.n_proposals = r.pad[0];   // a wide step (k_wide_finish): every batch's proposals
-        else for (int i = 0; i < pl[0]; i++) o.n_proposals += r.n_uniq[i];
+        o.id_f_sampled = r.id_f_sampled;
+        o.q4_hits = r.q4_hits; o.n_proposals = r.n_proposals;
     }
     return 0;
 }
@@ -1270,9 +1126,8 @@ extern "C" int ig_run_cycle(ig_handle* h, int32_t n_steps, const int32_t* frags,
                             ig_cycle_step* out) {
     return ig_run_cycle_wide(h, n_steps, frags, cands8, IG_MAX_CANDS, n_cands, out);
 }
-// cands = [n_steps][width].  A cycle whose steps all have at most IG_MAX_CANDS candidates runs from the narrow plan (cyc_in);
-// otherwise the wide plan (stride 2 + width) holds every step, steps of more than IG_MAX_CANDS candidates run as wide steps and
-// the others as narrow steps from the narrow plan, which then holds their entries (both plans are read at entry step_idx)
+// cands = [n_steps][width].  The plan holds every step at the stride 2 + W, W = max(IG_MAX_CANDS, longest list): a step of
+// more than IG_MAX_CANDS candidates runs as a wide step, the others as narrow steps of their own size
 extern "C" int ig_run_cycle_wide(ig_handle* h, int32_t n_steps, const int32_t* frags, const int32_t* cands, int32_t width,
                                  const int32_t* n_cands, ig_cycle_step* out) {
     if (use(h)) return -1;
@@ -1292,30 +1147,16 @@ extern "C" int ig_run_cycle_wide(ig_handle* h, int32_t n_steps, const int32_t* f
         }
         n_max = std::max(n_max, n);
     }
-    const bool wide = n_max > IG_MAX_CANDS;
-    std::vector<int> plan((size_t)n_steps * (2 + IG_MAX_CANDS), 0);
+    const int w = std::max(IG_MAX_CANDS, n_max), stride = 2 + w;
+    std::vector<int> plan((size_t)n_steps * stride, 0);
     for (int t = 0; t < n_steps; t++) {
-        const int n = n_cands[t];
-        if (n > IG_MAX_CANDS) continue;
-        int* p = &plan[(size_t)t * (2 + IG_MAX_CANDS)];
-        p[0] = n; p[1] = frags[t];
-        for (int i = 0; i < n; i++) p[2 + i] = cands[(size_t)t * width + i];
+        int* p = &plan[(size_t)t * stride];
+        p[0] = n_cands[t]; p[1] = frags[t];
+        for (int i = 0; i < n_cands[t]; i++) p[2 + i] = cands[(size_t)t * width + i];
     }
-    if (cycle_buffers(h, n_steps)) return -2;
-    CK(cudaMemcpyAsync(h->cyc_in, plan.data(), plan.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
-    if (wide) {
-        if (wide_plan_buffers(h, n_steps, width)) return -2;
-        std::vector<int> wp((size_t)n_steps * (2 + width), 0);
-        for (int t = 0; t < n_steps; t++) {
-            int* p = &wp[(size_t)t * (2 + width)];
-            p[0] = n_cands[t]; p[1] = frags[t];
-            for (int i = 0; i < n_cands[t]; i++) p[2 + i] = cands[(size_t)t * width + i];
-        }
-        CK(cudaMemcpyAsync(h->cyc_wide, wp.data(), wp.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
-        CK(cudaStreamSynchronize(h->stream));   // (pageable source)
-    } else {
-        h->plan_width = IG_MAX_CANDS;
-    }
+    if (cycle_buffers(h, n_steps, w)) return -2;
+    CK(cudaMemcpyAsync(h->cyc_plan, plan.data(), plan.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(&h->sc->plan_stride, &stride, sizeof(int), cudaMemcpyHostToDevice, h->stream));
     return run_plan(h, n_steps, [&](int t) { return n_cands[t]; }, out);
 }
 
@@ -1353,22 +1194,17 @@ static int prepare_device_plan(ig_handle* h, int32_t n_steps, const int32_t* fra
     if (h->nuis_on && !(h->lnz_cache && h->vinter_pos)) {
         h->err = "ig_run_cycle_device: the device nuisance step needs the per-contact likelihood records and v_inter > 0"; return -1;
     }
-    if (cycle_buffers(h, n_steps)) return -2;
+    const int w = std::max(IG_MAX_CANDS, (int)n_neighbours);   // every step's grid: n_neighbours slots (enqueue_plan_step)
+    if (cycle_buffers(h, n_steps, w)) return -2;
     CK(cudaMemcpyAsync(h->cyc_frags, frags, sizeof(int) * (size_t)n_steps, cudaMemcpyHostToDevice, h->stream));
     if (h->nuis_on) {
         k_nuis_begin<<<1, 1, 0, h->stream>>>(h->sc, (unsigned)(seed & 0xffffffffu), (unsigned)(seed >> 32), cycle);
         h->n_launches += 1;
     }
-    if (n_neighbours > IG_MAX_CANDS) {   // every step a wide step (enqueue_plan_step), candidates from the wide plan
-        if (wide_plan_buffers(h, n_steps, n_neighbours)) return -2;
-        k_draw_plan_wide<<<(n_steps + 127) / 128, 128, 0, h->stream>>>(h->cyc_wide, n_neighbours, h->cyc_frags, n_steps, n_neighbours, h->nf,
-                                                                     h->lvl->nb_ptr, h->lvl->nb_idx, h->lvl->nb_cdf, h->lvl->nb_nnz,
-                                                                     (unsigned)(seed & 0xffffffffu), (unsigned)(seed >> 32), cycle);
-    } else {
-        h->plan_width = IG_MAX_CANDS;
-        k_draw_plan<<<(n_steps + 127) / 128, 128, 0, h->stream>>>(h->cyc_in, h->cyc_frags, n_steps, n_neighbours, h->nf, h->lvl->nb_ptr, h->lvl->nb_idx,
-                                                                h->lvl->nb_cdf, h->lvl->nb_nnz, (unsigned)(seed & 0xffffffffu), (unsigned)(seed >> 32), cycle);
-    }
+    auto* draw = w == IG_MAX_CANDS ? k_draw_plan<IG_MAX_CANDS> : k_draw_plan<IG_MAX_NEIGHBOURS>;
+    draw<<<(n_steps + 127) / 128, 128, 0, h->stream>>>(h->cyc_plan, w, h->sc, h->cyc_frags, n_steps, n_neighbours, h->nf, h->lvl->nb_ptr,
+                                                       h->lvl->nb_idx, h->lvl->nb_cdf, h->lvl->nb_nnz, (unsigned)(seed & 0xffffffffu),
+                                                       (unsigned)(seed >> 32), cycle);
     if (launch_ok(h, "draw_plan")) return -2;
     h->n_launches += 1;
     return 0;
@@ -1426,20 +1262,15 @@ extern "C" int ig_cycle_wait(ig_handle* h, int32_t n_steps, ig_cycle_step* out) 
 extern "C" int ig_get_cycle_plan(ig_handle* h, int32_t n_steps, int32_t* out) {
     return ig_get_cycle_plan_wide(h, n_steps, IG_MAX_CANDS, out);
 }
-// the same as [n_steps][2 + width], from the plan the last cycle ran (narrow, or wide of stride 2 + plan_width)
+// the same as [n_steps][2 + width]
 extern "C" int ig_get_cycle_plan_wide(ig_handle* h, int32_t n_steps, int32_t width, int32_t* out) {
     if (use(h)) return -1;
     if (n_steps > h->cyc_cap) { h->err = "ig_get_cycle_plan: no such plan"; return -1; }
     if (width <= 0 || width > IG_MAX_NEIGHBOURS) { h->err = "ig_get_cycle_plan: width out of range (1 .. IG_MAX_NEIGHBOURS = 64)"; return -1; }
     if (n_steps <= 0) return 0;
-    if (h->plan_width == IG_MAX_CANDS && width == IG_MAX_CANDS) {
-        CK(cudaMemcpy(out, h->cyc_in, sizeof(int) * (size_t)n_steps * (2 + IG_MAX_CANDS), cudaMemcpyDeviceToHost));
-        return 0;
-    }
     const int src_w = h->plan_width;
-    if (src_w > IG_MAX_CANDS && (size_t)n_steps * (2 + src_w) > h->cyc_wide_cap) { h->err = "ig_get_cycle_plan: no such plan"; return -1; }
     std::vector<int> src((size_t)n_steps * (2 + src_w));
-    CK(cudaMemcpy(src.data(), src_w > IG_MAX_CANDS ? h->cyc_wide : h->cyc_in, src.size() * sizeof(int), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(src.data(), h->cyc_plan, src.size() * sizeof(int), cudaMemcpyDeviceToHost));
     for (int t = 0; t < n_steps; t++) {
         const int* p = &src[(size_t)t * (2 + src_w)];
         int* q = out + (size_t)t * (2 + width);
@@ -1493,26 +1324,31 @@ extern "C" int ig_set_gpu_share(ig_handle* h, int32_t share) {
     if (share < 1) { h->err = "ig_set_gpu_share: share must be >= 1"; return -1; }
     if (h->pending_steps) { h->err = "ig_set_gpu_share: an asynchronous cycle is still pending"; return -1; }
     CK(cudaStreamSynchronize(h->stream));
-    for (int i = 0; i < 8; i++) for (int j = 0; j <= IG_MAX_CANDS; j++) if (h->graph[i][j]) { cudaGraphExecDestroy(h->graph[i][j]); h->graph[i][j] = nullptr; }
-    destroy_wide_graphs(h, 0);
-    if (h->graph_nuis_dev) { cudaGraphExecDestroy(h->graph_nuis_dev); h->graph_nuis_dev = nullptr; }
+    destroy_graphs(h, 0);
     h->grid_score = std::max(8, h->grid_score_full / share);
     h->grid_flat = std::max(1, h->grid_score / 5);
     return 0;
 }
 
+// the head of step_sampler (fill_dist_single + eval_likelihood, CL:1407-1409) and a score-only pass of one candidate
 extern "C" int ig_eval_scores(ig_handle* h, int32_t id_frag, int32_t id_cand, int32_t flip_eject, double out24[24],
                               int32_t* n_uniq, int32_t* n_sub) {
     if (use(h)) return -1;
     if (!h->params_set) { h->err = "ig_eval_scores: parameters not set"; return -1; }
     h->incr_valid = false;
-    if (refresh_current(h, h->stream, false)) return -2;
-    if (int rc = score_candidates(h, id_frag, &id_cand, 1, flip_eject, false)) return rc;
+    if (id_frag < 0 || id_frag >= h->nf) { h->err = "id_frag out of range"; return -1; }
+    if (id_cand < 0 || id_cand >= h->nf) { h->err = "candidate out of range"; return -1; }
+    int* hs = h->h_small;
+    hs[0] = 1; hs[1] = id_frag;
+    for (int i = 0; i < IG_MAX_CANDS; i++) hs[2 + i] = i == 0 ? id_cand : 0;
+    CK(cudaMemcpyAsync(&h->sc->n_cands, hs, (2 + IG_MAX_CANDS) * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    enqueue_head(h, 1);
+    enqueue_pass(h, 1, flip_eject, nullptr, 0);
+    if (launch_ok(h, "eval_scores")) return -2;
+    h->n_launches += head_launches(h, 1) + pass_launches(h);
+    h->coords_fresh = true; h->coords_ever = true;
     ig_step_result r;
-    if (fetch_result(h, 1, &id_cand, &r, false)) return -2;
-    for (int i = 0; i < 24; i++) out24[i] = r.scores[i];
-    if (n_uniq) *n_uniq = r.n_uniq[0];
-    if (n_sub) *n_sub = r.n_sub[0];
+    if (fetch_result(h, 1, &id_cand, &r, false, true, out24, n_uniq, n_sub)) return -2;
     return 0;
 }
 
@@ -1579,17 +1415,7 @@ extern "C" int ig_full_likelihood(ig_handle* h, const float p8[8], int32_t use_s
     // the nuisance step's evaluation (stale coordinates, records) replays as ONE CUDA graph: 8 launches + 2 copies otherwise
     bool graphed = false;
     if (!write && records && h->use_graph && !h->nuis_graph_failed) {
-        if (!h->graph_nuis) {
-            cudaGraph_t g = nullptr;
-            cudaError_t e = cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal);
-            if (e == cudaSuccess) {
-                enqueue_full_likelihood(h, 0, true);
-                e = cudaStreamEndCapture(h->stream, &g);
-            }
-            if (e == cudaSuccess && g) e = cudaGraphInstantiate(&h->graph_nuis, g, 0);
-            if (g) cudaGraphDestroy(g);
-            if (e != cudaSuccess || !h->graph_nuis) { h->graph_nuis = nullptr; h->nuis_graph_failed = true; cudaGetLastError(); }
-        }
+        if (!h->graph_nuis) capture(h, h->graph_nuis, h->nuis_graph_failed, [&] { enqueue_full_likelihood(h, 0, true); });
         if (h->graph_nuis) { CK(cudaGraphLaunch(h->graph_nuis, h->stream)); graphed = true; }
     }
     if (!graphed) enqueue_full_likelihood(h, write, records);

@@ -4,7 +4,7 @@ attributes, implemented over the C ABI of ``libinstagraal_b200.so`` through ctyp
 
 Mirrors (reference file:line):
   sampler.__init__            CL:92-319    -> ig_create (+ host-side neighbour pmfs, CL:3053-3101)
-  step_sampler                CL:1401-1465 -> ig_step
+  step_sampler                CL:1401-1465 -> ig_step_wide
   step_nuisance_parameters    CL:2961-3051 -> ig_full_likelihood (+ host RNG / fsolve as in the reference);
                               production RNG mode: run_cycle_device(nuisance=True) -> ig_set_device_nuisance (on the device)
   bomb_the_genome             CL:1925-1948 -> ig_bomb
@@ -196,16 +196,19 @@ class sampler:
             "local_scramble d1", "local_scramble d2", "local_scramble d3", "local_scramble d4"]
         self.setup_distri_frags()
         self._nb_state = {}   # shared (by reference) with the clones of this chain: neighbour weights uploaded once per level
-        # one result record per handle, read through NumPy views (no per-step ctypes -> list conversions)
+        self._bind_step_buffers()
+
+    def _bind_step_buffers(self):
+        """this chain's host buffers of ig_step_wide (a result record, candidates, scores, n_uniq, n_sub of up to
+        IG_MAX_NEIGHBOURS candidates), bound once with the ctypes function: no per-step ctypes conversions"""
         self._res = L.ig_step_result()
-        self._res_scores = np.frombuffer(self._res, dtype=np.float64, count=L.IG_MAX_CANDS * L.IG_N_OPS,
-                                         offset=L.ig_step_result.scores.offset)
-        self._res_nuniq = np.frombuffer(self._res, dtype=np.int32, count=L.IG_MAX_CANDS, offset=L.ig_step_result.n_uniq.offset)
-        self._res_nsub = np.frombuffer(self._res, dtype=np.int32, count=L.IG_MAX_CANDS, offset=L.ig_step_result.n_sub.offset)
-        self._cand_buf = np.zeros(L.IG_MAX_CANDS, dtype=np.int32)
-        self._cand_ptr = _ptr(self._cand_buf)
-        self._res_ref = C.byref(self._res)
-        self._ig_step = L.lib().ig_step
+        self._cand_buf = np.zeros(L.IG_MAX_NEIGHBOURS, dtype=np.int32)
+        self._scores_buf = np.zeros(L.IG_MAX_NEIGHBOURS * L.IG_N_OPS, dtype=np.float64)
+        self._nuniq_buf = np.zeros(L.IG_MAX_NEIGHBOURS, dtype=np.int32)
+        self._nsub_buf = np.zeros(L.IG_MAX_NEIGHBOURS, dtype=np.int32)
+        self._step_args = (_ptr(self._cand_buf), C.byref(self._res), _ptr(self._scores_buf), _ptr(self._nuniq_buf),
+                           _ptr(self._nsub_buf))
+        self._ig_step_wide = L.lib().ig_step_wide
 
     @classmethod
     def clone_of(cls, other):
@@ -224,13 +227,7 @@ class sampler:
         s.likelihood_t = None
         s._nuis_follows, s._spec, s._spec_pool, s._twin, s._twin_synced = False, None, None, None, False
         s._nuis_device = False
-        s._res = L.ig_step_result()
-        s._res_scores = np.frombuffer(s._res, dtype=np.float64, count=L.IG_MAX_CANDS * L.IG_N_OPS, offset=L.ig_step_result.scores.offset)
-        s._res_nuniq = np.frombuffer(s._res, dtype=np.int32, count=L.IG_MAX_CANDS, offset=L.ig_step_result.n_uniq.offset)
-        s._res_nsub = np.frombuffer(s._res, dtype=np.int32, count=L.IG_MAX_CANDS, offset=L.ig_step_result.n_sub.offset)
-        s._cand_buf = np.zeros(L.IG_MAX_CANDS, dtype=np.int32)
-        s._cand_ptr = _ptr(s._cand_buf)
-        s._res_ref = C.byref(s._res)
+        s._bind_step_buffers()
         if other.param_simu is not None:
             s.set_param_simu(np.array(list(other.param_simu[0]), dtype=np.float32))
             s.param_simu_test = s.param_simu
@@ -412,8 +409,7 @@ class sampler:
             self.all_scores = np.zeros(0)
             self.n_uniq, self.n_sub_vals = [], []
             return (self.likelihood_t, self._last_dist, -1, int(id_frag), self.mean_length_contigs, self.n_contigs)
-        if n <= L.IG_MAX_CANDS:
-            self._cand_buf[:n] = self.candidates
+        self._cand_buf[:n] = self.candidates
         res = self._res
         fut = None
         if self._nuis_follows and self.param_simu is not None:   # the previous call was a nuisance step: expect the next one
@@ -422,24 +418,14 @@ class sampler:
                 self._spec_pool = ThreadPoolExecutor(max_workers=1, thread_name_prefix="ig-nuisance")
             fut = self._spec_pool.submit(self._speculate_nuisance)
         self._nuis_follows = False
-        if n <= L.IG_MAX_CANDS:
-            rc = self._ig_step(self._h, int(id_frag), self._cand_ptr, n, self._res_ref)
-        else:   # more candidates than one scoring pass takes: ig_step_wide (batches of IG_MAX_CANDS)
-            wide = self._wide_buffers()
-            wide["cands"][:n] = self.candidates
-            rc = L.lib().ig_step_wide(self._h, int(id_frag), _ptr(wide["cands"]), n, self._res_ref, _ptr(wide["scores"]),
-                                      _ptr(wide["n_uniq"]), _ptr(wide["n_sub"]))
+        cands, res_ref, scores, n_uniq, n_sub = self._step_args
+        rc = self._ig_step_wide(self._h, int(id_frag), cands, n, res_ref, scores, n_uniq, n_sub)   # (batches of IG_MAX_CANDS beyond)
         self._spec = fut.result() if fut is not None else None
         if rc != 0:
             L.check(self._h, rc, "ig_step")
-        if n <= L.IG_MAX_CANDS:
-            self.all_scores = self._res_scores[:self.n_tmp_struct * n].copy()
-            self.n_uniq = self._res_nuniq[:n].tolist()
-            self.n_sub_vals = self._res_nsub[:n].tolist()
-        else:
-            self.all_scores = wide["scores"][:self.n_tmp_struct * n].copy()
-            self.n_uniq = wide["n_uniq"][:n].tolist()
-            self.n_sub_vals = wide["n_sub"][:n].tolist()
+        self.all_scores = self._scores_buf[:self.n_tmp_struct * n].copy()
+        self.n_uniq = self._nuniq_buf[:n].tolist()
+        self.n_sub_vals = self._nsub_buf[:n].tolist()
         self.n_proposals_scored += sum(self.n_uniq)
         self.q4_hits = res.q4_hits
         global_id = np.int64(res.cand_index * self.n_tmp_struct + res.op_sampled)
@@ -453,16 +439,6 @@ class sampler:
         self.curr_likelihood_on_nz = res.lnz_full
         self._last_dist = res.dist
         return (o, res.dist, op_sampled, id_f_sampled, self.mean_length_contigs, self.n_contigs)
-
-    def _wide_buffers(self):
-        """host buffers of ig_step_wide (made on first use, per handle)"""
-        w = getattr(self, "_wide", None)
-        if w is None or w["owner"] is not self._h:
-            w = {"owner": self._h, "cands": np.zeros(L.IG_MAX_NEIGHBOURS, dtype=np.int32),
-                 "scores": np.zeros(L.IG_MAX_NEIGHBOURS * L.IG_N_OPS, dtype=np.float64),
-                 "n_uniq": np.zeros(L.IG_MAX_NEIGHBOURS, dtype=np.int32), "n_sub": np.zeros(L.IG_MAX_NEIGHBOURS, dtype=np.int32)}
-            self._wide = w
-        return w
 
     def run_cycle(self, list_frags, n_neighbours=5, candidates=None):
         """The inner loop of full_em (IG:217-241) for the fragments in ``list_frags`` as ONE library call:
@@ -490,13 +466,8 @@ class sampler:
         out = np.zeros(n, dtype=L.CYCLE_DTYPE)
         assert out.dtype.itemsize == C.sizeof(L.ig_cycle_step)
         L.check(self._h, L.lib().ig_run_cycle_wide(self._h, n, _ptr(frags), _ptr(c8), int(width), _ptr(nc), _ptr(out)), "ig_run_cycle")
-        self._plan_width = width
+        self._after_cycle(out, width)
         if n:
-            last = out[-1]
-            self.n_contigs = np.int32(last["n_contigs"])
-            self.mean_length_contigs = np.float32(last["sum_l_cont"]) / np.float32(last["n_contigs"])
-            self.likelihood_t = self.o = np.float64(last["likelihood"])
-            self.n_proposals_scored += int(out["n_proposals"].sum())
             self.candidates = c8[-1, :nc[-1]].tolist()
         return out
 
@@ -537,8 +508,7 @@ class sampler:
         out = np.zeros(n, dtype=L.CYCLE_DTYPE)
         L.check(self._h, L.lib().ig_run_cycle_device(self._h, n, _ptr(frags), int(n_neighbours), int(seed), int(cycle), _ptr(out)),
                 "ig_run_cycle_device")
-        self._plan_width = max(L.IG_MAX_CANDS, int(n_neighbours))
-        self._after_cycle(out)
+        self._after_cycle(out, max(L.IG_MAX_CANDS, int(n_neighbours)))
         if not nuisance:
             return out
         return out, self._after_nuisance(n)
@@ -587,7 +557,9 @@ class sampler:
                     "ig_set_neighbour_weights")
             self._nb_state["uploaded"] = True
 
-    def _after_cycle(self, out):
+    def _after_cycle(self, out, plan_width):
+        """the host copies of the last step's outputs after a cycle, and the candidate slots of its plan (last_cycle_plan)"""
+        self._plan_width = plan_width
         if len(out):
             last = out[-1]
             self.n_contigs = np.int32(last["n_contigs"])

@@ -85,8 +85,7 @@ class ReplicaSet:
                                                 int(cycle), _ptr(out))
         L.check(None, rc, "ig_run_cycles_device_multi")
         for i, c in enumerate(self.chains):
-            c._plan_width = max(L.IG_MAX_CANDS, int(n_neighbours))
-            c._after_cycle(out[i])
+            c._after_cycle(out[i], max(L.IG_MAX_CANDS, int(n_neighbours)))
         if not nuisance:
             return out
         return out, np.stack([c._after_nuisance(n_steps) for c in self.chains])
