@@ -95,6 +95,17 @@ typedef struct ig_nuisance_step {   /* one nuisance step of a production-mode cy
     int32_t pad;
 } ig_nuisance_step;
 
+typedef struct ig_tempered_step {   /* the move draw of one step at a chain temperature T > 0 (ig_set_temperature), 48 B */
+    double s_max;              /* M, the step's maximum score */
+    double log_w;              /* log(sum_i exp((s_i - M) / T)) over the scored proposals (log sum_b W_b of a wide step) */
+    double u;                  /* draw inside the (winning) batch: philox_uniform(t, cycle, 0x80000002, 0, seed) */
+    double u_batch;            /* batch draw of a wide step: philox_uniform(t, cycle, 0x80000003, 0, seed); 0 in a narrow step */
+    int32_t n_scored;          /* scored proposals of the step (non-zero, non-NaN score) */
+    int32_t batch;             /* drawn batch of IG_MAX_CANDS candidates (0 in a narrow step) */
+    int32_t index;             /* drawn flattened index over the whole step: candidate * IG_N_OPS + op */
+    int32_t pad;
+} ig_tempered_step;
+
 /* sampler.__init__ device part (CL:92-319: sparse_data_2_gpu, setup_all_gpu_struct, loadProgram) */
 int ig_create(const ig_config* cfg, const ig_level_data* data, ig_handle** out);
 /* sampler.free_gpu (CL:3167-3177) */
@@ -161,6 +172,16 @@ int ig_get_cycle_plan(ig_handle* h, int32_t n_steps, int32_t* out /* [n_steps][2
  * every call behaves as without it.  ig_get_nuisance_records returns the per-step records of the last cycle. */
 int ig_set_device_nuisance(ig_handle* h, int32_t on);
 int ig_get_nuisance_records(ig_handle* h, int32_t n_steps, ig_nuisance_step* out);
+/* Chain temperature T >= 0 of the production RNG mode (DESIGN.md 4e).  T = 0 (the default) is the reference's argmax.  At
+ * T > 0 every step of ig_run_cycle_device, ig_run_cycles_device_multi and ig_run_cycle_device_async draws its move among the
+ * scored proposals with probability exp((s_i - M) / T) / sum, M = the step's maximum score (Philox4x32-10 with the chain's
+ * seed as key, counters (t, cycle, 0x80000002, 0) and, for the batch of a step of more than IG_MAX_CANDS candidates,
+ * (t, cycle, 0x80000003, 0)), and the nuisance step accepts when exp((L_nuis - o) / T) >= u.  The host-RNG entry points
+ * (ig_step, ig_step_wide, ig_run_cycle, ig_run_cycle_wide) refuse to run at T > 0.  ig_set_temperature refuses NaN, +-inf,
+ * negative values and a pending asynchronous cycle; it is stream-ordered (the step graphs read T at replay).
+ * ig_get_tempered_records returns the per-step draws of the last cycle (written only at T > 0). */
+int ig_set_temperature(ig_handle* h, double temperature);
+int ig_get_tempered_records(ig_handle* h, int32_t n_steps, ig_tempered_step* out);
 /* eval = score every mutation of one (A,B) pair without applying: extract_uniq_mutations +
  * perform_mutations + slice_sparse_mat + extract_current_sub_likelihood + eval_all_sub_likelihood
  * (CL:1417-1431).  Refreshes the coordinates / full likelihood like the head of step_sampler. */
@@ -249,6 +270,9 @@ int ig_nccl_init(ig_handle* lead, int32_t rank, int32_t n_ranks, int32_t n_local
 int ig_allgather_best(ig_handle* lead, ig_handle** local_chains, int32_t n_local, double* lik, int32_t* n_contigs, int32_t* best,
                       float* ms);
 int ig_get_gathered_state(ig_handle* lead, int32_t index, int32_t* out13xNF);
+/* the live log-likelihood (likelihood_t: the last applied move's score, or L_nuis after an accepted nuisance proposal) of every
+ * chain in the last all-gather, out = [n_ranks * n_local] rank-major */
+int ig_get_gathered_live_likelihood(ig_handle* lead, double* out);
 int ig_adopt_gathered(ig_handle* lead, ig_handle** local_chains, int32_t n_local, int32_t index, float p8_out[8], int32_t valid_out[12],
                       double* likelihood_out);
 int ig_nccl_finalize(ig_handle* lead);

@@ -27,7 +27,7 @@ EXPORTS = (
     "ig_selftest_math", "ig_get_nuisance_stats", "ig_clone", "ig_run_cycles_device_multi", "ig_run_cycle_device_async", "ig_cycle_wait",
     "ig_bin_contacts", "ig_nccl_unique_id", "ig_nccl_init", "ig_allgather_best", "ig_get_gathered_state", "ig_nccl_finalize",
     "ig_set_device_nuisance", "ig_get_nuisance_records", "ig_step_wide", "ig_run_cycle_wide", "ig_get_cycle_plan_wide",
-    "ig_adopt_gathered",
+    "ig_adopt_gathered", "ig_set_temperature", "ig_get_tempered_records", "ig_get_gathered_live_likelihood",
 )
 
 
@@ -62,6 +62,10 @@ CYCLE_DTYPE = [("likelihood", "<f8"), ("lnz_full", "<f8"), ("dist", "<f8"), ("su
 # ig_nuisance_step (80 B): one device nuisance step of a production-mode cycle
 NUIS_DTYPE = [("likelihood_nuis", "<f8"), ("likelihood_t_after", "<f8"), ("u", "<f8"), ("draw", "<f8"), ("p_test", "<f4", (8,)),
               ("id_modif", "<i4"), ("accepted", "<i4"), ("valid", "<i4"), ("pad", "<i4")]
+
+# ig_tempered_step (48 B): the move draw of one production-mode step at a chain temperature T > 0
+TEMPERED_DTYPE = [("s_max", "<f8"), ("log_w", "<f8"), ("u", "<f8"), ("u_batch", "<f8"), ("n_scored", "<i4"), ("batch", "<i4"),
+                  ("index", "<i4"), ("pad", "<i4")]
 
 _lib = None
 
@@ -127,6 +131,9 @@ def lib():
         L.ig_step_wide.argtypes = [vp, i32, vp, i32, C.POINTER(ig_step_result), vp, vp, vp]
         L.ig_run_cycle_wide.argtypes = [vp, i32, vp, vp, i32, vp, vp]
         L.ig_get_cycle_plan_wide.argtypes = [vp, i32, i32, vp]
+        L.ig_set_temperature.argtypes = [vp, dbl]
+        L.ig_get_tempered_records.argtypes = [vp, i32, vp]
+        L.ig_get_gathered_live_likelihood.argtypes = [vp, vp]
         for name in EXPORTS:
             if name not in ("ig_destroy", "ig_last_error"):
                 getattr(L, name).restype = C.c_int

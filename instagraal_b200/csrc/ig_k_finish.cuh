@@ -228,27 +228,33 @@ __global__ void k_select(DevScalars* sc) {
 __device__ void select_step(DevScalars* sc, const IgDescriptor* __restrict__ desc_g) {
     const int n = sc->n_cands * IG_N_OPS;
     const int lane = threadIdx.x & 31;  // executed by one full warp
-    // first index of the maximum among the scored (non-zero) proposals (CL:1435-1446)
     int best = -1;
-    double bv = 0.0;
-    for (int i = lane; i < n; i += 32) {
-        const double v = __ldcg(&sc->scores[i]);
-        if (v == 0.0) continue;
-        if (best < 0 || v > bv) { best = i; bv = v; }
-    }
+    const double T = sc->temperature;
+    if (T > 0.0) {
+        best = temper_select(sc, n, T);   // a draw among the scored proposals (ig_k_temper.cuh)
+    } else {
+        // first index of the maximum among the scored (non-zero) proposals (CL:1435-1446)
+        double bv = 0.0;
+        for (int i = lane; i < n; i += 32) {
+            const double v = __ldcg(&sc->scores[i]);
+            if (v == 0.0) continue;
+            if (best < 0 || v > bv) { best = i; bv = v; }
+        }
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const int ob = __shfl_down_sync(0xffffffffu, best, o);
-        const double ov = __shfl_down_sync(0xffffffffu, bv, o);
-        if (ob >= 0 && (best < 0 || ov > bv || (ov == bv && ob < best))) { best = ob; bv = ov; }
+        for (int o = 16; o > 0; o >>= 1) {
+            const int ob = __shfl_down_sync(0xffffffffu, best, o);
+            const double ov = __shfl_down_sync(0xffffffffu, bv, o);
+            if (ob >= 0 && (best < 0 || ov > bv || (ov == bv && ob < best))) { best = ob; bv = ov; }
+        }
+        best = __shfl_sync(0xffffffffu, best, 0);
+        if (best < 0) best = 0;
     }
-    best = __shfl_sync(0xffffffffu, best, 0);
-    if (best < 0) best = 0;
     const int kc = best / IG_N_OPS, op = best % IG_N_OPS;
     const unsigned hit = __ballot_sync(0xffffffffu, lane < desc_g[kc].n_uniq && desc_g[kc].uniq[lane] == op);
     if (lane < 12 && op >= 12) sc->valid[lane] = desc_g[kc].valid[lane];
     if (lane != 0) return;
     sc->win_cand = kc; sc->win_op = op; sc->likelihood = __ldcg(&sc->scores[best]);
+    sc->live_likelihood = sc->likelihood;
     sc->n_heads = 0; sc->sum_l_cont = 0; sc->dist_half = 0; sc->q4_hits = 0;
     sc->max_label += 2;
     sc->prev_k = kc; sc->prev_u = hit ? (__ffs(hit) - 1) : 0;
@@ -390,7 +396,7 @@ __global__ void k_post_scalars(DevScalars* sc, const IgDescriptor* __restrict__ 
 }
 __global__ void __launch_bounds__(256)
 k_post(const FragRec* __restrict__ live, int nf, const int* __restrict__ init_prev, const int* __restrict__ init_next,
-       const int* __restrict__ orientable, DevScalars* sc, CycleOut* __restrict__ cyc_out) {
+       const int* __restrict__ orientable, DevScalars* sc, CycleOut* __restrict__ cyc_out, ig_tempered_step* __restrict__ trec_out) {
     TL(10);
     __shared__ int s_heads;
     __shared__ long long s_len, s_half;
@@ -448,6 +454,7 @@ k_post(const FragRec* __restrict__ live, int nf, const int* __restrict__ init_pr
                 for (int i = 0; i < sc->n_cands; i++) o.n_proposals += sc->res_nuniq[i];
                 o.id_f_sampled = sc->cands[sc->win_cand];
                 cyc_out[sc->step_idx] = o;
+                if (sc->temperature > 0.0) trec_out[sc->step_idx] = sc->trec;   // the tempered draw (ig_k_temper.cuh)
                 sc->step_idx += 1;
 #ifdef IG_TIMELINE
                 g_tl_step += 1;

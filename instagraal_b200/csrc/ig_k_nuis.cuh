@@ -78,7 +78,8 @@ __host__ __device__ inline int nuis_dmax_root(double kuhn, double lm, double slo
     return isfinite(*out) && *out > 0.0;
 }
 
-// the seed and cycle of the cycle being enqueued (once per cycle: the nuisance graph reads them from the record)
+// the seed and cycle of the cycle being enqueued (once per cycle: the nuisance graph and the tempered selection read them
+// from the record)
 __global__ void k_nuis_begin(DevScalars* sc, unsigned seed_lo, unsigned seed_hi, unsigned cycle) {
     sc->nuis_key_lo = seed_lo; sc->nuis_key_hi = seed_hi; sc->nuis_cycle = cycle;
 }
@@ -143,9 +144,10 @@ __global__ void k_nuis_accept(DevScalars* sc, ig_nuisance_step* __restrict__ rec
     const double l_t = sc->likelihood;
     const double u = sc->nuis_u;
     const int valid = sc->nuis_valid;
-    // temperature() is 1.0 in the reference; a NaN ratio is never >= u
-    const int acc = valid && (exp(__dsub_rn(l_nuis, l_t) / 1.0) >= u);
-    if (acc) { sc->p = q; sc->log10_vinter = sc->log10_vinter_test; }
+    // temperature() is 1.0 in the reference, the chain temperature T when one is set (DESIGN.md 4e); a NaN ratio is never >= u
+    const double T = sc->temperature;
+    const int acc = valid && (exp(__dsub_rn(l_nuis, l_t) / (T > 0.0 ? T : 1.0)) >= u);
+    if (acc) { sc->p = q; sc->log10_vinter = sc->log10_vinter_test; sc->live_likelihood = l_nuis; }
     sc->nuis_stale = acc;   // the next step's likelihood sums are stale exactly when this proposal was accepted
     ig_nuisance_step r;
     r.likelihood_nuis = l_nuis; r.likelihood_t_after = acc ? l_nuis : l_t; r.u = u; r.draw = sc->nuis_draw;

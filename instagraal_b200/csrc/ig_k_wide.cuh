@@ -21,6 +21,12 @@ struct WideStep {
     int best_b, n_prop;                         // first batch that reached the maximum (-1: none scored), proposals scored
     double best_v;
     int win_cand, pad;                          // index of the applied move's candidate in the whole list
+    // T > 0 (ig_k_temper.cuh): per batch the maximum score m_b, S_b = sum exp((s_i - m_b) / T) and the scored proposals;
+    // the step's maximum M, log(sum_b W_b), the batch draw and the scored proposals of the whole step
+    double t_m[IG_MAX_BATCHES], t_S[IG_MAX_BATCHES];
+    int t_cnt[IG_MAX_BATCHES];
+    double t_M, t_logW, t_ub;
+    int t_nsc, t_pad;
 };
 
 // before batch b: its candidates (8b .. 8b + n_b - 1 of the step's list) into sc, where k_cand_setup reads them, and the
@@ -43,6 +49,14 @@ __global__ void k_wide_stage(DevScalars* sc, WideStep* w, const int* __restrict_
 // the maximum over the non-zero scores, CL:1435-1446: a later batch wins only with a strictly larger score)
 __global__ void k_wide_stash(const DevScalars* __restrict__ sc, WideStep* w, int b) {
     const int nb = sc->n_cands;
+    const double T = sc->temperature;
+    if (T > 0.0 && threadIdx.x < 32) {   // the batch's part of the tempered draw
+        __shared__ double s_w[IG_MAX_CANDS * IG_N_OPS];
+        double m;
+        int cnt, last;
+        const double S = temper_weights(sc->scores, nb * IG_N_OPS, T, s_w, &m, &cnt, &last);
+        if (threadIdx.x == 0) { w->t_m[b] = m; w->t_S[b] = S; w->t_cnt[b] = cnt; }
+    }
     for (int i = threadIdx.x; i < nb * IG_N_OPS; i += blockDim.x) w->scores[b * IG_MAX_CANDS * IG_N_OPS + i] = sc->scores[i];
     if (threadIdx.x < nb) {
         w->n_uniq[b * IG_MAX_CANDS + threadIdx.x] = sc->res_nuniq[threadIdx.x];
@@ -63,11 +77,37 @@ __global__ void k_wide_stash(const DevScalars* __restrict__ sc, WideStep* w, int
     if (best >= 0 && (w->best_b < 0 || bv > w->best_v)) { w->best_b = b; w->best_v = bv; }
 }
 
-// before the re-score: the winning batch (batch 0 when nothing was scored, as np.argmax of an all -inf vector) staged
-// like k_wide_stage, from the validity list it started from
+// T > 0: the batch drawn with u_batch from W_b = S_b exp((m_b - M) / T), in batch order (ig_k_temper.cuh); the last batch
+// with a scored proposal if rounding leaves none, batch 0 when nothing was scored
+__device__ __noinline__ int wide_temper_batch(const DevScalars* sc, WideStep* w, double T) {
+    const int n_b = (w->n + IG_MAX_CANDS - 1) / IG_MAX_CANDS;
+    double M = -INFINITY;
+    int nsc = 0, last = -1;
+    for (int b = 0; b < n_b; b++) if (w->t_cnt[b] > 0) { M = fmax(M, w->t_m[b]); nsc += w->t_cnt[b]; last = b; }
+    auto W = [&](int b) { return w->t_cnt[b] > 0 ? __dmul_rn(w->t_S[b], exp(__ddiv_rn(__dsub_rn(w->t_m[b], M), T))) : 0.0; };
+    double sum = 0.0;
+    for (int b = 0; b < n_b; b++) sum = __dadd_rn(sum, W(b));
+    const double ub = temper_uniform(sc, IG_TEMPER_U_BATCH);
+    const double target = __dmul_rn(ub, sum);
+    int pick = last < 0 ? 0 : last;
+    double cum = 0.0;
+    for (int b = 0; b < n_b && last >= 0; b++) {
+        cum = __dadd_rn(cum, W(b));
+        if (cum > target) { pick = b; break; }
+    }
+    w->t_M = M; w->t_logW = log(sum); w->t_ub = ub; w->t_nsc = nsc;
+    return pick;
+}
+
+// before the re-score: the winning batch (batch 0 when nothing was scored, as np.argmax of an all -inf vector; at T > 0 the
+// drawn batch) staged like k_wide_stage, from the validity list it started from
 __global__ void k_wide_pick(DevScalars* sc, WideStep* w, const int* __restrict__ plan) {
     const int* src = plan ? plan + (size_t)sc->step_idx * sc->plan_stride : w->in;
-    const int b = max(w->best_b, 0);
+    __shared__ int s_b;
+    const double T = sc->temperature;
+    if (threadIdx.x == 0) s_b = T > 0.0 ? wide_temper_batch(sc, w, T) : max(w->best_b, 0);
+    __syncthreads();
+    const int b = s_b;
     const int nb = max(0, min(IG_MAX_CANDS, w->n - b * IG_MAX_CANDS));
     const int i = threadIdx.x;
     if (i < IG_MAX_CANDS) sc->cands[i] = i < nb ? src[2 + b * IG_MAX_CANDS + i] : 0;
@@ -87,7 +127,7 @@ __global__ void k_wide_flip(const DevScalars* __restrict__ sc, IgDescriptor* des
 // after the tail: the candidate index in the whole list, the step's proposal count (score-only passes), and the validity
 // list the reference leaves -- the last batch's, unless the applied op re-ran get_bounds (op >= 12, select_step).  The
 // fragment k_post recorded is already right: sc->cands holds the re-scored winning batch.
-__global__ void k_wide_finish(DevScalars* sc, WideStep* w, CycleOut* __restrict__ cyc_out) {
+__global__ void k_wide_finish(DevScalars* sc, WideStep* w, CycleOut* __restrict__ cyc_out, ig_tempered_step* __restrict__ trec_out) {
     const int i = threadIdx.x;
     if (i < 12 && sc->win_op < 12) sc->valid[i] = w->valid_end[i];
     if (i != 0) return;
@@ -95,5 +135,10 @@ __global__ void k_wide_finish(DevScalars* sc, WideStep* w, CycleOut* __restrict_
     if (cyc_out) {   // the record k_post just published (it advanced step_idx)
         CycleOut& o = cyc_out[sc->step_idx - 1];
         o.win_cand = w->win_cand; o.n_proposals = w->n_prop;
+        if (sc->temperature > 0.0) {   // the record k_post published holds the draw inside the batch: the whole step's
+            ig_tempered_step& r = trec_out[sc->step_idx - 1];
+            r.s_max = w->t_M; r.log_w = w->t_logW; r.u_batch = w->t_ub; r.n_scored = w->t_nsc;
+            r.batch = w->best_b; r.index = w->best_b * IG_MAX_CANDS * IG_N_OPS + r.index;
+        }
     }
 }

@@ -30,6 +30,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <cmath>
 #include <string>
 #include <vector>
 
@@ -102,6 +103,11 @@ struct DevScalars {
     unsigned nuis_key_lo, nuis_key_hi, nuis_cycle;
     int nuis_id, nuis_valid, nuis_stale;
     double nuis_u, nuis_draw;
+    // chain temperature (ig_set_temperature, read at replay; 0 = the argmax), the chain's live log-likelihood (the applied
+    // move's score, or L_nuis after an accepted nuisance proposal: the facade's likelihood_t) and the tempered draw of the
+    // step in flight (ig_k_temper.cuh)
+    double temperature, live_likelihood;
+    ig_tempered_step trec;
 };
 
 struct CycleOut {  // compact per-step record of a cycle (k_post; k_wide_finish fixes up a wide step's)
@@ -116,11 +122,13 @@ struct CycleOut {  // compact per-step record of a cycle (k_post; k_wide_finish 
 #include "ig_k_setup.cuh"   // per-candidate setup: descriptor, cut fragments, rigid-motion class tables, ordered affected-row list
 #include "ig_k_score.cuh"   // scoring: slice rule, row-end table + zero terms, evaluation queue, the row-per-warp scoring kernel
 #include "ig_k_flat.cuh"   // flat scoring path of small levels: k_pick + k_eval_flat
-#include "ig_k_finish.cuh"   // finalisation, move selection, incremental maintenance, apply, contig bookkeeping, histogram, thumbnail
 #include "ig_k_rng.cuh"   // production RNG mode: Philox4x32-10 neighbour draws of a whole cycle
+#include "ig_k_temper.cuh"   // production RNG mode: move selection at a chain temperature T > 0
+#include "ig_k_finish.cuh"   // finalisation, move selection, incremental maintenance, apply, contig bookkeeping, histogram, thumbnail
 #include "ig_k_nuis.cuh"   // production RNG mode: the nuisance-parameter step after every step of a cycle
 #include "ig_k_wide.cuh"   // steps of more than IG_MAX_CANDS candidates: batch staging, running maximum, fix-ups
 static_assert(sizeof(ig_nuisance_step) == 80, "ig_nuisance_step is 80 bytes (NUIS_DTYPE in _lib.py)");
+static_assert(sizeof(ig_tempered_step) == 48, "ig_tempered_step is 48 bytes (TEMPERED_DTYPE in _lib.py)");
 
 // ================================================================================================
 // host side
@@ -191,6 +199,9 @@ struct ig_handle {
     bool nuis_on = false, nuis_enqueued = false, nuis_graph_dev_failed = false;
     cudaGraphExec_t graph_nuis_dev = nullptr;
     ig_nuisance_step* nuis_rec = nullptr;
+    // chain temperature (ig_set_temperature; the device reads its copy in sc) and the per-step records of the tempered draws
+    double temperature = 0.0;
+    ig_tempered_step* temp_rec = nullptr;
     // the cycle plan [cyc_cap][2 + W] (n_cands, fragment, candidates), W <= cyc_width; plan_width = W of the last cycle
     int* cyc_plan; CycleOut* cyc_out; int cyc_cap, cyc_width, plan_width; bool graph_failed, capturing, use_graph; long long n_full;
     int pending_steps;   // steps enqueued by an asynchronous cycle call and not collected yet
@@ -528,6 +539,7 @@ extern "C" void ig_destroy(ig_handle* h) {
     if (h->d_p8) cudaFree(h->d_p8);
     if (h->graph_nuis) cudaGraphExecDestroy(h->graph_nuis);
     if (h->nuis_rec) cudaFree(h->nuis_rec);
+    if (h->temp_rec) cudaFree(h->temp_rec);
     if (h->wide) cudaFree(h->wide);
     if (h->h_wide) cudaFreeHost(h->h_wide);
     for (int i = 0; i < 6; i++) if (h->ev[i]) cudaEventDestroy(h->ev[i]);
@@ -724,7 +736,7 @@ static int apply_and_post(ig_handle* h, int forced_cand, int forced_op) {
     h->label_hi += 2;
     k_apply<<<(nf + 255) / 256, 256, 0, h->stream>>>(h->live, nf, h->sc, h->desc, forced_cand, forced_op);
     k_post_scalars<<<1, 1, 0, h->stream>>>(h->sc, h->desc, forced_cand, forced_op);
-    k_post<<<(nf + 255) / 256, 256, 0, h->stream>>>(h->live, nf, h->init_prev, h->init_next, h->orientable, h->sc, nullptr);
+    k_post<<<(nf + 255) / 256, 256, 0, h->stream>>>(h->live, nf, h->init_prev, h->init_next, h->orientable, h->sc, nullptr, nullptr);
     h->coords_fresh = false;
     h->n_launches += 3;
     return launch_ok(h, "apply");
@@ -870,7 +882,7 @@ static void enqueue_tail(ig_handle* h, int cycle) {
     k_apply<<<(h->nf + 255) / 256, 256, 0, h->stream>>>(h->live, h->nf, h->sc, h->desc, -1, -1);
     IG_MARK(10);
     k_post<<<(h->nf + 255) / 256, 256, 0, h->stream>>>(h->live, h->nf, h->init_prev, h->init_next, h->orientable, h->sc,
-                                                       cycle ? h->cyc_out : nullptr);
+                                                       cycle ? h->cyc_out : nullptr, cycle ? h->temp_rec : nullptr);
     IG_MARK(11);
     cudaStreamWaitEvent(h->stream, h->ev_out, 0);
 }
@@ -900,7 +912,7 @@ static void enqueue_wide_step(ig_handle* h, int full, int n_batches, int cycle) 
     k_wide_pick<<<1, 32, 0, h->stream>>>(h->sc, h->wide, plan);
     enqueue_pass(h, IG_MAX_CANDS, 1, nullptr, 1, true);
     enqueue_tail(h, cycle);
-    k_wide_finish<<<1, 32, 0, h->stream>>>(h->sc, h->wide, cycle ? h->cyc_out : nullptr);
+    k_wide_finish<<<1, 32, 0, h->stream>>>(h->sc, h->wide, cycle ? h->cyc_out : nullptr, cycle ? h->temp_rec : nullptr);
     if (!cycle) {
         cudaMemcpyAsync(h->h_sc, h->sc, sizeof(DevScalars), cudaMemcpyDeviceToHost, h->stream);
         cudaMemcpyAsync(h->h_wide, h->wide, sizeof(WideStep), cudaMemcpyDeviceToHost, h->stream);
@@ -983,6 +995,8 @@ extern "C" int ig_step_wide(ig_handle* h, int32_t id_frag, const int32_t* cands,
     if (!out || !cands) { h->err = "ig_step_wide: null argument"; return -1; }
     if (n_cands <= 0 || n_cands > IG_MAX_NEIGHBOURS) { h->err = "ig_step_wide: n_cands out of range (1 .. IG_MAX_NEIGHBOURS = 64)"; return -1; }
     if (!h->params_set) { h->err = "ig_step: parameters not set (ig_set_params)"; return -1; }
+    if (h->temperature > 0.0) { h->err = "ig_step: the chain temperature is > 0 (tempered selection needs the seeded production mode, "
+                                         "ig_run_cycle_device); set it back with ig_set_temperature(h, 0)"; return -1; }
     if (id_frag < 0 || id_frag >= h->nf) { h->err = "id_frag out of range"; return -1; }
     for (int i = 0; i < n_cands; i++) if (cands[i] < 0 || cands[i] >= h->nf) { h->err = "candidate out of range"; return -1; }
     for (int i = 0; i < n_cands; i++) if (cands[i] == id_frag) { h->err = "candidate equals the visited fragment (reference quirk Q4; see DESIGN.md D1)"; return -1; }
@@ -1018,15 +1032,16 @@ extern "C" int ig_step_wide(ig_handle* h, int32_t id_frag, const int32_t* cands,
 // Semantically identical to n_steps calls of ig_step (IG.full_em inner loop, instagraal.py:217-241).
 
 // The buffers of a cycle of n_steps steps whose plan entries hold `width` candidate slots: the plan [n_steps][2 + width],
-// the step records, the visiting order, the nuisance records.  They only grow; the cycle graphs bake them in.
+// the step records, the visiting order, the nuisance and tempered records.  They only grow; the cycle graphs bake them in.
 static int cycle_buffers(ig_handle* h, int n_steps, int width) {
     if (n_steps > h->cyc_cap || width > h->cyc_width) {
         const int cap = std::max(n_steps, h->cyc_cap), w = std::max(width, h->cyc_width);
-        for (void* q : {(void*)h->cyc_plan, (void*)h->cyc_out, (void*)h->cyc_frags, (void*)h->nuis_rec}) if (q) cudaFree(q);
-        h->cyc_plan = nullptr; h->cyc_out = nullptr; h->cyc_frags = nullptr; h->nuis_rec = nullptr; h->cyc_cap = 0; h->cyc_width = 0;
+        for (void* q : {(void*)h->cyc_plan, (void*)h->cyc_out, (void*)h->cyc_frags, (void*)h->nuis_rec, (void*)h->temp_rec}) if (q) cudaFree(q);
+        h->cyc_plan = nullptr; h->cyc_out = nullptr; h->cyc_frags = nullptr; h->nuis_rec = nullptr; h->temp_rec = nullptr;
+        h->cyc_cap = 0; h->cyc_width = 0;
         destroy_graphs(h, 4);
         if (dev_alloc(h, &h->cyc_plan, (size_t)cap * (2 + w)) || dev_alloc(h, &h->cyc_out, (size_t)cap) ||
-            dev_alloc(h, &h->cyc_frags, (size_t)cap) || dev_alloc(h, &h->nuis_rec, (size_t)cap)) return -2;
+            dev_alloc(h, &h->cyc_frags, (size_t)cap) || dev_alloc(h, &h->nuis_rec, (size_t)cap) || dev_alloc(h, &h->temp_rec, (size_t)cap)) return -2;
         h->cyc_cap = cap; h->cyc_width = w;
     }
     h->plan_width = width;
@@ -1134,6 +1149,8 @@ extern "C" int ig_run_cycle_wide(ig_handle* h, int32_t n_steps, const int32_t* f
     if (!h->params_set) { h->err = "ig_run_cycle: parameters not set"; return -1; }
     if (h->nuis_on) { h->err = "ig_run_cycle: the device nuisance step is on (it needs the seeded production mode, ig_run_cycle_device); "
                                 "turn it off with ig_set_device_nuisance(h, 0)"; return -1; }
+    if (h->temperature > 0.0) { h->err = "ig_run_cycle: the chain temperature is > 0 (tempered selection needs the seeded production mode, "
+                                         "ig_run_cycle_device); set it back with ig_set_temperature(h, 0)"; return -1; }
     if (width <= 0 || width > IG_MAX_NEIGHBOURS) { h->err = "ig_run_cycle: width out of range (1 .. IG_MAX_NEIGHBOURS = 64)"; return -1; }
     if (n_steps <= 0) return 0;
     int n_max = 0;
@@ -1197,7 +1214,7 @@ static int prepare_device_plan(ig_handle* h, int32_t n_steps, const int32_t* fra
     const int w = std::max(IG_MAX_CANDS, (int)n_neighbours);   // every step's grid: n_neighbours slots (enqueue_plan_step)
     if (cycle_buffers(h, n_steps, w)) return -2;
     CK(cudaMemcpyAsync(h->cyc_frags, frags, sizeof(int) * (size_t)n_steps, cudaMemcpyHostToDevice, h->stream));
-    if (h->nuis_on) {
+    if (h->nuis_on || h->temperature > 0.0) {   // the key and cycle of the nuisance and tempered-selection draws
         k_nuis_begin<<<1, 1, 0, h->stream>>>(h->sc, (unsigned)(seed & 0xffffffffu), (unsigned)(seed >> 32), cycle);
         h->n_launches += 1;
     }
@@ -1294,6 +1311,25 @@ extern "C" int ig_set_device_nuisance(ig_handle* h, int32_t on) {
         if (!h->vinter_pos) { h->err = "ig_set_device_nuisance: the live v_inter must be > 0"; return -1; }
     }
     h->nuis_on = on != 0;
+    return 0;
+}
+// the chain temperature of the tempered selection (ig_k_temper.cuh), written stream-ordered into the scalar record: the
+// captured step graphs read it at replay, so they stay valid and no launch is added to a step
+extern "C" int ig_set_temperature(ig_handle* h, double temperature) {
+    if (use(h)) return -1;
+    if (!(temperature >= 0.0) || !std::isfinite(temperature)) { h->err = "ig_set_temperature: the temperature must be finite and >= 0"; return -1; }
+    if (h->pending_steps) { h->err = "ig_set_temperature: an asynchronous cycle is still pending (ig_cycle_wait)"; return -1; }
+    k_set_temperature<<<1, 1, 0, h->stream>>>(h->sc, temperature);
+    if (launch_ok(h, "set_temperature")) return -2;
+    h->temperature = temperature;
+    return 0;
+}
+extern "C" int ig_get_tempered_records(ig_handle* h, int32_t n_steps, ig_tempered_step* out) {
+    if (use(h)) return -1;
+    if (n_steps == 0) return 0;
+    if (n_steps < 0 || n_steps > h->cyc_cap || !h->temp_rec) { h->err = "ig_get_tempered_records: no such records"; return -1; }
+    CK(cudaMemcpyAsync(out, h->temp_rec, sizeof(ig_tempered_step) * (size_t)n_steps, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
     return 0;
 }
 extern "C" int ig_get_nuisance_records(ig_handle* h, int32_t n_steps, ig_nuisance_step* out) {

@@ -45,8 +45,10 @@ struct ReplicaHeader {
     double likelihood; int n_contigs; int n_frags;
     float p8[8];
     int valid[12];
-    int max_label;
-    int pad[7];
+    int max_label, pad0;
+    double live_likelihood;   // the chain's likelihood_t: `likelihood` (the last applied move's score) is stale after an
+                              // accepted nuisance proposal
+    int pad[4];
 };
 static_assert(sizeof(ReplicaHeader) == 128, "ReplicaHeader is 128 bytes (the scaffold records that follow it stay 64-B aligned)");
 struct ig_replica_state {
@@ -66,8 +68,9 @@ __global__ void k_replica_header(const DevScalars* __restrict__ sc, int nf, Repl
     const float* p = &sc->p.kuhn;
     for (int i = 0; i < 8; i++) r.p8[i] = p[i];
     for (int i = 0; i < 12; i++) r.valid[i] = sc->valid[i];
-    r.max_label = sc->max_label;
-    for (int i = 0; i < 7; i++) r.pad[i] = 0;
+    r.max_label = sc->max_label; r.pad0 = 0;
+    r.live_likelihood = sc->live_likelihood;
+    for (int i = 0; i < 4; i++) r.pad[i] = 0;
     *out = r;
 }
 // a chain takes over the gathered chain's parameters (as k_set_params_dev sets them), validity list and label counter
@@ -78,6 +81,7 @@ __global__ void k_replica_adopt(const ReplicaHeader* __restrict__ src, DevScalar
     sc->p = p; sc->log10_vinter = log10((double)p.v_inter);
     for (int i = 0; i < 12; i++) sc->valid[i] = r.valid[i];
     sc->max_label = r.max_label;
+    sc->live_likelihood = r.live_likelihood;
 }
 __global__ void k_replica_compact(const char* __restrict__ recv, size_t rec_bytes, int n, ReplicaHeader* __restrict__ out) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -181,6 +185,15 @@ extern "C" int ig_allgather_best(ig_handle* h, ig_handle** local, int32_t n_loca
     }
     if (best) *best = b;
     if (ms) { *ms = 0.f; cudaEventElapsedTime(ms, r->ev0, r->ev1); }
+    return 0;
+}
+
+// live log-likelihood (likelihood_t) of every chain in the last all-gather, [n_ranks * n_local] rank-major
+extern "C" int ig_get_gathered_live_likelihood(ig_handle* h, double* out) {
+    if (use(h)) return -1;
+    ig_replica_state* r = h->rep;
+    if (!r || !r->gathered) { h->err = "ig_get_gathered_live_likelihood: no all-gather since ig_nccl_init (ig_allgather_best)"; return -1; }
+    for (int i = 0; i < r->n_ranks * r->n_local; i++) out[i] = r->h_heads[i].live_likelihood;
     return 0;
 }
 

@@ -189,6 +189,7 @@ class sampler:
         self._twin_synced = False
         self.n_nuis_overlapped = 0
         self._nuis_device = False   # ig_set_device_nuisance state of the handle
+        self.chain_temperature = 0.0   # set_chain_temperature (not the reference's temperature(t, n_step))
         self.modification_str = [  # CL:1601-1620
             "eject frag", "flip frag", "pop out split insert @ left or 1", "pop out split insert @ left or -1",
             "pop out split insert @ right or 1", "pop out split insert @ right or -1", "pop out insert @ right or 1",
@@ -227,6 +228,7 @@ class sampler:
         s.likelihood_t = None
         s._nuis_follows, s._spec, s._spec_pool, s._twin, s._twin_synced = False, None, None, None, False
         s._nuis_device = False
+        s.chain_temperature = 0.0   # a new handle starts at T = 0
         s._bind_step_buffers()
         if other.param_simu is not None:
             s.set_param_simu(np.array(list(other.param_simu[0]), dtype=np.float32))
@@ -302,7 +304,8 @@ class sampler:
         carried list_valid_insert (quirk Q3), the parameters, likelihood_t and the host RNG state.  The
         reference cannot resume a run (SURVEY section 5).  Saving re-synchronises the incremental
         likelihood state (one full refresh on the next step) so that the continued and the resumed run
-        perform identical arithmetic."""
+        perform identical arithmetic.  The chain temperature (set_chain_temperature) is a run setting like the seed and is
+        not saved."""
         st = self._get_state()
         valid = self.get_valid_insert()
         self._set_state(st)
@@ -520,6 +523,24 @@ class sampler:
         if on != self._nuis_device:
             L.check(self._h, L.lib().ig_set_device_nuisance(self._h, int(on)), "ig_set_device_nuisance")
             self._nuis_device = on
+
+    def set_chain_temperature(self, T):
+        """ig_set_temperature: the temperature T >= 0 at which this chain selects its moves in the production RNG mode
+        (run_cycle_device, ReplicaSet.run_cycle).  T = 0 (the default) is the reference's argmax.  At T > 0 a step draws its
+        move among the scored proposals with probability exp((s_i - max s) / T) / sum, and the device nuisance step accepts
+        when exp((L_nuis - likelihood_t) / T) >= u (DESIGN.md 4e).  step_sampler and run_cycle (the host-RNG,
+        reference-parity entry points) refuse to run at T > 0.  Like the seed, the temperature is a run setting: checkpoints
+        do not hold it."""
+        T = float(T)
+        L.check(self._h, L.lib().ig_set_temperature(self._h, C.c_double(T)), "ig_set_temperature")
+        self.chain_temperature = T
+
+    def last_tempered_records(self, n_steps):
+        """the ig_tempered_step records of the last production-mode cycle run at T > 0 (L.TEMPERED_DTYPE)"""
+        rec = np.zeros(int(n_steps), dtype=L.TEMPERED_DTYPE)
+        assert rec.dtype.itemsize == 48
+        L.check(self._h, L.lib().ig_get_tempered_records(self._h, int(n_steps), _ptr(rec)), "ig_get_tempered_records")
+        return rec
 
     def last_nuisance_records(self, n_steps):
         """the raw ig_nuisance_step records of the last production-mode cycle (L.NUIS_DTYPE)"""

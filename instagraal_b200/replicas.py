@@ -10,8 +10,14 @@ validity list, live scaffold} across the GPUs: ``ncclAllGather`` INSIDE the libr
 (``ig_adopt_gathered``), so the set searches as one population instead of N unrelated runs.
 No PyTorch here: the launcher only has to hand every rank the 128-byte NCCL id created by rank 0
 (``nccl_unique_id`` -> file / environment / any broadcast).
-The live path of the reference has no temperature (fragment moves are an argmax, CL:1435-1446), so the chains differ by
-their seeds only; every rank takes the same decision (best chain) from the gathered table.
+The live path of the reference has no temperature (fragment moves are an argmax, CL:1435-1446): by default the chains differ
+by their seeds only, and every rank takes the same decision (best chain) from the gathered table.
+
+Tempering (DESIGN.md 4e, 6b): ``set_ladder`` gives every chain of the whole set a temperature (``sampler.set_chain_temperature``;
+T = 0 is the argmax, a hot chain also takes worse moves), and ``swap_temperatures`` exchanges the temperatures of adjacent
+rungs after a gather with the replica-exchange rule, decided identically on every rank (``swap_decisions``).  Temperatures
+move and scaffolds stay, so a swap copies nothing on the device.  Like the seeds, the ladder is a run setting: checkpoints do
+not hold it.
 """
 from __future__ import annotations
 
@@ -26,6 +32,37 @@ def best_chain(likelihoods):
     """Deterministic on every rank: highest likelihood, lowest global chain index on ties (what ig_allgather_best returns)."""
     lik = np.asarray(likelihoods, dtype=np.float64)
     return int(np.flatnonzero(lik == lik.max())[0])
+
+
+def swap_decisions(temperatures, ladder, likelihoods, round_index, swap_seed=0):
+    """One round of temperature swaps between adjacent rungs; a pure function, so every rank decides the same.
+
+    temperatures[k] = the temperature of rung k, ladder[k] = the global chain at rung k, likelihoods[g] = the live
+    log-likelihood of global chain g.  Round r tries the pairs (k, k + 1) with k = r (mod 2), with the uniforms of
+    np.random.default_rng([swap_seed, r]) (uniform k for pair k), and accepts with probability
+    min(1, exp((beta_k - beta_k+1) (L_k+1 - L_k))), beta = 1 / T.  A rung at T = 0 takes the limit: the swap is accepted iff
+    it does not lower the likelihood the colder rung holds (ties accepted); two rungs at T = 0 always swap.
+    -> (pairs tried, pairs accepted, new ladder)."""
+    T = np.asarray(temperatures, dtype=np.float64)
+    lad = np.array(ladder, dtype=np.int64)
+    lik = np.asarray(likelihoods, dtype=np.float64)
+    u = np.random.default_rng([int(swap_seed), int(round_index)]).random(max(len(T) - 1, 0))
+    tried, accepted = [], []
+    for k in range(int(round_index) % 2, len(T) - 1, 2):
+        tried.append((k, k + 1))
+        t0, t1 = T[k], T[k + 1]
+        l0, l1 = lik[lad[k]], lik[lad[k + 1]]
+        if t0 == 0.0 and t1 == 0.0:
+            ok = True
+        elif t0 == 0.0 or t1 == 0.0:
+            ok = (l1 >= l0) if t0 == 0.0 else (l0 >= l1)   # the colder rung would then hold the other chain's likelihood
+        else:
+            log_a = (1.0 / t0 - 1.0 / t1) * (l1 - l0)
+            ok = bool(log_a >= 0.0 or u[k] < np.exp(log_a))
+        if ok:
+            accepted.append((k, k + 1))
+            lad[k], lad[k + 1] = lad[k + 1], lad[k]
+    return tried, accepted, lad
 
 
 def nccl_unique_id():
@@ -53,6 +90,11 @@ class ReplicaSet:
         self.gather_ms = 0.0
         self.n_gathers = 0
         self._gathered_nc = None   # n_contigs of every chain in the last all-gather
+        self.temperatures = None   # set_ladder: temperature of every rung of the whole set, the chain at every rung
+        self.ladder = None
+        self.swap_seed = 0
+        self.swap_round = 0
+        self.swap_stats = None
         # several chains on this GPU: each takes a share of the SMs so that their (latency-bound) kernels overlap
         self.gpu_share = min(n_chains, 4)
         for c in self.chains:
@@ -132,6 +174,50 @@ class ReplicaSet:
         best, lik, nc = self.allgather()
         self.adopt(best)
         return best, lik, nc
+
+    def gathered_live_likelihood(self):
+        """the live log-likelihood (likelihood_t) of every chain [n_ranks * n] in the last all-gather"""
+        out = np.zeros(self.n_ranks * self.n, dtype=np.float64)
+        lead = self.chains[0]
+        L.check(lead._h, L.lib().ig_get_gathered_live_likelihood(lead._h, _ptr(out)), "ig_get_gathered_live_likelihood")
+        return out
+
+    def set_ladder(self, temperatures, swap_seed=0):
+        """The temperatures of the whole set's n_ranks * n rungs, assigned rank-major at first (global chain g at rung g);
+        every rank passes the same list.  Resets the swap rounds and swap_stats (tried / accepted per adjacent rung pair)."""
+        T = np.array(temperatures, dtype=np.float64)
+        if T.shape != (self.n_ranks * self.n,):
+            raise ValueError("set_ladder: %d temperatures for %d chains" % (T.size, self.n_ranks * self.n))
+        if not np.all(np.isfinite(T)) or np.any(T < 0):
+            raise ValueError("set_ladder: temperatures must be finite and >= 0")
+        self.temperatures, self.ladder = T, np.arange(T.size, dtype=np.int64)
+        self.swap_seed, self.swap_round = int(swap_seed), 0
+        self.swap_stats = {"tried": np.zeros(max(T.size - 1, 0), np.int64), "accepted": np.zeros(max(T.size - 1, 0), np.int64)}
+        self._apply_ladder()
+
+    def _apply_ladder(self):
+        rung = np.empty_like(self.ladder)
+        rung[self.ladder] = np.arange(self.ladder.size)
+        for c, ch in enumerate(self.chains):
+            T = float(self.temperatures[rung[self.rank * self.n + c]])
+            if T != ch.chain_temperature:
+                ch.set_chain_temperature(T)
+
+    def swap_temperatures(self):
+        """One all-gather, then one round of swap_decisions on the gathered live likelihoods; the local chains take their
+        rungs' new temperatures.  -> (pairs tried, pairs accepted, ladder: rung -> global chain)."""
+        if self.ladder is None:
+            raise RuntimeError("swap_temperatures: no ladder (set_ladder)")
+        self.allgather()
+        lik = self.gathered_live_likelihood()
+        tried, accepted, self.ladder = swap_decisions(self.temperatures, self.ladder, lik, self.swap_round, self.swap_seed)
+        for k, _ in tried:
+            self.swap_stats["tried"][k] += 1
+        for k, _ in accepted:
+            self.swap_stats["accepted"][k] += 1
+        self.swap_round += 1
+        self._apply_ladder()
+        return tried, accepted, self.ladder.copy()
 
     def gathered_state(self, index):
         out = np.zeros((13, self.nf), dtype=np.int32)
