@@ -143,6 +143,7 @@ k_pick(const int2* __restrict__ cv, const CoordRec* __restrict__ coord, const in
     }
 }
 
+#define IG_FLAT_ITEMS 2   // smaller slot groups until every warp of a candidate's blocks has this many items
 // LIST = false: the flat list of small levels (rows own whole 32-contact chunks, per-chunk counts, fixed order, double sums);
 // LIST = true : the pick list of the streaming path (k_stream appends in arbitrary order; sc->flat_segtotal[k] = number of
 //               records; fixed-point sums, see acc_add).
@@ -151,7 +152,7 @@ __global__ void __launch_bounds__(IG_THREADS, IG_SCORE_CTAS_PER_SM)
 k_eval_flat(const DevScalars* __restrict__ sc, const IgDescriptor* __restrict__ desc_g, int ns, const int* __restrict__ flat_cnt,
             size_t chunk_stride, const FlatRec* __restrict__ flat, size_t flat_stride, const RowMut* __restrict__ table,
             const int* __restrict__ table_len, float mbar, const float* __restrict__ exz_tab, double* __restrict__ part_nz,
-            const IgClassTab* __restrict__ clstab, int items_per_warp) {
+            const IgClassTab* __restrict__ clstab) {
     TL(6);
     TLP_DECL();
     extern __shared__ double acc_s[];                 // [IG_N_OPS][IG_THREADS]
@@ -171,7 +172,7 @@ k_eval_flat(const DevScalars* __restrict__ sc, const IgDescriptor* __restrict__ 
     const int n_recs = LIST ? sc->flat_segtotal[k] : 0;
     const int nw = n_blocks_k * IG_WARPS_PER_BLOCK;
     int gs = IG_N_OPS;
-    while (gs > 3 && tiles_k * (IG_N_OPS / gs) < items_per_warp * nw) gs >>= 1;
+    while (gs > 3 && tiles_k * (IG_N_OPS / gs) < IG_FLAT_ITEMS * nw) gs >>= 1;
     const int ng = IG_N_OPS / gs;
     const int n_items = tiles_k * ng;
     const int wg = ((int)blockIdx.x - b_first) * IG_WARPS_PER_BLOCK + w;

@@ -96,20 +96,6 @@ k_precompute(const CoordRec* __restrict__ coord, const int* __restrict__ clen, c
     }
 }
 
-// Optional (IG_PREFETCH=1) L2 prefetch of the level's arrays at the start of a step, when they fit the L2
-// comfortably (yeast-scale levels): a step is a chain of a dozen short dependent kernels, each of which takes its
-// first-touch misses to HBM one latency at a time when the L2 is cold.  Measured on T: +1.5 % with the L2 flushed
-// between steps, -3 % when steps run back to back (warm L2, the production case) -- hence off by default.
-struct PfList { const char* p[12]; unsigned long long n[12]; int cnt; };
-__global__ void k_prefetch_l2(PfList L) {
-    TL(12);
-    for (int a = 0; a < L.cnt; a++) {
-        const unsigned long long lines = (L.n[a] + 127ull) >> 7;
-        for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < lines; i += (unsigned long long)gridDim.x * blockDim.x)
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(L.p[a] + (i << 7)));
-    }
-}
-
 // K8b: THE scoring kernel (replaces slice_sp_mat + host sort + prepare_sparse_call +
 //      extract_sub_likelihood + eval_sub_likelihood).  grid = (G, n_cands).  Work item = (affected
 //      CSR row, group of GS uniq slots); a warp takes one item at a time, its lanes stride the row's
@@ -151,8 +137,8 @@ __device__ __noinline__ void eval_queue(const QEnt* __restrict__ q, int n, doubl
     const int lane = threadIdx.x & 31;
     if (lane < n) {
         const QEnt e = q[lane];
-        const float exf = fmaxf((p.d == 2.0f) ? (p.c1 * IG_POWF(e.s, p.slope)) * p.fact
-                                              : (p.c1 * IG_POWF(e.s, p.slope) * expf((p.d - 2) / (IG_POWF(e.s * p.lm / p.kuhn, 2.0f) + p.d))) * p.fact,
+        const float exf = fmaxf((p.d == 2.0f) ? (p.c1 * powf_pos(e.s, p.slope)) * p.fact
+                                              : (p.c1 * powf_pos(e.s, p.slope) * expf((p.d - 2) / (powf_pos(e.s * p.lm / p.kuhn, 2.0f) + p.d))) * p.fact,
                                 p.v_inter);  // rippe_contacts for 0 < s < d_max (KA:153-163)
         double t = pxl_term(exf, (double)e.val, 0.0, l10v, p.v_inter) + (double)exz_tab[e.dp] * LOG10E_F;
         if (e.mask & IG_QSUB) t = -t;
@@ -237,6 +223,8 @@ __device__ __forceinline__ void queue_push(bool push, float s, int dp, unsigned 
 //     the ROW end is warp-uniform and staged from the k_precompute table into shared memory once per item.
 //   * A pair whose (same-contig flag, s, sub-fragment separation) is bit-identical to the current state is
 //     skipped; the rest is either a cheap constant (other contig / outside (0, d_max)) or goes to the queue.
+#define IG_GS_DIV 4       // split a row into slot groups while rows * groups < warps / IG_GS_DIV
+#define IG_SPARSE_DIV 4   // deal (contact, mutation) pairs to the lanes when fewer than 32 / IG_SPARSE_DIV lanes are busy
 __global__ void __launch_bounds__(IG_THREADS, IG_SCORE_CTAS_PER_SM)
 k_score(const long long* __restrict__ row_ptr, const int2* __restrict__ cv, const CoordRec* __restrict__ coord,
         const int* __restrict__ clen, const DevScalars* __restrict__ sc, const IgDescriptor* __restrict__ desc_g,
@@ -244,9 +232,8 @@ k_score(const long long* __restrict__ row_ptr, const int2* __restrict__ cv, cons
         const RowMut* __restrict__ table, const int* __restrict__ table_len, float mbar, const float* __restrict__ exz_tab,
         double* __restrict__ part_nz,   // [cand][25][gridDim.x]  (24 uniq slots; slot 24 unused = 0)
         int* __restrict__ part_c,       // [cand][2][gridDim.x]   (contacts selected, contacts read)
-        int gs_div,                     // work-splitting knob: split a row into slot groups while rows*groups < warps/gs_div
         const IgClassTab* __restrict__ clstab, const SubX* __restrict__ subx, const RowInfo* __restrict__ rinfo,
-        int sparse_div)                 // deal (contact, mutation) pairs to the lanes when fewer than 32/sparse_div lanes are busy
+        int2 split)                     // (slots per item, parts per row) forced by tests; (0, 0): chosen from the work
 {
     TL(6);
     TLB();
@@ -269,24 +256,15 @@ k_score(const long long* __restrict__ row_ptr, const int2* __restrict__ cv, cons
     // part when there are more rows than warps, fewer slots per item and rows cut into `parts` interleaved
     // chunk sets when a candidate has few rows (yeast-scale assemblies), so that the grid stays occupied and
     // the longest row does not set the kernel's critical path.
-    // (IG_BLOCK_MODE: one BLOCK per item, kept for experiments -- measured slower at yeast scale.)
-    const bool block_mode = (gs_div < 0) && ci_k.n_rows < nw / (-gs_div);
-    const int div = gs_div < 0 ? -gs_div : gs_div;
     int gs = IG_N_OPS, parts = 1;
-    if (block_mode) {
-        const int want = (int)gridDim.x / 2;
-        gs = (ci_k.n_rows >= want) ? 24 : ((ci_k.n_rows * 4 >= want) ? 6 : ((ci_k.n_rows * 8 >= want) ? 3 : 1));
-    } else {
-        const int want = nw / div;
-        if (ci_k.n_rows < want) gs = (ci_k.n_rows * 4 >= want) ? 6 : ((ci_k.n_rows * 8 >= want) ? 3 : 1);
-        if (ci_k.n_rows * (IG_N_OPS / gs) * 2 <= nw) parts = 2;
-        if (ci_k.n_rows * (IG_N_OPS / gs) * 4 <= nw) parts = 4;
-        if (sparse_div >> 16) { gs = (sparse_div >> 16) & 0xff; parts = (sparse_div >> 24) & 0xff; }  // experiments: forced split
-    }
+    const int want = nw / IG_GS_DIV;
+    if (ci_k.n_rows < want) gs = (ci_k.n_rows * 4 >= want) ? 6 : ((ci_k.n_rows * 8 >= want) ? 3 : 1);
+    if (ci_k.n_rows * (IG_N_OPS / gs) * 2 <= nw) parts = 2;
+    if (ci_k.n_rows * (IG_N_OPS / gs) * 4 <= nw) parts = 4;
+    if (split.x) { gs = split.x; parts = split.y; }
     const int ng = IG_N_OPS / gs;
     const int n_items = ci_k.n_rows * ng * parts;
-    const int it0 = block_mode ? (int)blockIdx.x : wg, it_step = block_mode ? (int)gridDim.x : nw;
-    if ((block_mode ? (int)blockIdx.x : (int)blockIdx.x * IG_WARPS_PER_BLOCK) >= n_items) {  // nothing for this block
+    if ((int)blockIdx.x * IG_WARPS_PER_BLOCK >= n_items) {  // nothing for this block
         if (threadIdx.x < 25) part_nz[PART_IDX(k, 25, threadIdx.x, gridDim.x, blockIdx.x)] = 0.0;
         if (threadIdx.x < 2) part_c[PART_IDX(k, 2, threadIdx.x, gridDim.x, blockIdx.x)] = 0;
         return;
@@ -316,14 +294,14 @@ k_score(const long long* __restrict__ row_ptr, const int2* __restrict__ cv, cons
     RowMut* myrow = s_row[w];
     unsigned* mychg = s_chg[w];
     int* myoff = s_off[w];
-    // constant term of a contact whose endpoints lie in different contigs (KA:4348-4352) minus the ob part
-    const double inter_const = (double)p.v_inter * LOG10E_F;
+    // (double)p.v_inter * LOG10E_F below: the constant term of a contact whose endpoints lie in different contigs
+    // (KA:4348-4352) minus the ob part, written out at each use -- held in a variable it costs k_score spill slots
     TLP(0);   // block prologue
-    for (int it = it0; it < n_items; it += it_step) {
+    for (int it = wg; it < n_items; it += nw) {
         TLB_ITEM();
         const int rg = it / parts, part = it - rg * parts;
         const int ri = rg / ng, g = rg - ri * ng;
-        const int q_off = block_mode ? 32 * w : 32 * part, q_step = block_mode ? 32 * IG_WARPS_PER_BLOCK : 32 * parts;
+        const int q_off = 32 * part, q_step = 32 * parts;
         const int u0 = g * gs;
         if (u0 >= n_uniq && g != 0) continue;
         const int u1 = min(u0 + gs, n_uniq);
@@ -366,15 +344,13 @@ k_score(const long long* __restrict__ row_ptr, const int2* __restrict__ cv, cons
                     const bool cur_same = ci.id_c == cj.id_c;
                     m = __ldg(&mrow[x.rjc >> IG_CLS_SHIFT]) & gmask;
                     // far beyond d_max before and after: every non-reflecting mutation leaves the floor term
-#ifndef IG_NO_FAR
                     if (m && cur_same && ci.s_tot == 0 && x.cur_s >= far_s && x.cur_dp >= far_dp)
                         m &= ~__ldg(&g_farok[cls_r * IG_MAX_CLS + (x.rjc >> IG_CLS_SHIFT)]);
-#endif
                     if (m) {  // current-state term of the lanes that have something to evaluate
                         const SubX sx = subx[c.x];
                         x.start_bp = sx.start_bp; x.len_ori = sx.len_ori; x.watson = sx.watson; x.crick = sx.crick;
                         const double ob = (double)c.y;
-                        if (!cur_same) x.t_cur = pxl_term(p.v_inter, ob, 0.0, l10v, p.v_inter) + inter_const;
+                        if (!cur_same) x.t_cur = pxl_term(p.v_inter, ob, 0.0, l10v, p.v_inter) + (double)p.v_inter * LOG10E_F;
                         else if (ci.s_tot != 0) x.t_cur = contact_term(ci, cj, clen[c.x], ob, 0.0, p, l10v, mbar, exz_tab);  // circular (rare)
                         else if (!((x.cur_s > 0.0f) && (x.cur_s < p.d_max))) x.t_cur = pxl_term(p.v_inter, ob, 0.0, l10v, p.v_inter) + (double)exz_tab[x.cur_dp] * LOG10E_F;
                         else x.flags |= 2;  // powf + log10: goes through the queue once, with the mask of changed slots
@@ -391,7 +367,7 @@ k_score(const long long* __restrict__ row_ptr, const int2* __restrict__ cv, cons
             unsigned chg = 0;
             // number of (contact, mutation) pairs of this chunk
             const int n_pairs = __reduce_add_sync(0xffffffffu, __popc(mr));
-            if (n_pairs * (sparse_div & 0xffff) > __popc(um) * 32) {
+            if (n_pairs * IG_SPARSE_DIV > __popc(um) * 32) {
                 // DENSE: most lanes take part in most mutations -> loop over the mutations, lane = contact
 #pragma unroll 1
                 for (unsigned uw = um; uw; uw &= uw - 1) {
@@ -400,7 +376,7 @@ k_score(const long long* __restrict__ row_ptr, const int2* __restrict__ cv, cons
                     unsigned mem = 1u << (u - u0);
                     if ((mr >> u) & 1u) {
                         double add;
-                        if (eval_pair(x, u, myrow[u - u0], g_mot, ci.s_tot, p, l10v, inter_const, mbar, exz_tab, tab, tlen, ns, s_m, dp_m, push, add)) {
+                        if (eval_pair(x, u, myrow[u - u0], g_mot, ci.s_tot, p, l10v, (double)p.v_inter * LOG10E_F, mbar, exz_tab, tab, tlen, ns, s_m, dp_m, push, add)) {
                             if (dedup) mem = __ldg(&g_mem[t_pair * IG_N_OPS + u]) & m;
                             chg |= mem;
                             for (unsigned mm = mem; mm; mm &= mm - 1) my_acc[(__ffs(mm) - 1) * IG_THREADS] += add;
@@ -442,7 +418,7 @@ k_score(const long long* __restrict__ row_ptr, const int2* __restrict__ cv, cons
                         u = __fns(msrc, 0, pi - myoff[src] + 1);
                         mem = 1u << (u - u0);
                         double add;
-                        if (eval_pair(y, u, myrow[u - u0], g_mot, ci.s_tot, p, l10v, inter_const, mbar, exz_tab, tab, tlen, ns, s_m, dp_m, push, add)) {
+                        if (eval_pair(y, u, myrow[u - u0], g_mot, ci.s_tot, p, l10v, (double)p.v_inter * LOG10E_F, mbar, exz_tab, tab, tlen, ns, s_m, dp_m, push, add)) {
                             if (dedup) mem = __ldg(&g_mem[(cls_r * IG_MAX_CLS + (y.rjc >> IG_CLS_SHIFT)) * IG_N_OPS + u]) & mfull;
                             atomicOr(&mychg[src], mem);
                             for (unsigned mm = mem; mm; mm &= mm - 1) my_acc[(__ffs(mm) - 1) * IG_THREADS] += add;
@@ -472,8 +448,7 @@ k_score(const long long* __restrict__ row_ptr, const int2* __restrict__ cv, cons
             row_sel = __reduce_add_sync(0xffffffffu, row_sel);
             if (lane == 0) {
                 redi[w][0] += row_sel;
-                if (block_mode) { if (row_sel) atomicAdd(&my_cnt[ri], row_sel); if (w == 0) redi[w][1] += (int)(e - b); }
-                else if (parts > 1) { if (row_sel) atomicAdd(&my_cnt[ri], row_sel); if (part == 0) redi[w][1] += (int)(e - b); }
+                if (parts > 1) { if (row_sel) atomicAdd(&my_cnt[ri], row_sel); if (part == 0) redi[w][1] += (int)(e - b); }
                 else { my_cnt[ri] = row_sel; redi[w][1] += (int)(e - b); }
             }
         }

@@ -323,7 +323,7 @@ k_rows_write(const CoordRec* __restrict__ coord, int ns, const DevScalars* __res
         const long long rb = row_ptr[r];
         RowInfo ri; ri.r = r; ri.cls = cls; ri.n = (int)(row_ptr[r + 1] - rb); ri.pad = 0; ri.b = rb; ri.seg = 0; ri.ci = cr;
         rinfo[(size_t)k * rows_stride + off] = ri;
-        row_cnt[(size_t)k * rows_stride + off] = 0;  // k_score (block mode) accumulates into it
+        row_cnt[(size_t)k * rows_stride + off] = 0;  // k_score (rows cut into parts) and k_stream accumulate into it
     }
 }
 

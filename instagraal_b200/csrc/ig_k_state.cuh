@@ -55,12 +55,12 @@ k_coords(const FragRec* __restrict__ live, const SubRec* __restrict__ sub, Coord
 struct __align__(8) LnzQ { float s; int val; };
 #define IG_LNZ_QCAP 96
 __device__ __forceinline__ double lnz_eval(const LnzQ e, const Params& p, double l10v) {
-    const float pw = IG_POWF(e.s, p.slope);
+    const float pw = powf_pos(e.s, p.slope);
     float exf;
     if (p.d == 2.0f) exf = __fmul_rn(__fmul_rn(p.c1, pw), p.fact);
     else exf = (p.c1 * pw * expf((p.d - 2) / (powf(e.s * p.lm / p.kuhn, 2.0f) + p.d))) * p.fact;
     exf = fmaxf(exf, p.v_inter);
-    const double lg = (exf == p.v_inter) ? l10v : IG_LOG10F(exf);
+    const double lg = (exf == p.v_inter) ? l10v : log10_f32(exf);
     return (double)e.val * lg - (double)exf;
 }
 __global__ void __launch_bounds__(IG_THREADS)

@@ -15,8 +15,8 @@
 //     the fly from its class motion with the reference's float32 operations.
 //   * scores are sums of DIFFERENCES to the current state over the contacts whose term changes;
 //     class-pair bit tables say which (contact, mutation) pairs need a look at all.
-//   * two scoring paths: k_score (warp per affected row, large levels) and k_pick + k_eval_flat (packed
-//     per-chunk contact lists, levels up to 1.5 M contacts).
+//   * three scoring paths, one per handle (choose_scoring): flat (k_pick + k_eval_flat, small levels), stream
+//     (k_stream + k_eval_flat, large levels) and rows (k_score, a warp per affected row, the largest levels).
 //   * all sums in double, fixed (deterministic) reduction order: lane -> warp shuffle -> block ->
 //     partial array -> single-block tree.  No floating-point atomics anywhere.
 //   * expected contacts in float32 exactly as the reference kernel writes them (same libdevice
@@ -37,14 +37,13 @@
 #include "../../include/instagraal_b200.h"
 #include "ig_moves.cuh"
 
-#ifndef IG_WARPS_PER_BLOCK
 #define IG_WARPS_PER_BLOCK 8
-#endif
 #define IG_SCORE_CTAS_PER_SM (24 / IG_WARPS_PER_BLOCK)
 #define IG_THREADS (IG_WARPS_PER_BLOCK * 32)
 #define IG_ROW_CHUNK 1024
 #define IG_FLAT_MAX_NNZ 1500000   // levels up to 1.5 M stored contacts take the flat scoring path (list: 64 B x nnz x 8)
 #define IG_ROWS_SMALL_CHUNKS 16  // levels of up to 16 Ki sub-fragments build the affected-row list in one launch
+#define IG_STREAM_SMEM_MAX (200 * 1024)   // largest membership bitmap (NS / 8 bytes) k_stream stages in shared memory
 #define IG_LANE_CUR 24  // lane that owns the current-state zero term in the score kernel
 
 struct Params { float kuhn, lm, c1, slope, d, d_max, fact, v_inter; };  // KA:91-100
@@ -141,6 +140,12 @@ struct LevelBlock {
     int* sym_diag;
     long long* nb_ptr; int* nb_idx; double* nb_cdf; int* nb_nnz;
 };
+// How a step scores its candidates (choose_scoring):
+//   PATH_FLAT    k_rows_small -> k_pick -> k_eval_flat<false>
+//   PATH_STREAM  k_rows_count / k_rows_write -> k_stream -> k_eval_flat<true>, beside k_score for the candidates k_cand_setup
+//                leaves to it (circular contigs; reference-faithful mode: candidates whose picks might not fit the list)
+//   PATH_ROWS    k_rows_count / k_rows_write -> k_score (a warp per affected row) for every candidate
+enum ScoringPath { PATH_FLAT, PATH_STREAM, PATH_ROWS };
 struct ig_replica_state;
 struct ig_handle {
     ig_config cfg;
@@ -150,11 +155,9 @@ struct ig_handle {
     long long nnz;
     cudaStream_t stream, side, pf;
     cudaEvent_t ev_coords, ev_lnz, ev_fork, ev_sel, ev_out, ev_cuts, ev_cls, ev_pre, ev_ksc;
-    bool rows_small;  // affected-row list in one launch (small levels)
-    bool flat;        // flat scoring path (k_pick + k_eval_flat) for small levels
-    int grid_flat, flat_items; int* flat_cnt; FlatRec* flat_list; size_t flat_stride, chunk_stride;
-    bool prefetch;  // the level's arrays fit the L2 comfortably: prefetch them at the start of a step
-    bool streaming; // streaming scoring path (k_stream + k_eval_flat<true>): large levels with rigid_pruning != 0
+    ScoringPath path;   // chosen once per handle (choose_scoring)
+    int2 split;         // k_score's (slots per item, parts per row) forced by IG_FORCE_SPLIT; (0, 0): chosen from the work
+    int grid_flat; int* flat_cnt; FlatRec* flat_list; size_t flat_stride, chunk_stride;
     unsigned* bitmap; int bitmap_words; unsigned short* cls16; FlatRec* pick_list; size_t pick_cap; int stream_smem;
     int stream_rows_max;   // candidates with at most this many affected rows take the streaming path (exact mode: bounded by the pick list)
     FragRec *live, *init_live;
@@ -189,7 +192,6 @@ struct ig_handle {
     bool vinter_pos;  // live v_inter > 0 (the per-contact records assume it)
     bool lnz_stale;   // the parameters changed since lnz_full / z_cur were computed (the scaffold bookkeeping is intact)
     double* part_out;
-    int gs_div, sparse_div, grid_split;
     long long last_n_full;
     // one graph per [step kind + 4 * cycle][shape]: shape = candidates in the grid (1 .. IG_MAX_CANDS) of a narrow step,
     // IG_MAX_CANDS + number of batches of a wide step (get_graph)
@@ -260,6 +262,58 @@ static int upload_state(ig_handle* h, const int32_t* in13, FragRec* dst) {
     return 0;
 }
 
+// The handle's scoring path and what it sizes, decided once per handle: PATH_FLAT up to 16 Ki sub-fragments and 1.5 M
+// contacts, otherwise PATH_STREAM while the membership bitmap fits k_stream's shared memory, otherwise PATH_ROWS; the pick
+// list of the streaming path; whether the per-contact likelihood records fit the level.  Tests override the choice:
+// IG_SCORING_PATH=flat|stream|rows, IG_FORCE_SPLIT=gs,parts (k_score's work split: gs uniq slots per item, rows cut into
+// `parts`; it selects no path, so it acts wherever k_score runs: every candidate of the rows path, the candidates the stream
+// path leaves to it, none of the flat path), IG_LNZ_CACHE=0|1.  An override that is malformed or that the level cannot
+// honour fails ig_create.
+static int choose_scoring(ig_handle* h) {
+    const bool flat_ok = h->n_chunks <= IG_ROWS_SMALL_CHUNKS, stream_ok = h->stream_smem <= IG_STREAM_SMEM_MAX;
+    h->path = (flat_ok && h->nnz <= IG_FLAT_MAX_NNZ) ? PATH_FLAT : stream_ok ? PATH_STREAM : PATH_ROWS;
+    if (const char* e = getenv("IG_SCORING_PATH")) {
+        if (!strcmp(e, "flat") && flat_ok) h->path = PATH_FLAT;
+        else if (!strcmp(e, "stream") && stream_ok) h->path = PATH_STREAM;
+        else if (!strcmp(e, "rows")) h->path = PATH_ROWS;
+        else {
+            h->err = std::string("ig_create: IG_SCORING_PATH=") + e + " is not one of flat, stream, rows that this level can take "
+                     "(flat: up to 16 Ki sub-fragments; stream: up to 1.6 M sub-fragments)";
+            return -1;
+        }
+    }
+    h->split = make_int2(0, 0);
+    if (const char* e = getenv("IG_FORCE_SPLIT")) {
+        int gs = 0, parts = 0, len = 0;
+        if (sscanf(e, "%d,%d%n", &gs, &parts, &len) != 2 || e[len] || gs <= 0 || IG_N_OPS % gs || parts < 1 || parts > 32) {
+            h->err = std::string("ig_create: IG_FORCE_SPLIT=") + e + " is not gs,parts (gs divides 24, 1 <= parts <= 32)";
+            return -1;
+        }
+        h->split = make_int2(gs, parts);
+    }
+    h->pick_cap = 0; h->stream_rows_max = 0;
+    if (h->path == PATH_STREAM) {
+        h->pick_cap = std::min<size_t>((size_t)h->nnz + 64, (size_t)2 << 20);   // 64-byte records: 128 MB per candidate slot at most
+        // rigid pruning: every linear candidate (a few per cent of its contacts are picked).  Reference-faithful mode: almost
+        // every selected contact is a pick, so only candidates whose contacts are sure to fit the pick list take it (the
+        // mid-assembly regime: two contigs of a few hundred sub-fragments, where the row-per-warp kernel is all latency)
+        h->stream_rows_max = h->rigid ? INT32_MAX : (int)std::min<long long>(INT32_MAX, (long long)h->pick_cap / std::max<long long>(h->lvl->max_row_len, 1));
+    }
+    // packed likelihood records: table index (sub-fragment separation, or one of two special slots) in the low bits, the
+    // observed count above them
+    h->dp_bits = 1;
+    while ((1 << h->dp_bits) < h->ns + 3) h->dp_bits++;
+    h->lnz_cache = h->nnz > 0 && h->dp_bits <= 24 && (long long)h->lvl->max_val < (1LL << (32 - h->dp_bits));
+    if (const char* e = getenv("IG_LNZ_CACHE")) {
+        if (!strcmp(e, "0")) h->lnz_cache = false;
+        else if (strcmp(e, "1") || !h->lnz_cache) {
+            h->err = std::string("ig_create: IG_LNZ_CACHE=") + e + " is not 0, or 1 on a level whose counts and size fit the records";
+            return -1;
+        }
+    }
+    return 0;
+}
+
 // parent != nullptr: a further chain on the same level (ig_clone): the level's read-only arrays are borrowed, not uploaded
 static int create_impl(const ig_config* cfg, const ig_level_data* data, ig_handle* parent, ig_handle** out) {
     ig_handle* h = nullptr;
@@ -277,17 +331,6 @@ static int create_impl(const ig_config* cfg, const ig_level_data* data, ig_handl
     h->rigid = cfg->rigid_pruning ? 1 : 0;
     h->params_set = false; h->coords_fresh = false; h->coords_ever = false;
     h->incr_valid = false; h->lnz_stale = false; h->refresh_every = 4096; h->steps_since_full = 0;
-    h->gs_div = 4;
-    h->sparse_div = 4;
-    h->grid_split = 0;
-    if (const char* e = getenv("IG_GRID_SPLIT")) h->grid_split = atoi(e);   // 0: the full grid per candidate (experiments)
-    if (const char* e = getenv("IG_SPARSE_DIV")) h->sparse_div = atoi(e) & 0xffff;
-    if (const char* e = getenv("IG_FORCE_SPLIT")) {  // "gs,parts" (experiments)
-        int g = 0, pp = 0;
-        if (sscanf(e, "%d,%d", &g, &pp) == 2 && g > 0 && pp > 0 && IG_N_OPS % g == 0) h->sparse_div |= (g << 16) | (pp << 24);
-    }
-    if (const char* e = getenv("IG_GS_DIV")) h->gs_div = std::max(1, atoi(e));
-    if (const char* e = getenv("IG_BLOCK_MODE")) if (atoi(e)) h->gs_div = -h->gs_div;
     memset(h->graph, 0, sizeof h->graph); h->cyc_plan = nullptr; h->cyc_out = nullptr; h->cyc_frags = nullptr;
     h->cyc_cap = 0; h->cyc_width = 0; h->plan_width = IG_MAX_CANDS;
     h->graph_failed = false; h->capturing = false; h->use_graph = true; h->n_full = 0; h->pending_steps = 0; h->rep = nullptr;
@@ -319,6 +362,11 @@ static int create_impl(const ig_config* cfg, const ig_level_data* data, ig_handl
         } else {
             h->lvl = new LevelBlock();
             memset(h->lvl, 0, sizeof(LevelBlock)); h->lvl->refs = 1;
+            long long mr = 0, tot = 0;
+            int mv = 0;
+            for (int r = 0; r < ns; r++) mr = std::max(mr, (long long)(data->row_ptr[r + 1] - data->row_ptr[r]));
+            for (long long i = 0; i < h->nnz; i++) { mv = std::max(mv, data->val[i]); tot += data->val[i]; }
+            h->lvl->max_row_len = mr; h->lvl->max_val = mv; h->lvl->val_total = (double)tot;
             if (dev_alloc(h, &h->init_live, nf) || dev_alloc(h, &h->sub, ns)) return -2;
             if (dev_alloc(h, &h->row_ptr, (size_t)ns + 1) || dev_alloc(h, &h->cv, (size_t)h->nnz + 2)) return -2;
             if (dev_alloc(h, &h->init_prev, nf) || dev_alloc(h, &h->init_next, nf) || dev_alloc(h, &h->orientable, nf)) return -2;
@@ -327,41 +375,18 @@ static int create_impl(const ig_config* cfg, const ig_level_data* data, ig_handl
         if (dev_alloc(h, &h->exz, (size_t)ns + 3) || dev_alloc(h, &h->exz_test, (size_t)ns + 3)) return -2;   // + the two slots of k_lnz_stream
         h->n_chunks = (ns + IG_ROW_CHUNK - 1) / IG_ROW_CHUNK;
         if (dev_alloc(h, &h->chunk_cnt, (size_t)IG_MAX_CANDS * h->n_chunks)) return -2;
-        h->rows_small = h->n_chunks <= IG_ROWS_SMALL_CHUNKS;
-        if (const char* e = getenv("IG_ROWS_SMALL")) h->rows_small = h->rows_small && atoi(e) != 0;   // tests: force the two-pass list
-        h->flat = h->rows_small && h->nnz <= IG_FLAT_MAX_NNZ;
-        if (const char* e = getenv("IG_FLAT")) h->flat = h->flat && atoi(e) != 0;
-        if (getenv("IG_FORCE_SPLIT")) h->flat = false;   // experiments / tests of the row-per-warp kernel
+        h->bitmap_words = (ns + 31) / 32;
+        h->stream_smem = h->bitmap_words * (int)sizeof(unsigned);
+        if (int rc = choose_scoring(h)) return rc;
         h->flat_cnt = nullptr; h->flat_list = nullptr; h->flat_stride = (size_t)h->nnz + 32 * (size_t)ns + 32;   // rows own whole 32-contact chunks
         h->chunk_stride = h->flat_stride / 32 + 1;
-        if (h->flat) {
+        if (h->path == PATH_FLAT) {
             if (dev_alloc(h, &h->flat_cnt, (size_t)IG_MAX_CANDS * h->chunk_stride) ||
                 dev_alloc(h, &h->flat_list, (size_t)IG_MAX_CANDS * h->flat_stride)) return -2;
         }
         if (dev_alloc(h, &h->rows, (size_t)IG_MAX_CANDS * ns) || dev_alloc(h, &h->row_cnt, (size_t)IG_MAX_CANDS * ns)) return -2;
         h->bitmap = nullptr; h->cls16 = nullptr; h->pick_list = nullptr;
-        h->bitmap_words = (ns + 31) / 32;
-        h->stream_smem = h->bitmap_words * (int)sizeof(unsigned);
-        // rigid pruning: every linear candidate (a few per cent of its contacts are picked).  Reference-faithful mode: almost
-        // every selected contact is a pick, so only candidates whose contacts are sure to fit the pick list take it (the
-        // mid-assembly regime: two contigs of a few hundred sub-fragments, where the row-per-warp kernel is all latency)
-        h->streaming = !h->flat && h->stream_smem <= 200 * 1024;
-        if (const char* e = getenv("IG_STREAM")) h->streaming = h->streaming && atoi(e) != 0;   // experiments / tests
-        if (getenv("IG_FORCE_STREAM") && h->stream_smem <= 200 * 1024) {   // tests: small levels through the streaming path
-            h->streaming = true; h->flat = false;
-        }
-        h->stream_rows_max = 0;
-        if (h->streaming) {
-            h->rows_small = false;   // the two-pass row list also writes the bitmap and the class words
-            h->pick_cap = std::min<size_t>((size_t)h->nnz + 64, (size_t)2 << 20);   // 64-byte records: 128 MB per candidate slot at most
-            if (const char* e = getenv("IG_PICK_CAP")) h->pick_cap = (size_t)std::max(64, atoi(e));
-            if (!parent) {
-                long long mr = 0;
-                for (int r = 0; r < ns; r++) mr = std::max(mr, (long long)(data->row_ptr[r + 1] - data->row_ptr[r]));
-                h->lvl->max_row_len = mr;
-            }
-            h->stream_rows_max = h->rigid ? INT32_MAX : (int)std::min<long long>(INT32_MAX, (long long)h->pick_cap / std::max<long long>(h->lvl->max_row_len, 1));
-            if (const char* e = getenv("IG_STREAM_ROWS")) h->stream_rows_max = atoi(e);   // experiments
+        if (h->path == PATH_STREAM) {   // (the two-pass row list also writes the bitmap and the class words)
             if (dev_alloc(h, &h->bitmap, (size_t)IG_MAX_CANDS * h->bitmap_words) || dev_alloc(h, &h->cls16, (size_t)IG_MAX_CANDS * ns) ||
                 dev_alloc(h, &h->pick_list, (size_t)IG_MAX_CANDS * h->pick_cap)) return -2;
             CK(cudaFuncSetAttribute(k_stream, cudaFuncAttributeMaxDynamicSharedMemorySize, h->stream_smem));
@@ -375,14 +400,7 @@ static int create_impl(const ig_config* cfg, const ig_level_data* data, ig_handl
         CK(cudaFuncSetAttribute(k_eval_flat<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)IG_SCORE_SMEM));
         CK(cudaFuncSetAttribute(k_eval_flat<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)IG_SCORE_SMEM));
         h->grid_flat = (sms * IG_SCORE_CTAS_PER_SM) / 5;   // k_pick grid per candidate: a step's (usually 5) candidates fill the GPU once
-        h->flat_items = 2;
-        if (const char* e = getenv("IG_FLAT_ITEMS")) h->flat_items = std::max(1, atoi(e));   // a step's (usually 5) candidates fill the GPU once
         h->grid_pre = std::min(sms * 2, (ns + 31) / 32);   // 2 resident CTAs of 25 warps per SM; one tile of 32 rows per block at most
-        {
-            const char* e = getenv("IG_PREFETCH");
-            const size_t bytes = sizeof(int2) * (size_t)h->nnz + 64 * (size_t)ns + 80 * (size_t)nf;
-            h->prefetch = e ? (atoi(e) != 0 && bytes <= ((size_t)48 << 20)) : false;
-        }
         if (dev_alloc(h, &h->part_nz, (size_t)IG_MAX_CANDS * h->grid_score * 25)) return -2;
         if (dev_alloc(h, &h->part_c, (size_t)IG_MAX_CANDS * h->grid_score * 2)) return -2;
         if (dev_alloc(h, &h->part_z, (size_t)IG_MAX_CANDS * h->grid_pre * 25)) return -2;
@@ -393,7 +411,7 @@ static int create_impl(const ig_config* cfg, const ig_level_data* data, ig_handl
         if (dev_alloc(h, &h->clstab, (size_t)IG_MAX_CANDS) || dev_alloc(h, &h->subx, (size_t)ns) || dev_alloc(h, &h->rinfo, (size_t)IG_MAX_CANDS * ns)) return -2;
         h->n_part_full = sms * 8;
         if (dev_alloc(h, &h->part_full, 2 * (size_t)h->n_part_full)) return -2;
-        h->lnz_rec = nullptr; h->row_dirty = nullptr; h->lnz_cache = false; h->grid_lnz = sms * 4;
+        h->lnz_rec = nullptr; h->row_dirty = nullptr; h->grid_lnz = sms * 4;
         if (dev_alloc(h, &h->part_out, h->n_part_full)) return -2;
         h->n_part_zc = sms * 2;
         if (dev_alloc(h, &h->part_zc, h->n_part_zc) || dev_alloc(h, &h->part_nc, h->n_part_zc)) return -2;
@@ -437,19 +455,9 @@ static int create_impl(const ig_config* cfg, const ig_level_data* data, ig_handl
             CK(h2d_sync(h->init_next, data->init_next, sizeof(int) * nf));
             CK(h2d_sync(h->orientable, data->orientable, sizeof(int) * nf));
         }
-        if (!parent) {
-            int mv = 0; long long tot = 0;
-            for (long long i = 0; i < h->nnz; i++) { mv = std::max(mv, data->val[i]); tot += data->val[i]; }
-            h->lvl->max_val = mv; h->lvl->val_total = (double)tot;
-        }
-        {   // packed likelihood records: table index (sub-fragment separation, or one of two special slots) in the low
-            // bits, the observed count above them; streamed in whole trips of 64 record pairs
-            h->dp_bits = 1;
-            while ((1 << h->dp_bits) < ns + 3) h->dp_bits++;
+        {   // packed likelihood records (choose_scoring), streamed in whole trips of 64 record pairs
             h->lnz_pairs = ((h->nnz + 1) / 2 + 63) / 64 * 64;
             h->lnz_pad = (int)(2 * h->lnz_pairs - h->nnz);
-            h->lnz_cache = h->nnz > 0 && h->dp_bits <= 24 && (long long)h->lvl->max_val < (1LL << (32 - h->dp_bits));
-            if (const char* e = getenv("IG_LNZ_CACHE")) h->lnz_cache = h->lnz_cache && atoi(e) != 0;   // tests / A-B runs
             if (h->lnz_cache) {
                 if (dev_alloc(h, &h->lnz_rec, (size_t)(2 * h->lnz_pairs)) || dev_alloc(h, &h->row_dirty, (size_t)ns)) return -2;
                 std::vector<int2> pad(h->lnz_pad);
@@ -669,19 +677,12 @@ static int labels_guard(ig_handle* h) {
     return ig_set_state(h, st.data());
 }
 
-// k_score grid: the candidates of a step run side by side, so the resident capacity (3 CTAs per SM) is shared
-// between them -- one wave for the whole step instead of one (mostly latency) wave per candidate
-static int score_grid_x(const ig_handle* h, int n) {
-    if (h->grid_split <= 0) return h->grid_score;
-    return std::max(h->grid_score / std::max(n, 1), h->grid_score / 8) * h->grid_split;
-}
-
 // rows + precompute + scoring kernels of one pass (after k_cand_setup / k_find_cuts were enqueued, k_classes on h->pf)
 #define IG_MARK(i) do { if (h->profile && !h->capturing) cudaEventRecord(h->evk[i], h->stream); } while (0)
 static void enqueue_scoring(ig_handle* h, int n) {
     const float mbar = h->cfg.mean_sub_len_kb;
     const FragRec* live = h->live;
-    if (h->rows_small) {
+    if (h->path == PATH_FLAT) {
         IG_MARK(3);
         k_rows_small<<<n, IG_ROW_CHUNK, 0, h->stream>>>(h->coord, h->ns, h->sc, h->n_chunks, h->rows, h->rowidx, h->row_cnt, h->ns,
                                                         h->clstab, h->row_ptr, h->rinfo);
@@ -698,31 +699,30 @@ static void enqueue_scoring(ig_handle* h, int n) {
     if (h->profile && !h->capturing) cudaEventRecord(h->ev[4], h->stream);
     cudaStreamWaitEvent(h->stream, h->ev_cls, 0);
     IG_MARK(5);
-    const int gsx = h->flat ? h->grid_flat : score_grid_x(h, n);
-    if (h->flat) {
-        k_pick<<<dim3(gsx, n), IG_THREADS, 0, h->stream>>>(h->cv, h->coord, h->clen, h->sc, h->desc, h->rowidx, h->ns, h->row_cnt,
+    if (h->path == PATH_FLAT) {
+        k_pick<<<dim3(h->grid_flat, n), IG_THREADS, 0, h->stream>>>(h->cv, h->coord, h->clen, h->sc, h->desc, h->rowidx, h->ns, h->row_cnt,
                                                                     h->flat_cnt, h->chunk_stride, h->part_c, h->flat_list, h->flat_stride, mbar, h->exz,
                                                                     h->clstab, h->subx, h->rinfo);
         k_eval_flat<false><<<h->grid_score, IG_THREADS, IG_SCORE_SMEM, h->stream>>>(h->sc, h->desc, h->ns, h->flat_cnt, h->chunk_stride, h->flat_list,
-                                                                            h->flat_stride, h->table, h->table_len, mbar, h->exz, h->part_nz, h->clstab, h->flat_items);
+                                                                            h->flat_stride, h->table, h->table_len, mbar, h->exz, h->part_nz, h->clstab);
     } else {
         // (streaming mode: k_score only works for the candidates k_stream leaves to it -- circular contigs, and in the
         //  reference-faithful mode the candidates whose picks would not fit the list.  It runs BESIDE the streaming pair on
         //  the third stream -- different candidates, different partials -- and joins before k_finalize.)
         cudaStream_t ks = h->stream;
-        if (h->streaming) {
+        if (h->path == PATH_STREAM) {
             ks = h->pf;   // (k_classes ran on it: already ordered)
             cudaEventRecord(h->ev_pre, h->stream);
             cudaStreamWaitEvent(ks, h->ev_pre, 0);
-            k_stream<<<dim3(gsx, n), IG_THREADS, h->stream_smem, h->stream>>>(h->cv, h->coord, h->clen, h->sc, h->desc, h->rowidx, h->ns, h->row_cnt,
+            k_stream<<<dim3(h->grid_score, n), IG_THREADS, h->stream_smem, h->stream>>>(h->cv, h->coord, h->clen, h->sc, h->desc, h->rowidx, h->ns, h->row_cnt,
                                                                              h->bitmap, h->bitmap_words, h->cls16, h->part_c, h->pick_list, h->pick_cap,
                                                                              mbar, h->exz, h->clstab, h->subx, h->rinfo);
             k_eval_flat<true><<<h->grid_score, IG_THREADS, IG_SCORE_SMEM, h->stream>>>(h->sc, h->desc, h->ns, nullptr, 0, h->pick_list, h->pick_cap,
-                                                                               h->table, h->table_len, mbar, h->exz, h->part_nz, h->clstab, h->flat_items);
+                                                                               h->table, h->table_len, mbar, h->exz, h->part_nz, h->clstab);
         }
-        k_score<<<dim3(gsx, n), IG_THREADS, IG_SCORE_SMEM, ks>>>(h->row_ptr, h->cv, h->coord, h->clen, h->sc, h->desc, h->rows, h->rowidx,
-                                                                h->ns, h->row_cnt, h->table, h->table_len, mbar, h->exz, h->part_nz,
-                                                                h->part_c, h->gs_div, h->clstab, h->subx, h->rinfo, h->sparse_div);
+        k_score<<<dim3(h->grid_score, n), IG_THREADS, IG_SCORE_SMEM, ks>>>(h->row_ptr, h->cv, h->coord, h->clen, h->sc, h->desc, h->rows,
+                                                                          h->rowidx, h->ns, h->row_cnt, h->table, h->table_len, mbar, h->exz,
+                                                                          h->part_nz, h->part_c, h->clstab, h->subx, h->rinfo, h->split);
         if (ks != h->stream) {
             cudaEventRecord(h->ev_ksc, ks);
             cudaStreamWaitEvent(h->stream, h->ev_ksc, 0);
@@ -752,7 +752,7 @@ static int fetch_result(ig_handle* h, int n, const int32_t* cands, ig_step_resul
         CK(cudaStreamSynchronize(h->stream));
     }
     const DevScalars& s = *h->h_sc;
-    if (s.list_overflow) { h->err = "pick list of the streaming scoring path overflowed (IG_PICK_CAP)"; return -4; }
+    if (s.list_overflow) { h->err = "pick list of the streaming scoring path overflowed"; return -4; }
     const bool wide = n > IG_MAX_CANDS;
     const double* sv = wide ? h->h_wide->scores : s.scores;
     const int* nu = wide ? h->h_wide->n_uniq : s.res_nuniq;
@@ -788,19 +788,6 @@ static void enqueue_head(ig_handle* h, int full) {
     cudaEventRecord(h->ev_fork, h->stream);
     cudaStreamWaitEvent(h->side, h->ev_fork, 0);
     cudaStreamWaitEvent(h->pf, h->ev_fork, 0);
-    if (h->prefetch) {
-        PfList L;
-        int c = 0;
-        auto add = [&](const void* ptr, size_t bytes) { L.p[c] = (const char*)ptr; L.n[c] = bytes; c++; };
-        add(h->cv, sizeof(int2) * (size_t)h->nnz); add(h->row_ptr, sizeof(long long) * ((size_t)h->ns + 1));
-        add(h->coord, sizeof(CoordRec) * (size_t)h->ns); add(h->clen, sizeof(int) * (size_t)h->ns);
-        add(h->subx, sizeof(SubX) * (size_t)h->ns); add(h->sub, sizeof(SubRec) * (size_t)h->ns);
-        add(h->live, sizeof(FragRec) * (size_t)h->nf); add(h->exz, sizeof(float) * ((size_t)h->ns + 1));
-        add(h->init_prev, sizeof(int) * (size_t)h->nf); add(h->init_next, sizeof(int) * (size_t)h->nf);
-        add(h->orientable, sizeof(int) * (size_t)h->nf);
-        L.cnt = c;
-        k_prefetch_l2<<<h->n_part_zc, 256, 0, h->pf>>>(L);
-    }
     if (full == 2 || full == 3) {
         // parameters changed, scaffold bookkeeping intact (an accepted nuisance proposal): coordinates as in the incremental
         // step (k_commit_coords flags the rows of the previous move), zero terms and the full non-zero likelihood recomputed
@@ -847,7 +834,7 @@ static void enqueue_pass(ig_handle* h, int n, int first_flip_eject, const int* p
     const float mbar = h->cfg.mean_sub_len_kb;
     const FragRec* live = h->live;
     IG_MARK(0);
-    k_cand_setup<<<1, 32, 0, h->stream>>>(live, h->sc, h->desc, h->cfg.max_bounds_insert, first_flip_eject, plan, h->streaming ? h->stream_rows_max : 0);
+    k_cand_setup<<<1, 32, 0, h->stream>>>(live, h->sc, h->desc, h->cfg.max_bounds_insert, first_flip_eject, plan, h->path == PATH_STREAM ? h->stream_rows_max : 0);
     if (wide_rescore) k_wide_flip<<<1, 32, 0, h->stream>>>(h->sc, h->desc, h->wide);
     IG_MARK(1);
     k_find_cuts<<<(h->nf + 255) / 256, 256, 0, h->stream>>>(live, h->nf, h->sc, h->desc, h->clstab);
@@ -858,12 +845,13 @@ static void enqueue_pass(ig_handle* h, int n, int first_flip_eject, const int* p
     cudaStreamWaitEvent(h->stream, h->ev_coords, 0);
     IG_MARK(2);
     enqueue_scoring(h, n);
-    const int gsx = h->flat ? h->grid_flat : score_grid_x(h, n);
+    const bool flat = h->path == PATH_FLAT;
     cudaStreamWaitEvent(h->stream, h->ev_lnz, 0);
     IG_MARK(6);
     k_finalize<<<n, 1024, 0, h->stream>>>(h->row_ptr, h->cv, h->coord, h->sc, h->desc, h->rows, h->rowidx, h->ns, h->row_cnt, h->table,
-                                         h->table_len, mbar, h->exz, h->part_nz, h->part_c, h->flat ? h->grid_score : gsx, h->part_z, h->part_i,
-                                         h->grid_pre, h->cfg.n_pix, h->cfg.compat_last_block, h->d_nuniq, h->d_nsub, do_select, gsx, h->flat ? 1 : 0);
+                                         h->table_len, mbar, h->exz, h->part_nz, h->part_c, h->grid_score, h->part_z, h->part_i, h->grid_pre,
+                                         h->cfg.n_pix, h->cfg.compat_last_block, h->d_nuniq, h->d_nsub, do_select,
+                                         flat ? h->grid_flat : h->grid_score, flat ? 1 : 0);
     IG_MARK(7);
 }
 // the move selected by the last pass: incremental maintenance beside it, apply, contig bookkeeping (+ the cycle record)
@@ -934,14 +922,16 @@ static int step_kind(const ig_handle* h) {
     if (h->lnz_stale) return (h->lnz_cache && h->vinter_pos) ? 2 : 1;
     return 0;
 }
-// kernel launches of enqueue_head (per kind) and of one enqueue_pass
-static int head_launches(const ig_handle* h, int kind) { return (h->prefetch ? 1 : 0) + (kind >= 2 ? 6 : kind ? 4 : 1); }
-static int pass_launches(const ig_handle* h) { return 8 - (h->rows_small ? 1 : 0) + (h->flat ? 1 : 0) + (h->streaming ? 2 : 0); }
+// kernel launches of enqueue_head (per kind) and of one enqueue_pass: k_cand_setup, k_find_cuts, k_classes, the row list
+// (flat: one launch, else two), k_precompute, the scoring kernels (flat: k_pick + k_eval_flat; stream: k_stream +
+// k_eval_flat + k_score; rows: k_score) and k_finalize
+static int head_launches(int kind) { return kind >= 2 ? 6 : kind ? 4 : 1; }
+static int pass_launches(const ig_handle* h) { return h->path == PATH_STREAM ? 10 : 8; }
 // ... of a step of grid_n candidate slots: head, pass, tail (k_lnz_outside unless rigid, k_apply, k_post); a wide step adds
 // one pass with k_wide_stage and k_wide_stash per batch, and k_wide_pick, k_wide_flip, k_wide_finish
 static int step_launches(const ig_handle* h, int kind, int grid_n) {
     const int wide = grid_n > IG_MAX_CANDS ? n_batches_of(grid_n) * (pass_launches(h) + 2) + 3 : 0;
-    return head_launches(h, kind) + pass_launches(h) + (h->rigid ? 2 : 3) + wide;
+    return head_launches(kind) + pass_launches(h) + (h->rigid ? 2 : 3) + wide;
 }
 
 // capture what `enqueue` launches on the handle's stream into `exec`; a failed capture leaves it null and sets `failed`
@@ -1115,7 +1105,7 @@ static int collect_plan(ig_handle* h, int n_steps, ig_cycle_step* out) {
         h->vinter_pos = p.v_inter > 0.0f;   // (always: a proposal with v_inter <= 0 is never accepted)
     }
     h->nuis_enqueued = false;
-    if (overflow) { h->err = "pick list of the streaming scoring path overflowed (IG_PICK_CAP)"; return -4; }
+    if (overflow) { h->err = "pick list of the streaming scoring path overflowed"; return -4; }
     float ms = 0.f;
     if (cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]) == cudaSuccess) h->ms_step += ms;
     h->n_steps += n_steps;
@@ -1381,7 +1371,7 @@ extern "C" int ig_eval_scores(ig_handle* h, int32_t id_frag, int32_t id_cand, in
     enqueue_head(h, 1);
     enqueue_pass(h, 1, flip_eject, nullptr, 0);
     if (launch_ok(h, "eval_scores")) return -2;
-    h->n_launches += head_launches(h, 1) + pass_launches(h);
+    h->n_launches += head_launches(1) + pass_launches(h);
     h->coords_fresh = true; h->coords_ever = true;
     ig_step_result r;
     if (fetch_result(h, 1, &id_cand, &r, false, true, out24, n_uniq, n_sub)) return -2;

@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
 """Diagnostic: lockstep of the product vs the reference kernels (cubin) on a workload; at the first step whose scores
-differ by more than --tol, prints the per-proposal differences for the default path, the row-per-warp path (IG_FLAT=0)
+differ by more than --tol, prints the per-proposal differences for the default path, the row-per-warp path (IG_SCORING_PATH=rows)
 and the NumPy oracle.   python scripts/gpu_diag_lockstep.py --workload T --steps 900"""
 import argparse, os, sys
 import numpy as np
@@ -21,9 +21,9 @@ level = make_workload(a.workload); p8 = workload_params(level)
 st = burnt_state(level, p8, 2, 1000, "bomb")
 ref = RefReplaySampler(level, p8, backend="gpu")
 mine = GpuImpl(level)
-os.environ["IG_FLAT"] = "0"
+os.environ["IG_SCORING_PATH"] = "rows"
 rowp = GpuImpl(level)
-del os.environ["IG_FLAT"]
+del os.environ["IG_SCORING_PATH"]
 for i in (mine, rowp): i.set_params(p8)
 ref.set_state(st)
 distri = setup_distri_frags(level.sub_sampled_sparse_matrix, level.n_frags)

@@ -20,6 +20,17 @@ def make_sampler(level, **kw):
     return sampler(*level.sampler_args(), **kw)
 
 
+def assert_scoring_path(s, path, rigid=False):
+    """the handle scores through `path` (the level's natural one, or IG_SCORING_PATH when it was created): one host step
+    from a re-uploaded scaffold launches 4 head kernels (full refresh), the scoring pass -- 10 kernels on the stream path,
+    8 on the flat and rows paths -- and 3 tail kernels (2 with rigid pruning).  It moves the scaffold: call it last."""
+    s._set_state(s._get_state())
+    s.get_stats(reset=True)
+    s.step_sampler(0, 3, np.float32(0.01), candidates=[1, 2, 3])
+    want = 4 + (10 if path == "stream" else 8) + (2 if rigid else 3)
+    assert s.get_stats()["launches"] == want, (path, s.get_stats()["launches"], want)
+
+
 class GpuImpl:
     def __init__(self, level, **kw):
         self.s = make_sampler(level, **kw)
@@ -50,7 +61,9 @@ class GpuImpl:
 @pytest.mark.parametrize("split", ["", "24,1"])
 @pytest.mark.parametrize("name", GOLDEN_CASES)
 def test_cuda_replays_reference_trajectory(built, name, split, monkeypatch):
+    """the golden levels' natural flat path; `split`: the row-per-warp kernel (rows path) with that forced work split"""
     if split:
+        monkeypatch.setenv("IG_SCORING_PATH", "rows")
         monkeypatch.setenv("IG_FORCE_SPLIT", split)
     g = load_golden(name)
     level = make_level(WORKLOADS[str(g["workload"])])
@@ -60,6 +73,7 @@ def test_cuda_replays_reference_trajectory(built, name, split, monkeypatch):
     assert res.same_choice >= 0.9 * res.steps
     assert res.nuis_checked > 0
     assert res.max_rel < 1e-7
+    assert_scoring_path(impl.s, "rows" if split else "flat")
     impl.s.free_gpu()
 
 
@@ -72,13 +86,14 @@ def _oracle(level, p8):
 @pytest.mark.parametrize("seed", [0, 1, 2])
 def test_cuda_vs_oracle_random_scaffolds_with_circular_contigs(built, seed, split, d_exp, monkeypatch):
     """eval (score) + apply on random scaffolds the trajectories never reach (circular contigs,
-    reversed fragments), every op forced once through ig_apply.  `split` forces the scoring kernel's work
-    split (all 24 mutations per item = the large-assembly path with one evaluation per group of identical
-    motions; 6 mutations x 4 row parts = the small-assembly path), which small test levels would not reach;
-    `d_exp` = the exponent-cutoff parameter d of the p(s) model."""
+    reversed fragments), every op forced once through ig_apply.  `split` scores through the row-per-warp kernel
+    (rows path) with a forced work split (all 24 mutations per item = the large-assembly path with one evaluation per
+    group of identical motions; 6 mutations x 4 row parts = the small-assembly path), which small test levels would not
+    reach; `d_exp` = the exponent-cutoff parameter d of the p(s) model."""
     from oracle import moves as mv
     from oracle.fuzz import random_state
     if split:
+        monkeypatch.setenv("IG_SCORING_PATH", "rows")
         monkeypatch.setenv("IG_FORCE_SPLIT", split)
     level = make_level(WORKLOADS["micro"])
     rng = np.random.RandomState(seed)
@@ -124,6 +139,7 @@ def test_cuda_vs_oracle_random_scaffolds_with_circular_contigs(built, seed, spli
         got_state = s._get_state()
         for i, k in enumerate(FIELDS13):
             assert np.array_equal(got_state[i], new[k]), (it, op, k)
+    assert_scoring_path(s, "rows" if split else "flat")
     s.free_gpu()
 
 
@@ -292,9 +308,10 @@ def test_run_cycle_equals_stepwise(built):
     assert np.array_equal(res[0][2], res[1][2])
 
 
-def _lockstep(level, p8, n_steps, seed, bomb=False, n_neigh=5):
+def _lockstep(level, p8, n_steps, seed, bomb=False, n_neigh=5, path=None):
     """product and oracle advance together; after every step the oracle is resynchronised to the
-    product's state (so an exact tie broken differently cannot cascade)."""
+    product's state (so an exact tie broken differently cannot cascade).  path: the scoring path the product must
+    have taken (assert_scoring_path)."""
     import oracle.score as sc
     s = make_sampler(level)
     s.set_param_simu(p8)
@@ -329,6 +346,8 @@ def _lockstep(level, p8, n_steps, seed, bomb=False, n_neigh=5):
             ties += 1
             o.live = {k: st[i].copy() for i, k in enumerate(FIELDS13)}
         o.valid = [int(x) for x in s.get_valid_insert()]
+    if path:
+        assert_scoring_path(s, path)
     s.free_gpu()
     return ties
 
@@ -503,15 +522,16 @@ def test_yeast_toy_config0_lockstep(built):
     assert ties <= 8
 
 
-@pytest.mark.parametrize("env", [{"IG_ROWS_SMALL": "0"}, {"IG_PREFETCH": "1"}, {"IG_ROWS_SMALL": "0", "IG_FORCE_SPLIT": "24,1"}])
+@pytest.mark.parametrize("env", [{"IG_SCORING_PATH": "stream"}, {"IG_SCORING_PATH": "rows"},
+                                 {"IG_SCORING_PATH": "rows", "IG_FORCE_SPLIT": "24,1"}])
 def test_large_level_code_paths_on_a_small_level(built, env, monkeypatch):
-    """The two-pass affected-row list (levels above 16 Ki sub-fragments), the optional L2 prefetch and the
-    whole-row work split only run on large levels by default; forced here on the toy level, in lockstep with
-    the oracle."""
+    """The two-pass affected-row list (levels above 16 Ki sub-fragments) with the streaming path, with the row-per-warp
+    kernel, and with its whole-row work split only run on large levels by default; forced here on the toy level, in
+    lockstep with the oracle."""
     for k, v in env.items():
         monkeypatch.setenv(k, v)
     level = make_level(WORKLOADS["toy"])
-    ties = _lockstep(level, P8_RIPPE, 80, seed=6, bomb=True)
+    ties = _lockstep(level, P8_RIPPE, 80, seed=6, bomb=True, path=env["IG_SCORING_PATH"])
     assert ties <= 40
 
 
@@ -523,23 +543,24 @@ def test_medium_level_with_long_contigs_takes_the_large_level_paths_naturally(bu
     at a size the oracle still finishes in seconds per step.  Lockstep with the oracle."""
     level = make_level(SynthSpec(n_frags=6000, n_contigs=12, n_chrom=2, max_offset=300, lambda1=30.0, trans_per_row=2.0, seed=11))
     assert level.n_sub_frags > 16 * 1024
-    ties = _lockstep(level, P8_RIPPE, 30, seed=3)
+    ties = _lockstep(level, P8_RIPPE, 30, seed=3, path="stream")
     assert ties <= 6
 
 
 @pytest.mark.parametrize("rigid", [True, False])
 @pytest.mark.parametrize("workload,steps", [("T", 1200), ("toy", 400)])
 def test_streaming_path_equals_row_per_warp_rigid_path(built, workload, steps, rigid, monkeypatch):
-    """The streaming scoring path of large levels (k_stream + k_eval_flat<true>, rigid_pruning=1) forced on small levels:
-    same selected-contact counts, scores equal to the row-per-warp kernel's in rigid mode up to the 2^-32 fixed-point
-    rounding of its order-independent sums, same trajectory (unless two scores are that close), and two runs of the
-    streaming path are bit-identical although its pick list is appended in arbitrary order.  rigid = False: the same in the
-    reference-faithful mode, where large levels send their small candidates (mid-assembly contigs) down this path."""
+    """The streaming scoring path of large levels (k_stream + k_eval_flat<true>, rigid_pruning=1) forced on small levels
+    against the row-per-warp kernel k_score (rows path): same selected-contact counts, scores equal up to the 2^-32
+    fixed-point rounding of the streaming path's order-independent sums, same trajectory (unless two scores are that
+    close), and two runs of the streaming path are bit-identical although its pick list is appended in arbitrary order.
+    rigid = False: the same in the reference-faithful mode, where large levels send their small candidates (mid-assembly
+    contigs) down this path."""
     level = make_level(WORKLOADS[workload])
     p8 = P8_RIPPE if workload == "T" else P8
-    monkeypatch.setenv("IG_FLAT", "0")
+    monkeypatch.setenv("IG_SCORING_PATH", "rows")
     ref = make_sampler(level, rigid_pruning=rigid)        # k_score (rigid: with the rigid class-pair table)
-    monkeypatch.setenv("IG_FORCE_STREAM", "1")
+    monkeypatch.setenv("IG_SCORING_PATH", "stream")
     st1 = make_sampler(level, rigid_pruning=rigid)
     st2 = make_sampler(level, rigid_pruning=rigid)
     ss = [ref, st1, st2]
@@ -572,19 +593,20 @@ def test_streaming_path_equals_row_per_warp_rigid_path(built, workload, steps, r
                 s.set_valid_insert(ss[0].get_valid_insert())
     assert np.array_equal(ss[0]._get_state(), ss[1]._get_state()) or n_div > 0
     print("streaming vs row-per-warp (rigid): worst |score difference|", worst, "tie divergences", n_div)
-    for s in ss:
+    for s, path in zip(ss, ("rows", "stream", "stream")):
+        assert_scoring_path(s, path, rigid)
         s.free_gpu()
 
 
 @pytest.mark.parametrize("rigid", [True, False])
 def test_streaming_path_random_scaffolds_with_circular_contigs(built, rigid, monkeypatch):
     """eval on random scaffolds incl. circular contigs (left to k_score inside a streaming-mode step) and reversed
-    fragments: streaming == row-per-warp in rigid mode."""
+    fragments: the streaming path == the row-per-warp kernel (rows path)."""
     from oracle.fuzz import random_state
     level = make_level(WORKLOADS["micro"])
-    monkeypatch.setenv("IG_FLAT", "0")
+    monkeypatch.setenv("IG_SCORING_PATH", "rows")
     ref = make_sampler(level, rigid_pruning=rigid)
-    monkeypatch.setenv("IG_FORCE_STREAM", "1")
+    monkeypatch.setenv("IG_SCORING_PATH", "stream")
     st = make_sampler(level, rigid_pruning=rigid)
     for s in (ref, st):
         s.set_param_simu(P8)
@@ -606,6 +628,8 @@ def test_streaming_path_random_scaffolds_with_circular_contigs(built, rigid, mon
         assert res[0][1] == res[1][1], (it, a, b)
         assert np.array_equal(res[0][0] != 0, res[1][0] != 0)
         assert np.max(np.abs(res[0][0] - res[1][0])) < 1e-6, (it, a, b, np.max(np.abs(res[0][0] - res[1][0])))
+    assert_scoring_path(ref, "rows", rigid)
+    assert_scoring_path(st, "stream", rigid)
     ref.free_gpu(); st.free_gpu()
 
 

@@ -28,7 +28,7 @@ from oracle import moves as mv
 from oracle.fuzz import random_state
 from oracle.sampler_oracle import OracleSampler, distance_histogram
 from parity_common import FIELDS13
-from test_gpu_parity import P8, P8_RIPPE, _rebuild_offsets, make_sampler
+from test_gpu_parity import P8, P8_RIPPE, _rebuild_offsets, assert_scoring_path, make_sampler
 
 pytestmark = pytest.mark.gpu
 
@@ -379,17 +379,18 @@ def _score_pairs(name, rng, n):
 def test_large_level_scores_and_apply_match_oracle(built, name, d_exp):
     """eval_all_sub_likelihood (scores, scored set, n_sub_vals, validity list) and test_copy_struct (whole 13 x NF state)
     against the oracle on random scaffolds with long circular contigs and reversed fragments, through the level's natural
-    path, the reference-faithful streaming mode (IG_FLAT=0 IG_FORCE_STREAM=1) and the whole-row split (IG_FORCE_SPLIT=24,1).
+    path (the streaming path, in the reference-faithful mode), the row-per-warp kernel (IG_SCORING_PATH=rows) and its
+    whole-row split (IG_FORCE_SPLIT=24,1).
     The wrap level's zero terms count intra pairs with a wrapping int32 (k_precompute / k_finalize) against a wrapped n_pix."""
     level = _level(name)
     _check_level_size(name, level)
     p8 = P8_RIPPE.copy()
     p8[4] = d_exp
-    handles = [("natural", make_sampler(level))]
-    with _env(IG_FLAT=0, IG_FORCE_STREAM=1):
-        handles.append(("streaming", make_sampler(level)))
-    with _env(IG_FORCE_SPLIT="24,1"):
-        handles.append(("split 24,1", make_sampler(level)))
+    handles = [("stream", make_sampler(level))]
+    with _env(IG_SCORING_PATH="rows"):
+        handles.append(("rows", make_sampler(level)))
+    with _env(IG_SCORING_PATH="rows", IG_FORCE_SPLIT="24,1"):
+        handles.append(("rows split 24,1", make_sampler(level)))
     o = OracleSampler(level, p8)
     di = int(d_exp != 2.0)
     rng = np.random.RandomState(100 + di)
@@ -428,6 +429,8 @@ def test_large_level_scores_and_apply_match_oracle(built, name, d_exp):
                 got_state = s._get_state()
                 for i, k in enumerate(FIELDS13):
                     assert np.array_equal(got_state[i], new[k]), (where, op, k)
+        for label, s in handles:
+            assert_scoring_path(s, label.split()[0])
     finally:
         for _, s in handles:
             s.free_gpu()

@@ -114,12 +114,13 @@ def _mk(level, **kw):
     return make_sampler(level, **kw)
 
 
-def _wide_lockstep(level, p8, n_steps, seed, n_neigh, rigid=False):
+def _wide_lockstep(level, p8, n_steps, seed, n_neigh, rigid=False, path=None):
     """product and oracle advance together on steps of exactly n_neigh random candidates; besides the checks of
     test_gpu_parity._lockstep: the chosen move is the first index of the maximum non-zero score, its score is the step's
     likelihood, and the carried validity list equals the oracle's before any resynchronisation (quirk Q3).  rigid: scores
-    within the rigid mode's coordinate-rounding noise.  Returns (ties, steps won by a candidate of batch >= 1)."""
-    from test_gpu_parity import _oracle
+    within the rigid mode's coordinate-rounding noise; path: the scoring path the product must have taken.  Returns (ties,
+    steps won by a candidate of batch >= 1)."""
+    from test_gpu_parity import _oracle, assert_scoring_path
     s = _mk(level, rigid_pruning=rigid)
     s.set_param_simu(p8)
     o = _oracle(level, p8)
@@ -160,6 +161,8 @@ def _wide_lockstep(level, p8, n_steps, seed, n_neigh, rigid=False):
             ties += 1
             o.live = {k: st[i].copy() for i, k in enumerate(FIELDS13)}
         o.valid = [int(x) for x in s.get_valid_insert()]
+    if path:
+        assert_scoring_path(s, path, rigid)
     s.free_gpu()
     return ties, later
 
@@ -168,28 +171,31 @@ def _wide_lockstep(level, p8, n_steps, seed, n_neigh, rigid=False):
 @pytest.mark.parametrize("n_neigh", [9, 12, 16, 24])
 def test_wide_lockstep_toy(built, n_neigh):
     from test_gpu_parity import P8
-    ties, later = _wide_lockstep(make_level(WORKLOADS["toy"]), P8, 40, seed=n_neigh, n_neigh=n_neigh)
+    ties, later = _wide_lockstep(make_level(WORKLOADS["toy"]), P8, 40, seed=n_neigh, n_neigh=n_neigh, path="flat")
     assert ties <= 20
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("env", [{"IG_ROWS_SMALL": "0"}, {"IG_FORCE_SPLIT": "24,1"}])
+@pytest.mark.parametrize("env", [{"IG_SCORING_PATH": "rows"}, {"IG_SCORING_PATH": "rows", "IG_FORCE_SPLIT": "24,1"}])
 @pytest.mark.parametrize("n_neigh", [9, 12, 16, 24])
 def test_wide_lockstep_large_level_paths_on_toy(built, env, n_neigh, monkeypatch):
+    """the two-pass affected-row list and the row-per-warp kernel of the largest levels (rows path), with its adaptive
+    and its whole-row work split"""
     from test_gpu_parity import P8_RIPPE
     for k, v in env.items():
         monkeypatch.setenv(k, v)
-    ties, _ = _wide_lockstep(make_level(WORKLOADS["toy"]), P8_RIPPE, 30, seed=40 + n_neigh, n_neigh=n_neigh)
+    ties, _ = _wide_lockstep(make_level(WORKLOADS["toy"]), P8_RIPPE, 30, seed=40 + n_neigh, n_neigh=n_neigh, path="rows")
     assert ties <= 15
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("n_neigh", [9, 12, 16, 24])
 def test_wide_lockstep_medium_level(built, n_neigh):
-    """6000 fragments / 18k sub-fragments: the two-pass affected-row list and the row-per-warp kernel of large levels"""
+    """6000 fragments / 18k sub-fragments: the two-pass affected-row list and the streaming path of large levels, which
+    leaves the candidates that involve a circular contig to the row-per-warp kernel"""
     from test_gpu_parity import P8_RIPPE
     level = make_level(SynthSpec(n_frags=6000, n_contigs=12, n_chrom=2, max_offset=300, lambda1=30.0, trans_per_row=2.0, seed=11))
-    ties, _ = _wide_lockstep(level, P8_RIPPE, 4, seed=3, n_neigh=n_neigh)
+    ties, _ = _wide_lockstep(level, P8_RIPPE, 4, seed=3, n_neigh=n_neigh, path="stream")
     assert ties <= 2
 
 
@@ -198,9 +204,8 @@ def test_wide_lockstep_medium_level(built, n_neigh):
 @pytest.mark.parametrize("n_neigh", [9, 12, 16, 24])
 def test_wide_lockstep_streaming_path(built, n_neigh, rigid, monkeypatch):
     from test_gpu_parity import P8
-    monkeypatch.setenv("IG_FLAT", "0")
-    monkeypatch.setenv("IG_FORCE_STREAM", "1")
-    ties, _ = _wide_lockstep(make_level(WORKLOADS["toy"]), P8, 30, seed=70 + n_neigh, n_neigh=n_neigh, rigid=rigid)
+    monkeypatch.setenv("IG_SCORING_PATH", "stream")
+    ties, _ = _wide_lockstep(make_level(WORKLOADS["toy"]), P8, 30, seed=70 + n_neigh, n_neigh=n_neigh, rigid=rigid, path="stream")
     assert ties <= 15
 
 
